@@ -1,7 +1,7 @@
 """Headline benchmark: nanoGPT training step on char-level ABC tokens (BASELINE.json metric
 "train tokens/s & MFU, GPT-2-124M char-level ABC, 1/2/4/8 B200").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload cfg3|cfg2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload cfg3|cfg2] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -12,6 +12,7 @@ nanoGPT/bench.py:98-117).  Weak scaling: the per-GPU micro-batch is fixed as N g
 `value`  : tokens/s with the batch already resident in HBM (CUDA-event timed, max over ranks).
 `e2e`    : the same step driven through the public API with pinned-host -> device copies of X, Y and a
            device -> host read of the loss inside every timed step.
+`--dump-outputs DIR` : after the timed steps, what the last of them computed goes to DIR as float32 .npy files (dump_outputs).
 `roofline`, `kernel_breakdown` : per-kernel-family times from an instrumented pass (CUDA events on the launch
            stream around every C-ABI call), GEMM family against the measured cuBLAS bf16 peak.
 `cpu_baseline` / `--impl reference` : the reference step on the host cores (fp32, all host threads, also under torchrun) on a
@@ -174,7 +175,7 @@ def run_reference_arm(args, wl):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps, warmup = max(1, min(args.steps, 5)), max(1, min(args.warmup, 2))
+    steps, warmup = args.steps, max(1, min(args.warmup, 2))
     tps, dt, B, threads, kind = cpu_reference_tokens_per_s(wl, steps, warmup)
     what = "unmodified reference nanoGPT/model.py" if kind == "reference" else "oracle port"
     sample = f"{steps} timed + {warmup} warm-up optimizer steps of {B}x{wl['cfg']['block_size']} tokens (fp32, CPU, {what})"
@@ -200,6 +201,34 @@ def attn_flops(meta, bwd):
     return 2.5 * fwd if bwd else fwd
 
 
+# ----------------------------------------------------------------------------------------------------------------
+LOGITS_SAMPLE = 1 << 22   # elements; the default cfg3 / cfg2 batches (3.1 M / 1.6 M logits) are written whole
+PARAM_SAMPLE = 1 << 16    # elements per parameter tensor; a cfg3 dump (75 tensors + logits) is ~25 MB, well under 64 MB
+
+
+def _sample(t, limit):
+    """t as float32 numpy; above `limit` elements a fixed, seeded sample of `limit` of them (the same positions in every run)."""
+    import torch
+    t = t.detach()
+    if t.numel() > limit:
+        idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:limit].sort().values
+        t = t.reshape(-1)[idx.to(t.device)]
+    return t.float().cpu().numpy()
+
+
+def dump_outputs(out_dir, model, logits, loss, norm):
+    """What one training step hands its caller, as DIR/<name>.npy: `logits` and `loss` of the forward, `grad_norm` (the
+    pre-clip total norm clip_grad_norm_ returns) and `param.<name>` for every parameter after the optimizer step.  With the
+    same bench.py arguments the inputs are identical from run to run, so two builds can be compared file by file."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"logits": _sample(logits, LOGITS_SAMPLE), "loss": _sample(loss, 1), "grad_norm": _sample(norm, 1)}
+    for name, p in model.named_parameters():
+        arrays["param." + name] = _sample(p, PARAM_SAMPLE)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -212,7 +241,14 @@ def main():
     ap.add_argument("--dropout", type=float, default=0.0, help="train with dropout (music configs use 0.2; the headline uses 0 like nanoGPT/bench.py:54)")
     ap.add_argument("--bucket-mb", type=float, default=64.0,
                     help="gradient all-reduce bucket size (N > 1); a huge value = one exposed all-reduce after the backward")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (float32; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        # the reference arm times a bounded fp32 CPU sample (cpu_batch sequences), not the step of a build of this project
+        ap.error("--dump-outputs writes the outputs of the GPU training step; --impl reference has none")
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference_arm(args, wl)
@@ -256,12 +292,12 @@ def main():
     xd, yd = host[0][0].to(dev), host[0][1].to(dev)
 
     def step_resident():
-        _, loss = net(xd, yd)
+        logits, loss = net(xd, yd)
         opt.zero_grad(set_to_none=True)
         loss.backward()
-        model.clip_grad_norm_(1.0)
+        norm = model.clip_grad_norm_(1.0)
         opt.step()
-        return loss
+        return logits, loss, norm
 
     loss_host = torch.empty(1, dtype=torch.float32).pin_memory()
     loss_ready = torch.cuda.Event()
@@ -288,11 +324,12 @@ def main():
         torch.cuda.synchronize()
 
     def timed(fn, steps):
+        """(ms over `steps` calls of fn, what the last call returned)"""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for i in range(steps):
-            fn(i)
+            out = fn(i)
         e1.record()
         barrier()
         ms = e0.elapsed_time(e1)
@@ -300,7 +337,7 @@ def main():
             t = torch.tensor([ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = t.item()
-        return ms
+        return ms, out
 
     for i in range(max(args.warmup, 3)):
         step_resident()
@@ -308,14 +345,18 @@ def main():
     if rank == 0:
         sampler.start()
     launches0 = ops.LAUNCHES
-    ms_total = timed(lambda i: step_resident(), args.steps)
+    ms_total, last = timed(lambda i: step_resident(), args.steps)
     launches = ops.LAUNCHES - launches0
     clocks = sampler.stop() if rank == 0 else None
-    final_loss = step_resident().item()
+    if args.dump_outputs and rank == 0:
+        # before the next forward: the logits are a view of the activation buffer that it overwrites
+        dump_outputs(args.dump_outputs, model, *last)
+    del last
+    final_loss = step_resident()[1].item()
 
     for i in range(2):
         step_e2e(i)
-    ms_e2e = timed(step_e2e, args.steps)
+    ms_e2e, _ = timed(step_e2e, args.steps)
 
     # ---- instrumented pass: CUDA events around every C-ABI call (kernel family shares + GEMM roofline) -----------
     prof = []

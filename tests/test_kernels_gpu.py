@@ -39,7 +39,7 @@ def test_missing_cuda_tensor_is_loud(cuda_device):
                  out=torch.zeros(128, 128, dtype=torch.bfloat16))
 
 
-def test_pair_gemm_dynamic_tile_scheduler(cuda_device):
+def test_pair_gemm_dynamic_tile_scheduler(cuda_device, tmp_path):
     """Opt-in ticket-based tile scheduler of the CTA-pair GEMM (ABCGPT_DYNAMIC_TILES=1, read once per process): the same
     parity cases in a child process, including split-K wgrad (work items = tiles x splits) and the full cfg3 shapes (5-21
     tiles per pair, several trips around the 16-slot ring)."""
@@ -50,7 +50,8 @@ def test_pair_gemm_dynamic_tile_scheduler(cuda_device):
     names = ["gemm2_nt_small", "gemm2_nt_k512", "gemm2_nn", "gemm2_tn_red", "gemm2_ragged", "gemm2_gelu", "gemm2_resid",
              "gemm_perf_c_attn", "gemm_perf_c_fc_gelu", "gemm_perf_wgrad_fc", "gemm_perf_dgrad_fc"]
     r = subprocess.run([sys.executable, os.path.join(root, "tools", "gpu_probe.py"), *names],
-                       env=dict(os.environ, ABCGPT_DYNAMIC_TILES="1"), capture_output=True, text=True, timeout=600, cwd=root)
+                       env=dict(os.environ, ABCGPT_DYNAMIC_TILES="1", ABCGPT_PROBE_OUT=str(tmp_path)), capture_output=True,
+                       text=True, timeout=600, cwd=root)
     assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
     import re
     m = re.search(r"PROBE SUMMARY: (\d+)/(\d+) ok", r.stdout)   # names select by prefix (gemm2_gelu also runs gemm2_gelu_tanh)
