@@ -19,7 +19,7 @@ DEBUG_HEADER_PATH = os.path.join(os.path.dirname(HERE), "include", "abcgpt_debug
 
 EPI_BF16, EPI_GELU, EPI_RESID, EPI_DGELU, EPI_F32_RED, EPI_F32 = range(6)
 FN_IDS = {"abcgpt_gemm_bf16": 1, "abcgpt_embed_fwd": 2, "abcgpt_layernorm_fwd": 3, "abcgpt_attn_decode": 4, "abcgpt_argmax": 5,
-          "abcgpt_sample_topk": 6}
+          "abcgpt_sample_topk": 6, "abcgpt_attn_decode_hd": 7}
 ACT_TANH = 0x100  # OR-ed into EPI_GELU / EPI_DGELU: tanh form of GELU (include/abcgpt.h ABCGPT_ACT_TANH)
 
 _P = c_void_p
@@ -39,6 +39,8 @@ _SIGNATURES = {
     "abcgpt_layernorm_bwd": (c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, c_int, c_int, c_float, c_uint32, _P]),
     "abcgpt_attn_fwd": (c_int, [_P, _P, _P, c_int, c_int, c_int, c_float, c_uint32, _P]),
     "abcgpt_attn_bwd": (c_int, [_P, _P, _P, _P, _P, _P, c_int, c_int, c_int, c_float, c_uint32, _P]),
+    "abcgpt_attn_fwd_hd": (c_int, [_P, _P, _P, c_int, c_int, c_int, c_int, c_float, c_uint32, _P]),
+    "abcgpt_attn_bwd_hd": (c_int, [_P, _P, _P, _P, _P, _P, c_int, c_int, c_int, c_int, c_float, c_uint32, _P]),
     "abcgpt_ce_fwd": (c_int, [_P, c_int64, _P, _P, c_int, c_int, _P]),
     "abcgpt_ce_finalize": (c_int, [_P, _P, c_int, _P, _P, _P]),
     "abcgpt_ce_bwd": (c_int, [_P, c_int64, _P, _P, _P, _P, c_int, c_int, _P]),
@@ -47,6 +49,7 @@ _SIGNATURES = {
                              c_float, _P]),
     "abcgpt_cast_f32_to_bf16": (c_int, [_P, _P, c_int64, _P]),
     "abcgpt_attn_decode": (c_int, [_P, _P, c_int, c_int, c_int, c_int, _P]),
+    "abcgpt_attn_decode_hd": (c_int, [_P, _P, _P, c_int, c_int, c_int, c_int, c_int, _P]),
     "abcgpt_sample_batch": (c_int, [_P, c_int, c_int64, _P, _P, _P, c_int, c_int, _P]),
     "abcgpt_colsum_bf16": (c_int, [_P, c_int64, c_int, c_int, _P, _P]),
     "abcgpt_replay": (c_int, [_P, c_int64, c_int64]),

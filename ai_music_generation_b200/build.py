@@ -18,7 +18,7 @@ CSRC = os.path.join(HERE, "csrc")
 OBJ_DIR = os.path.join(HERE, "build")
 LIB_PATH = os.path.join(HERE, "libabcgpt.so")
 DEBUG_LIB_PATH = os.path.join(HERE, "libabcgpt_debug.so")  # product objects + instrumentation entry points (tools/ only)
-SOURCES = ["common.cu", "gemm.cu", "attn.cu", "attn_pair.cu", "attn_fwd3.cu", "layernorm.cu", "elementwise.cu", "nvls.cu", "sample.cu", "api.cu"]
+SOURCES = ["common.cu", "gemm.cu", "attn.cu", "attn_pair.cu", "attn_fwd3.cu", "attn_hd.cu", "layernorm.cu", "elementwise.cu", "nvls.cu", "sample.cu", "api.cu"]
 DEBUG_SOURCES = ["microbench.cu", "debug_api.cu"]  # include/abcgpt_debug.h; never linked into libabcgpt.so
 HEADERS = ["common.h", "kernels.h", "ptx.cuh", "dropout.cuh", "attn_helpers.cuh", os.path.join("..", "..", "include", "abcgpt.h"),
            os.path.join("..", "..", "include", "abcgpt_debug.h")]

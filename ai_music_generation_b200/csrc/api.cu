@@ -68,6 +68,16 @@ int abcgpt_attn_bwd(const void* qkv, const void* out, const void* dout, const fl
                     int B, int T, int H, float dropout_p, uint32_t dropout_key, void* stream) {
   return attn_bwd(qkv, out, dout, lse, delta, dqkv, B, T, H, dropout_p, dropout_key, S(stream));
 }
+int abcgpt_attn_fwd_hd(const void* qkv, void* out, float* lse, int B, int T, int H, int head_size, float dropout_p,
+                       uint32_t dropout_key, void* stream) {
+  if (head_size == 64) return abcgpt_attn_fwd(qkv, out, lse, B, T, H, dropout_p, dropout_key, stream);
+  return attn_fwd_hd(qkv, out, lse, B, T, H, head_size, dropout_p, dropout_key, S(stream));
+}
+int abcgpt_attn_bwd_hd(const void* qkv, const void* out, const void* dout, const float* lse, float* delta, void* dqkv, int B,
+                       int T, int H, int head_size, float dropout_p, uint32_t dropout_key, void* stream) {
+  if (head_size == 64) return abcgpt_attn_bwd(qkv, out, dout, lse, delta, dqkv, B, T, H, dropout_p, dropout_key, stream);
+  return attn_bwd_hd(qkv, out, dout, lse, delta, dqkv, B, T, H, head_size, dropout_p, dropout_key, S(stream));
+}
 
 int abcgpt_ce_fwd(const void* logits, int64_t ldl, const int64_t* targets, float* row_loss, int M, int V,
                   void* stream) {
@@ -95,6 +105,10 @@ int abcgpt_cast_f32_to_bf16(const float* x, void* y_bf16, int64_t n, void* strea
 }
 int abcgpt_attn_decode(const void* cache, void* out, int B, int Tmax, int n_keys, int H, void* stream) {
   return attn_decode(cache, out, B, Tmax, n_keys, H, S(stream));
+}
+int abcgpt_attn_decode_hd(const void* qkv_row, void* cache, void* out, int B, int Tmax, int t, int H, int head_size,
+                          void* stream) {
+  return attn_decode_hd(qkv_row, cache, out, B, Tmax, t, H, head_size, S(stream));
 }
 int abcgpt_sample_batch(const void* data, int token_bytes, int64_t n_tokens, const int64_t* ix, int64_t* x, int64_t* y, int B,
                         int T, void* stream) {
@@ -157,6 +171,10 @@ int abcgpt_replay(const int64_t* prog, int64_t n_words, int64_t k) {
       case ABCGPT_FN_ARGMAX:
         if (nargs != 7) return fail(-1, "abcgpt_replay: argmax takes 7 arguments");
         rc = abcgpt_argmax(P_(0), a[1], I_(2), MP_(int64_t, 3), a[4], I_(5), P_(6));
+        break;
+      case ABCGPT_FN_ATTN_DECODE_HD:
+        if (nargs != 9) return fail(-1, "abcgpt_replay: attn_decode_hd takes 9 arguments");
+        rc = abcgpt_attn_decode_hd(CP_(void, 0), P_(1), P_(2), I_(3), I_(4), I_(5), I_(6), I_(7), P_(8));
         break;
       case ABCGPT_FN_SAMPLE_TOPK:
         if (nargs != 11) return fail(-1, "abcgpt_replay: sample_topk takes 11 arguments");

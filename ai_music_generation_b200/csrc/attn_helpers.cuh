@@ -15,6 +15,10 @@ constexpr float kLog2e = 1.4426950408889634f;
 constexpr float kLn2 = 0.6931471805599453f;
 constexpr float kScale = 0.125f;  // 1/sqrt(64)
 constexpr float kSl2 = kScale * kLog2e;
+// softmax scale 1/sqrt(D) of the supported head sizes (csrc/attn_hd.cu: D = 32, 128); D = 64 gives exactly kScale / kSl2, so
+// the head-size-64 kernels compile to the same code as before the head size became a template parameter
+__host__ __device__ constexpr float scale_of(int D) { return D == 32 ? 0.17677669529663687f : (D == 128 ? 0.08838834764831845f : kScale); }
+__host__ __device__ constexpr float sl2_of(int D) { return D == HS ? kSl2 : scale_of(D) * kLog2e; }
 constexpr int kThreads = 192;  // warp 0 TMA, warp 1 MMA, warps 2..5 one thread per tile row
 
 __device__ __forceinline__ long long globaltimer_ns() {
@@ -172,7 +176,7 @@ __device__ __forceinline__ uint32_t prmt_sign(uint32_t x, uint32_t sel) {
 }
 
 // backward (dQ kernel): dS = P * (dP*scale - delta*scale) for one chunk; row statistics are per thread
-template <int MODE, bool DROP>
+template <int MODE, bool DROP, int D = HS>
 __device__ __forceinline__ void dq_chunk(uint32_t taddr_s, uint32_t taddr_dp, int lane, float neg_lse2, float neg_delta8,
                                          uint32_t* pk, const DropCfg& dcfg, uint32_t drop_rk, int kv0) {
   if (MODE == kMasked) {
@@ -184,8 +188,8 @@ __device__ __forceinline__ void dq_chunk(uint32_t taddr_s, uint32_t taddr_dp, in
   ptx::tmem_ld32(taddr_s, s);
   ptx::tmem_ld32(taddr_dp, dp);
   ptx::tmem_ld_wait();
-  const float2 sl = make_float2(kSl2, kSl2), nl = make_float2(neg_lse2, neg_lse2);
-  const float scv = DROP ? kScale * dcfg.inv_keep : kScale;  // dP = (dO V^T) o mask / (1-p): the factor rides on the scale
+  const float2 sl = make_float2(sl2_of(D), sl2_of(D)), nl = make_float2(neg_lse2, neg_lse2);
+  const float scv = DROP ? scale_of(D) * dcfg.inv_keep : scale_of(D);  // dP = (dO V^T) o mask / (1-p): the factor rides on the scale
   const float2 sc = make_float2(scv, scv), nd = make_float2(neg_delta8, neg_delta8);
   const uint32_t drop_b = drop_row_key2(drop_rk);
   const uint32_t drop_s = drop_rk + (static_cast<uint32_t>(kv0) >> 1) * kDropWeyl;
@@ -211,7 +215,7 @@ __device__ __forceinline__ void dq_chunk(uint32_t taddr_s, uint32_t taddr_dp, in
 
 // backward (dK/dV kernel): P^T and dS^T for one chunk; statistics are per COLUMN (query), read from shared memory.
 // MODE kDiag here is the general path: keep iff (q >= kv) && (q < T).
-template <int MODE, bool DROP>
+template <int MODE, bool DROP, int D = HS>
 __device__ __forceinline__ void dkv_chunk(uint32_t taddr_s, uint32_t taddr_dp, uint32_t st_lse2, uint32_t st_delta8,
                                           int q_base, int kv_t, int T, uint32_t* pk_p, uint32_t* pk_ds, const DropCfg& dcfg,
                                           uint32_t st_rowkey, int kv_real) {
@@ -224,8 +228,8 @@ __device__ __forceinline__ void dkv_chunk(uint32_t taddr_s, uint32_t taddr_dp, u
   ptx::tmem_ld32(taddr_s, s);
   ptx::tmem_ld32(taddr_dp, dp);
   ptx::tmem_ld_wait();
-  const float scv = DROP ? kScale * dcfg.inv_keep : kScale;  // the 1/(1-p) of dP rides on the scale, that of dV on its epilogue
-  const float2 sl = make_float2(kSl2, kSl2), sc = make_float2(scv, scv);
+  const float scv = DROP ? scale_of(D) * dcfg.inv_keep : scale_of(D);  // the 1/(1-p) of dP rides on the scale, that of dV on its epilogue
+  const float2 sl = make_float2(sl2_of(D), sl2_of(D)), sc = make_float2(scv, scv);
   // the mask row is the QUERY (a column here), so every element needs its own hash: lane (kv & 1) of pair kv >> 1
   const uint32_t drop_off = (static_cast<uint32_t>(kv_real) >> 1) * kDropWeyl;  // kv_real: key position in its real sequence
   const uint32_t drop_sel = (kv_t & 1) ? 0xBBBBu : 0x9999u;
@@ -286,7 +290,7 @@ __device__ __forceinline__ int real_col(int c, int seq_shift) { return c & ((1 <
 // p = 2^(s*sl2 - m_ref) for one 32-column chunk, also tracks the raw row max; MODE as for the other chunk helpers
 // DROP: attention dropout (SDPA dropout_p, model.py:64): the row sum uses the undropped probabilities, the P fed to P V is
 // masked and scaled by 1/(1-p); mask bit = f(site key, row (b,h,q), key position), regenerated in the backward kernels.
-template <int MODE, bool DROP>
+template <int MODE, bool DROP, int D = HS>
 __device__ __forceinline__ void fwd_chunk(uint32_t taddr, int lane, float neg_m, float& tmax, float& rowsum, uint32_t* pk,
                                           const DropCfg& dcfg, uint32_t drop_rk, int kv0) {
   if (MODE == kMasked) {
@@ -297,7 +301,7 @@ __device__ __forceinline__ void fwd_chunk(uint32_t taddr, int lane, float neg_m,
   uint32_t v[32];
   ptx::tmem_ld32(taddr, v);
   ptx::tmem_ld_wait();
-  const float2 sl = make_float2(kSl2, kSl2), nm = make_float2(neg_m, neg_m);
+  const float2 sl = make_float2(sl2_of(D), sl2_of(D)), nm = make_float2(neg_m, neg_m);
   float2 acc0 = make_float2(0.f, 0.f), acc1 = make_float2(0.f, 0.f);
   float m0 = tmax, m1 = -1e30f;
   const uint32_t drop_b = drop_row_key2(drop_rk);
@@ -333,16 +337,16 @@ __device__ __forceinline__ void fwd_chunk(uint32_t taddr, int lane, float neg_m,
   rowsum += (acc0.x + acc0.y) + (acc1.x + acc1.y);
 }
 
-template <bool DROP>
+template <bool DROP, int D = HS>
 __device__ __forceinline__ void fwd_tile(uint32_t tm_s, int lane, int cls0, int cls1, float neg_m, float& tmax, float& rowsum,
                                          uint32_t* pk, const DropCfg& dcfg, uint32_t drop_rk, int kv_tile0, int seq_shift) {
 #pragma unroll
   for (int c = 0; c < 2; ++c) {
     const int cls = c == 0 ? cls0 : cls1;
     const int kv0 = real_col(kv_tile0 + c * 32, seq_shift);
-    if (cls == kFull) fwd_chunk<kFull, DROP>(tm_s + c * 32, lane, neg_m, tmax, rowsum, pk + c * 16, dcfg, drop_rk, kv0);
-    else if (cls == kDiag) fwd_chunk<kDiag, DROP>(tm_s + c * 32, lane, neg_m, tmax, rowsum, pk + c * 16, dcfg, drop_rk, kv0);
-    else fwd_chunk<kMasked, DROP>(tm_s + c * 32, lane, neg_m, tmax, rowsum, pk + c * 16, dcfg, drop_rk, kv0);
+    if (cls == kFull) fwd_chunk<kFull, DROP, D>(tm_s + c * 32, lane, neg_m, tmax, rowsum, pk + c * 16, dcfg, drop_rk, kv0);
+    else if (cls == kDiag) fwd_chunk<kDiag, DROP, D>(tm_s + c * 32, lane, neg_m, tmax, rowsum, pk + c * 16, dcfg, drop_rk, kv0);
+    else fwd_chunk<kMasked, DROP, D>(tm_s + c * 32, lane, neg_m, tmax, rowsum, pk + c * 16, dcfg, drop_rk, kv0);
   }
 }
 

@@ -34,6 +34,12 @@ int attn_fwd(const void* qkv, void* out, float* lse, int B, int T, int H, float 
              cudaStream_t stream);
 int attn_bwd(const void* qkv, const void* out, const void* dout, const float* lse, float* delta, void* dqkv, int B,
              int T, int H, float drop_p, uint32_t drop_key, cudaStream_t stream);
+// csrc/attn_hd.cu: head sizes 32 and 128
+int attn_fwd_hd(const void* qkv, void* out, float* lse, int B, int T, int H, int D, float drop_p, uint32_t drop_key,
+                cudaStream_t stream);
+int attn_bwd_hd(const void* qkv, const void* out, const void* dout, const float* lse, float* delta, void* dqkv, int B, int T,
+                int H, int D, float drop_p, uint32_t drop_key, cudaStream_t stream);
+int attn_decode_hd(const void* qkv_row, void* cache, void* out, int B, int Tmax, int t, int H, int D, cudaStream_t stream);
 
 int ce_fwd(const void* logits, long long ldl, const int64_t* targets, float* row_loss, int M, int V,
            cudaStream_t stream);

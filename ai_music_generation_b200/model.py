@@ -87,6 +87,20 @@ def _round_up(x, m):
     return (x + m - 1) // m * m
 
 
+HEAD_SIZES = (32, 64, 128)   # head sizes the sm_100a attention kernels are built for (csrc/attn.cu: 64, csrc/attn_hd.cu: 32, 128)
+
+
+def head_size_of(cfg: GPTConfig) -> int:
+    """n_embd // n_head; raises ValueError unless n_embd splits evenly into heads of a supported size."""
+    if cfg.n_head <= 0 or cfg.n_embd % cfg.n_head != 0:
+        raise ValueError(f"n_embd ({cfg.n_embd}) must be a multiple of n_head ({cfg.n_head})")
+    D = cfg.n_embd // cfg.n_head
+    if D not in HEAD_SIZES:
+        raise ValueError(f"head size n_embd // n_head = {D} is not supported: the sm_100a attention kernels support head sizes "
+                         f"{', '.join(map(str, HEAD_SIZES))}")
+    return D
+
+
 class _Buffers:
     """Activation / scratch buffers for one (B, T) shape, allocated once and reused every step."""
 
@@ -135,16 +149,19 @@ class _Buffers:
 
 
 class _DecodeState:
-    """Buffers of the single-token decode path: the per-layer cache of c_attn outputs [B, Tmax, 3C] and the [B, *] row
-    buffers of one step."""
+    """Buffers of the single-token decode path: the per-layer head-major cache of c_attn outputs and the [B, *] row buffers of
+    one step.  Head size 64: [B, 3H, Tmax, 64] (q | k | v heads, written by the head-strided GEMM); other head sizes:
+    [B, 2H, Tmax, D] (k | v heads, appended by the decode kernel from the [B, 3C] row `qkv`)."""
 
     def __init__(self, cfg: GPTConfig, B: int, Tmax: int, device):
         C, L = cfg.n_embd, cfg.n_layer
         bf, f32 = torch.bfloat16, torch.float32
         e = lambda *s, dt=bf: torch.empty(*s, device=device, dtype=dt)  # noqa: E731
         self.B, self.Tmax = B, Tmax
+        self.D = head_size_of(cfg)
         self.Vpad = _round_up(cfg.vocab_size, 128) if cfg.vocab_size <= 1024 else _round_up(cfg.vocab_size, 8)
-        self.cache = [e(B, Tmax * 3 * C) for _ in range(L)]
+        self.cache = [e(B, Tmax * (3 if self.D == 64 else 2) * C) for _ in range(L)]
+        self.qkv = e(B, 3 * C) if self.D != 64 else None
         self.x = [e(B, C, dt=f32) for _ in range(2)]
         self.ln = e(B, C)
         self.att = e(B, C)
@@ -228,7 +245,7 @@ class GPT(nn.Module):
     def __init__(self, config: GPTConfig):
         super().__init__()
         assert config.vocab_size is not None and config.block_size is not None
-        assert config.n_embd // config.n_head == 64, "the sm_100a attention kernels are specialised for head size 64"
+        self._head_size = head_size_of(config)
         assert config.activation in ("gelu", "gelu_tanh"), config.activation
         self._act = ops.ACT_TANH if config.activation == "gelu_tanh" else 0
         self.config = config
@@ -469,7 +486,8 @@ class GPT(nn.Module):
             b = lambda name: None if lw[name] is None else lw[name][0]  # noqa: E731
             ops.layernorm_fwd(x_in, lw["ln_1.weight"][0], b("ln_1.bias"), bufs.ln1[k], st[0], st[1])
             ops.gemm(bufs.ln1[k], lw["attn.c_attn.weight"][1], epilogue=ops.EPI_BF16, out=bufs.qkv[k], bias=b("attn.c_attn.bias"))
-            ops.attn_fwd(bufs.qkv[k], bufs.att[k], bufs.lse[k], B, T, H, drop_p=p_drop, drop_key=keys[1 + 3 * li])
+            ops.attn_fwd(bufs.qkv[k], bufs.att[k], bufs.lse[k], B, T, H, drop_p=p_drop, drop_key=keys[1 + 3 * li],
+                         head_size=self._head_size)
             # attention branch: the K = 768 projection with the residual add in its epilogue was bound by its fp32 residual
             # loads (0.080 ms against 0.038 ms of HBM time at cfg3); the add rides on the LayerNorm pass that follows instead
             # (x_mid = x + drop(c_proj(att)), ln_2(x_mid) in one kernel; the bf16 branch output mostly stays in L2 in between)
@@ -604,7 +622,7 @@ class GPT(nn.Module):
                 ops.record_callback(lambda li_=held: sync.layer_done(li_))
                 held = None
             ops.attn_bwd(bufs.qkv[li], bufs.att[li], bufs.datt, bufs.lse[li], bufs.delta, bufs.dqkv, B, T, H,
-                         drop_p=p_drop, drop_key=keys[1 + 3 * li])
+                         drop_p=p_drop, drop_key=keys[1 + 3 * li], head_size=self._head_size)
             wgrad(bufs.dqkv, bufs.ln1[li], "attn.c_attn", J3)
             ops.gemm(bufs.dqkv, lw["attn.c_attn.weight"][1], b_mn=True, epilogue=ops.EPI_BF16, out=bufs.dln)
             before_overwrite(J0)
@@ -868,11 +886,17 @@ class GPT(nn.Module):
         for li, lw in enumerate(layers):
             b = lambda name: None if lw[name] is None else lw[name][0]  # noqa: E731
             ops.layernorm_fwd(x, lw["ln_1.weight"][0], b("ln_1.bias"), st.ln, st.stat[0], st.stat[1])
-            # the GEMM writes this position's q | k | v straight into the head-major cache [B, 3H, Tmax, 64]
-            qkv_t = st.cache[li].view(B, 3 * H, st.Tmax, 64)[:, 0, t, :]
-            ops.gemm(st.ln, lw["attn.c_attn.weight"][1], epilogue=ops.EPI_BF16, out=qkv_t, bias=b("attn.c_attn.bias"), tile_n=128,
-                     head_stride=st.Tmax * 64)
-            ops.attn_decode(st.cache[li], st.att, B, st.Tmax, t + 1, H)
+            if st.D == 64:
+                # the GEMM writes this position's q | k | v straight into the head-major cache [B, 3H, Tmax, 64]
+                qkv_t = st.cache[li].view(B, 3 * H, st.Tmax, 64)[:, 0, t, :]
+                ops.gemm(st.ln, lw["attn.c_attn.weight"][1], epilogue=ops.EPI_BF16, out=qkv_t, bias=b("attn.c_attn.bias"),
+                         tile_n=128, head_stride=st.Tmax * 64)
+                ops.attn_decode(st.cache[li], st.att, B, st.Tmax, t + 1, H)
+            else:
+                # other head sizes: a plain [B, 3C] row; the decode kernel appends its k | v to the cache [B, 2H, Tmax, D]
+                ops.gemm(st.ln, lw["attn.c_attn.weight"][1], epilogue=ops.EPI_BF16, out=st.qkv, bias=b("attn.c_attn.bias"),
+                         tile_n=128)
+                ops.attn_decode_hd(st.qkv, st.cache[li], st.att, B, st.Tmax, t, H, st.D)
             ops.gemm(st.att, lw["attn.c_proj.weight"][1], epilogue=ops.EPI_RESID, out=y, aux=x, bias=b("attn.c_proj.bias"),
                      tile_n=128)
             ops.layernorm_fwd(y, lw["ln_2.weight"][0], b("ln_2.bias"), st.ln, st.stat[0], st.stat[1])

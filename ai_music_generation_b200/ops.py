@@ -335,15 +335,26 @@ def layernorm_bwd(dy_bf16, x, weight, mean, rstd, dresid_in, dx_out, dx_bf16, dw
           _ptr(dbias), M, C, drop_p, drop_key, _stream())
 
 
-def attn_fwd(qkv, out, lse, B, T, H, drop_p=0.0, drop_key=0):
+def attn_fwd(qkv, out, lse, B, T, H, drop_p=0.0, drop_key=0, head_size=64):
+    """Causal attention over the packed [B*T, 3C] qkv buffer, C = H * head_size.  head_size 64 runs the tuned kernels of
+    csrc/attn.cu; 32 and 128 those of csrc/attn_hd.cu (abcgpt_attn_fwd_hd), recorded under the same name so that a launch
+    plan patches their dropout keys like any other attention launch."""
     _chk(qkv, torch.bfloat16, "attn qkv")
-    _call("attn_fwd", 1, (B, T, H), _C.lib().abcgpt_attn_fwd, qkv.data_ptr(), out.data_ptr(), lse.data_ptr(), B, T, H,
-          drop_p, drop_key, _stream())
+    if head_size == 64:
+        _call("attn_fwd", 1, (B, T, H), _C.lib().abcgpt_attn_fwd, qkv.data_ptr(), out.data_ptr(), lse.data_ptr(), B, T, H,
+              drop_p, drop_key, _stream())
+    else:
+        _call("attn_fwd", 1, (B, T, H, head_size), _C.lib().abcgpt_attn_fwd_hd, qkv.data_ptr(), out.data_ptr(), lse.data_ptr(),
+              B, T, H, int(head_size), drop_p, drop_key, _stream())
 
 
-def attn_bwd(qkv, out, dout, lse, delta, dqkv, B, T, H, drop_p=0.0, drop_key=0):
-    _call("attn_bwd", 3, (B, T, H), _C.lib().abcgpt_attn_bwd, qkv.data_ptr(), out.data_ptr(), dout.data_ptr(),
-          lse.data_ptr(), delta.data_ptr(), dqkv.data_ptr(), B, T, H, drop_p, drop_key, _stream())
+def attn_bwd(qkv, out, dout, lse, delta, dqkv, B, T, H, drop_p=0.0, drop_key=0, head_size=64):
+    if head_size == 64:
+        _call("attn_bwd", 3, (B, T, H), _C.lib().abcgpt_attn_bwd, qkv.data_ptr(), out.data_ptr(), dout.data_ptr(),
+              lse.data_ptr(), delta.data_ptr(), dqkv.data_ptr(), B, T, H, drop_p, drop_key, _stream())
+    else:
+        _call("attn_bwd", 3, (B, T, H, head_size), _C.lib().abcgpt_attn_bwd_hd, qkv.data_ptr(), out.data_ptr(), dout.data_ptr(),
+              lse.data_ptr(), delta.data_ptr(), dqkv.data_ptr(), B, T, H, int(head_size), drop_p, drop_key, _stream())
 
 
 def ce_fwd(logits, targets, row_loss, sum_count, loss, V):
@@ -419,6 +430,13 @@ def colsum_bf16(dy, out):
 def attn_decode(cache, out, B, Tmax, n_keys, H):
     _call("attn_decode", 1, (B, n_keys, H), _C.lib().abcgpt_attn_decode, cache.data_ptr(), out.data_ptr(), B, Tmax, n_keys, H,
           _stream())
+
+
+def attn_decode_hd(qkv_row, cache, out, B, Tmax, t, H, head_size):
+    """Decode position t for head sizes 32 / 128 (include/abcgpt.h abcgpt_attn_decode_hd): appends k, v of qkv_row [B, 3C] to the
+    head-major cache [B, 2H, Tmax, head_size] and attends over its rows [0, t]; out [B, C]."""
+    _call("attn_decode_hd", 1, (B, t + 1, H, head_size), _C.lib().abcgpt_attn_decode_hd, qkv_row.data_ptr(), cache.data_ptr(),
+          out.data_ptr(), B, Tmax, t, H, int(head_size), _stream())
 
 
 def sample_batch(data, ix, x, y):

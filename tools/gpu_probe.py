@@ -131,14 +131,14 @@ def case_gemm(name, M, N, K, a_mn, b_mn, epi, tile_n, splits=0, timing=True, tan
     return res
 
 
-def _attn_ref(qkv, B, T, H):
+def _attn_ref(qkv, B, T, H, D=64):
     import torch
-    C = H * 64
+    C = H * D
     q, k, v = qkv.float().split(C, dim=1)
-    q = q.view(B, T, H, 64).transpose(1, 2)
-    k = k.view(B, T, H, 64).transpose(1, 2)
-    v = v.view(B, T, H, 64).transpose(1, 2)
-    s = (q @ k.transpose(-1, -2)) * 0.125
+    q = q.view(B, T, H, D).transpose(1, 2)
+    k = k.view(B, T, H, D).transpose(1, 2)
+    v = v.view(B, T, H, D).transpose(1, 2)
+    s = (q @ k.transpose(-1, -2)) * (1.0 / math.sqrt(D))
     mask = torch.ones(T, T, device=qkv.device, dtype=torch.bool).tril()
     s = s.masked_fill(~mask, float("-inf"))
     lse = torch.logsumexp(s, dim=-1)
@@ -147,12 +147,13 @@ def _attn_ref(qkv, B, T, H):
     return o, lse
 
 
-def case_attn(name, B, T, H, bwd, timing=True, spike=False):
+def case_attn(name, B, T, H, bwd, timing=True, spike=False, D=64):
+    """D: head size (64: csrc/attn.cu; 32 / 128: csrc/attn_hd.cu)."""
     import torch
     from ai_music_generation_b200 import ops
     torch.manual_seed(0)
     dev = "cuda"
-    C = H * 64
+    C = H * D
     qkv = torch.randn(B * T, 3 * C, device=dev)
     if spike:
         # scores jump by ~2^100 after the first 64 keys: exercises the lazy-rescale path of the forward kernel
@@ -164,12 +165,12 @@ def case_attn(name, B, T, H, bwd, timing=True, spike=False):
     out = torch.zeros(B * T, C, device=dev, dtype=torch.bfloat16)
     lse = torch.zeros(B, H, T, device=dev)
     res = {"case": name}
-    ops.attn_fwd(qkv, out, lse, B, T, H)
+    ops.attn_fwd(qkv, out, lse, B, T, H, head_size=D)
     torch.cuda.synchronize()
     small = B * H * T * T <= 64 * 1024 * 1024
     if small:
         qkv_f = qkv.float().requires_grad_(True)
-        o_ref, lse_ref = _attn_ref(qkv_f, B, T, H)
+        o_ref, lse_ref = _attn_ref(qkv_f, B, T, H, D)
         res["errs"] = [_err(out, o_ref.detach()), _err(lse, lse_ref.detach())]
         res["ok"] = res["errs"][0]["max_abs"] < 0.03 and res["errs"][1]["max_abs"] < 0.01
         if not res["ok"]:
@@ -180,7 +181,7 @@ def case_attn(name, B, T, H, bwd, timing=True, spike=False):
         dout = torch.randn(B * T, C, device=dev).bfloat16()
         dqkv = torch.zeros(B * T, 3 * C, device=dev, dtype=torch.bfloat16)
         delta = torch.zeros(B, H, T, device=dev)
-        ops.attn_bwd(qkv, out, dout, lse, delta, dqkv, B, T, H)
+        ops.attn_bwd(qkv, out, dout, lse, delta, dqkv, B, T, H, head_size=D)
         torch.cuda.synchronize()
         if small:
             o_ref.backward(dout.float())
@@ -188,18 +189,21 @@ def case_attn(name, B, T, H, bwd, timing=True, spike=False):
             e = {"dq": _err(dqkv[:, :C], g[:, :C]), "dk": _err(dqkv[:, C:2 * C], g[:, C:2 * C]),
                  "dv": _err(dqkv[:, 2 * C:], g[:, 2 * C:])}
             res["bwd_errs"] = e
-            res["bwd_ok"] = all(v["rel_l2"] < 0.02 for v in e.values())
+            # T = 1: dQ and dK are exactly zero (softmax over one key), where only an absolute bound is meaningful
+            zero = {"dq": g[:, :C].abs().max().item() == 0, "dk": g[:, C:2 * C].abs().max().item() == 0,
+                    "dv": g[:, 2 * C:].abs().max().item() == 0}
+            res["bwd_ok"] = all(v["rel_l2"] < 0.02 or (zero[k] and v["max_abs"] < 1e-5) for k, v in e.items())
             if not res["bwd_ok"]:
                 res["map_dq"] = _mismatch_map(dqkv[:, :64], g[:, :64], 0.05, rb=16, cb=8, max_r=256, max_c=64)
                 res["map_dk"] = _mismatch_map(dqkv[:, C:C + 64], g[:, C:C + 64], 0.05, rb=16, cb=8, max_r=256, max_c=64)
                 res["map_dv"] = _mismatch_map(dqkv[:, 2 * C:2 * C + 64], g[:, 2 * C:2 * C + 64], 0.05, rb=16, cb=8, max_r=256, max_c=64)
             res["ok"] = res["ok"] and res["bwd_ok"]
     if timing and res["ok"]:
-        ms = _timeit(lambda: ops.attn_fwd(qkv, out, lse, B, T, H))
-        fl = 4.0 * B * H * T * T * 64 / 2
+        ms = _timeit(lambda: ops.attn_fwd(qkv, out, lse, B, T, H, head_size=D))
+        fl = 4.0 * B * H * T * T * D / 2
         res["fwd_ms"], res["fwd_tflops_causal"] = ms, fl / ms / 1e9
         if bwd:
-            ms = _timeit(lambda: ops.attn_bwd(qkv, out, dout, lse, delta, dqkv, B, T, H))
+            ms = _timeit(lambda: ops.attn_bwd(qkv, out, dout, lse, delta, dqkv, B, T, H, head_size=D))
             res["bwd_ms"], res["bwd_tflops_causal"] = ms, 2.5 * fl / ms / 1e9
     return res
 
@@ -440,6 +444,14 @@ def build_cases():
     cases["attn_spike"] = lambda: case_attn("attn_spike", 2, 320, 2, True, timing=False, spike=True)
     cases["attn_perf_cfg2"] = lambda: case_attn("attn_perf_cfg2", 64, 256, 6, True)
     cases["attn_perf_cfg3"] = lambda: case_attn("attn_perf_cfg3", 32, 1024, 12, True)
+    # --- head sizes 32 and 128 (csrc/attn_hd.cu): ragged tails, one position, the rescale path, same tolerances
+    for D, H in ((32, 4), (128, 2)):
+        for T, B in ((1, 3), (32, 3), (100, 2), (128, 2), (200, 2), (256, 2), (1024, 2)):
+            n = f"attn_d{D}_t{T}"
+            cases[n] = (lambda n=n, B=B, T=T, H=H, D=D: case_attn(n, B, T, H, True, timing=False, D=D))
+        cases[f"attn_d{D}_spike"] = (lambda D=D, H=H: case_attn(f"attn_d{D}_spike", 2, 320, H, True, timing=False, spike=True, D=D))
+    for D, H in ((32, 24), (128, 6)):   # the GPT-2-small width (C = 768) at 32 x 1024 tokens
+        cases[f"attn_d{D}_perf_c768"] = (lambda D=D, H=H: case_attn(f"attn_d{D}_perf_c768", 32, 1024, H, True, D=D))
     # --- memory-bound kernels
     cases["ln_384"] = lambda: case_layernorm("ln_384", 16384, 384, False)
     cases["ln_768"] = lambda: case_layernorm("ln_768", 32768, 768, False)
