@@ -225,6 +225,15 @@ __device__ __forceinline__ uint32_t mapa(uint32_t local_smem_addr, uint32_t rank
   asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(local_smem_addr), "r"(rank));
   return r;
 }
+// distributed shared memory: plain load from / min-reduction into a peer CTA's shared memory (address from mapa)
+__device__ __forceinline__ uint32_t ld_shared_cluster_u32(uint32_t cluster_addr) {
+  uint32_t v;
+  asm volatile("ld.shared::cluster.u32 %0, [%1];" : "=r"(v) : "r"(cluster_addr) : "memory");
+  return v;
+}
+__device__ __forceinline__ void red_min_shared_cluster_s32(uint32_t cluster_addr, int v) {
+  asm volatile("red.shared::cluster.min.s32 [%0], %1;" ::"r"(cluster_addr), "r"(v) : "memory");
+}
 __device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
   asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
 }
