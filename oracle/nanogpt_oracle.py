@@ -158,10 +158,11 @@ def _attention(qkv, n_head, bf16, drop_mask=None, p=0.0, key_padding=None):
         y = F.scaled_dot_product_attention(q, k, v, attn_mask=None, dropout_p=0.0, is_causal=True)
         return y.transpose(1, 2).contiguous().view(B, T, C)
     att = (q @ k.transpose(-2, -1)) * (1.0 / math.sqrt(hs))
-    mask = torch.ones(T, T, dtype=torch.bool).tril()
+    mask = torch.ones(T, T, dtype=torch.bool, device=qkv.device).tril()   # qkv's device: the kernel tests run this on the GPU
     att = att.masked_fill(~mask, float("-inf"))
     if key_padding is not None:  # HF attention_mask of TunesFormer's char decoder (tunesformer/utils.py:128-133,152-154): bool [B, T], True = pad key
-        att = att.masked_fill(key_padding[:, None, None, :] & ~torch.eye(T, dtype=torch.bool)[None, None], float("-inf"))
+        att = att.masked_fill(key_padding[:, None, None, :] & ~torch.eye(T, dtype=torch.bool, device=qkv.device)[None, None],
+                              float("-inf"))
     att = torch.softmax(att, dim=-1)
     if drop_mask is not None:  # attn_dropout (:70) / SDPA dropout_p (:64) on the probabilities
         att = att * drop_mask.to(att.dtype) / (1.0 - p)
