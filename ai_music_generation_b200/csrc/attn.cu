@@ -42,28 +42,15 @@ struct FwdSmem {
   static constexpr int Q = 0;                       // 2 items x (128 x 64 bf16)
   static constexpr int KV = 32768;                  // kFwdRing stages x (K 64x64 | V 64x64)
   static constexpr int BAR = KV + kFwdRing * 16384;
-  static constexpr int XCH = BAR + 256;             // NH = 2: row statistics exchanged between the two column halves
-  static constexpr int TOTAL = XCH + 4608 + 1024;   //   [2 parities][2 halves][128] step max | same for the item row sums | flags
+  static constexpr int TOTAL = BAR + 256 + 1024;
 };
 
-// NH = number of column halves of a score tile that separate warps work on.  NH = 1: four compute warps, a thread owns one row
-// and all 64 columns of every step.  NH = 2: EIGHT compute warps, two per 32-row quarter of the tile (a warp can only reach the
-// tensor-memory lanes of its own quarter), each thread owns one row and 32 of the 64 columns.  Why: a step of the NH = 1 kernel
-// is ~1150 cycles of ONE warp per scheduler issuing ~600 dependent instructions and 64 MUFU (step traces, tools/attn_trace.py:
-// IPC 0.4 per warp, issue slots 46 % busy with both resident CTAs), while the tensor pipe needs ~320 cycles for the step's eight
-// MMAs (tools/tmem_mma_bench.py: 48 cycles per 128x64x16 from shared memory, not the 74 an earlier benchmark loop reported);
-// twice the warps per scheduler is twice the issue and MUFU concurrency.  The two halves of a row share the reference exponent
-// (exchanged once per item) and agree on the rare in-TMEM rescale through a flag exchange per step (named barrier per quarter,
-// 64 threads); row sums are kept per half and added in the item epilogue.
-// MEASURED: parity-green and NO faster (0.124 vs 0.121 ms per layer at cfg3; with half of the exponentials moved to the FMA pipe,
-// -DABCGPT_POLY_EXP, 0.134 vs 0.131 ms).  With both resident CTAs in their softmax phase the SM already runs 2 x 8192
-// exponentials per ~1300-cycle step = 12.6 per clock of the MUFU's 16, and its issue slots are 60 % (MUFU form) to 85 % (polynomial
-// form) busy in steady state: the kernel sits on BOTH limits, so neither more warps nor trading MUFU for FMA instructions moves
-// it.  What would: fewer instructions AND fewer MUFU operations per element (packed half-precision ex2 straight into the MMA
-// operand format, row sums from a ones column of V), i.e. a different inner loop.  NH = 1 is the default; ABCGPT_ATTN_FWD_NH=2
-// selects this form.
-template <bool DROP, int NH>
-__global__ void __launch_bounds__(64 + 128 * NH, 2)
+// Four compute warps, one per 32-row quarter of the tile (a warp can only reach the tensor-memory lanes of its own quarter): a
+// thread owns one row and all 64 columns of every step.  With both resident CTAs in their softmax phase the SM runs 2 x 8192
+// exponentials per ~1300-cycle step = 12.6 per clock of the MUFU's 16, with its issue slots ~60 % busy: the kernel sits on both
+// limits, so neither more warps per row nor trading MUFU for FMA instructions moves it (DESIGN.md §4.2 records both attempts).
+template <bool DROP>
+__global__ void __launch_bounds__(kThreads, 2)
 attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmKV,
                 __nv_bfloat16* __restrict__ out, float* __restrict__ lse, int T, int H, int C, int BH, int nitems,
                 long long* trace, const DropCfg dcfg, long long* cta_trace, int seq_shift, const FastDiv fBH, const FastDiv fH) {
@@ -81,9 +68,6 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
   uint64_t* o_full = p_empty + 2;                // [2]
   uint64_t* o_free = o_full + 2;                 // [2]
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(o_free + 2);
-  float* xch_max = reinterpret_cast<float*>(smem + FwdSmem::XCH);          // [2][2][128]
-  float* xch_l = xch_max + 512;                                            // [2][2][128]
-  uint32_t* xch_flag = reinterpret_cast<uint32_t*>(xch_l + 512);           // [2][4 quarters][2 halves]
 
   const int warp = ptx::uniform(threadIdx.x >> 5), lane = threadIdx.x & 31;
   const int nqt = (T + 127) / 128;
@@ -99,10 +83,10 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
       ptx::mbar_init(&q_full[s], 1);
       ptx::mbar_init(&q_empty[s], 1);
       ptx::mbar_init(&s_full[s], 1);
-      ptx::mbar_init(&p_full[s], 128 * NH);
+      ptx::mbar_init(&p_full[s], 128);
       ptx::mbar_init(&p_empty[s], 1);
       ptx::mbar_init(&o_full[s], 1);
-      ptx::mbar_init(&o_free[s], 128 * NH);
+      ptx::mbar_init(&o_free[s], 128);
     }
     for (int s = 0; s < kFwdRing; ++s) {
       ptx::mbar_init(&kv_full[s], 1);
@@ -190,7 +174,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
         const uint32_t tP = tmem_base + (p_gt & 1) * 64;  // bf16 P (32 packed columns) written over the consumed S tile
         const uint32_t tO = tmem_base + 128 + (p_k & 1) * 64;
 #pragma unroll
-        for (int k = 0; k < 4; ++k) if (leader) ptx::umma_ts(tO, tP + 8 * k + ((NH == 2 && k >= 2) ? 16 : 0), desc_mn(sV, k), idesc_o, (p_j > 0 || k > 0));
+        for (int k = 0; k < 4; ++k) if (leader) ptx::umma_ts(tO, tP + 8 * k, desc_mn(sV, k), idesc_o, (p_j > 0 || k > 0));
         if (leader) ptx::umma_commit(&kv_empty[p_gt % kFwdRing]);
         if (leader) ptx::umma_commit(&p_empty[p_gt & 1]);
         if (leader && (p_j == p_n - 1)) ptx::umma_commit(&o_full[p_k & 1]);
@@ -207,30 +191,26 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
     __syncwarp();
   } else {
     const int quarter = warp & 3;
-    const int half = NH == 2 ? (warp - 2) >> 2 : 0;   // NH = 2: which 32 of the 64 score / output columns this thread owns
     const int r = quarter * 32 + lane;  // row inside the tile == TMEM lane
     const uint32_t lane_off = static_cast<uint32_t>(quarter * 32) << 16;
-    constexpr int OC = 64 / NH;         // output columns per thread
     // item epilogue: O / l -> bf16, LSE.  The O buffer is released as soon as it sits in registers.  It runs AFTER the
     // first tile of the following item: by then the last P V of this item has completed (no stall on o_full) and the
-    // tensor core already has the next S tiles to chew on.  NH = 2: the other half's row sum was published at the end of the
-    // item and a step barrier of the following item (or the explicit one after the loop) lies in between.
+    // tensor core already has the next S tiles to chew on.
     auto epilogue = [&](int k, int it, float l, float m_ref) {
       const int qt = nqt - 1 - fdiv(it, fBH), bh = fmodi(it, fBH), b = fdiv(bh, fH), h = fmodi(bh, fH);
-      const uint32_t tm_O = tmem_base + 128 + (k & 1) * 64 + half * OC;
-      if (NH == 2) l += xch_l[((k & 1) * 2 + (half ^ 1)) * 128 + r];
+      const uint32_t tm_O = tmem_base + 128 + (k & 1) * 64;
       ptx::mbar_wait(&o_full[k & 1], (k >> 1) & 1, 20);
       ptx::tc_fence_after();
-      uint32_t v0[32], v1[NH == 1 ? 32 : 1];
+      uint32_t v0[32], v1[32];
       ptx::tmem_ld32(tm_O + lane_off, v0);
-      if constexpr (NH == 1) ptx::tmem_ld32(tm_O + lane_off + 32, v1);
+      ptx::tmem_ld32(tm_O + lane_off + 32, v1);
       ptx::tmem_ld_wait();
       ptx::tc_fence_before();
       ptx::mbar_arrive(&o_free[k & 1]);
       const int t = qt * 128 + r;
       if (t < T) {
         const float inv = (DROP ? dcfg.inv_keep : 1.0f) / l;
-        __nv_bfloat16* o = out + static_cast<long long>(b * T + t) * C + h * HS + half * OC;
+        __nv_bfloat16* o = out + static_cast<long long>(b * T + t) * C + h * HS;
 #pragma unroll
         for (int q = 0; q < 4; ++q) {
           uint4 w;
@@ -240,25 +220,17 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
           w.w = ptx::pack_bf16x2(__uint_as_float(v0[8 * q + 6]) * inv, __uint_as_float(v0[8 * q + 7]) * inv);
           reinterpret_cast<uint4*>(o)[q] = w;
         }
-        if constexpr (NH == 1) {
 #pragma unroll
-          for (int q = 0; q < 4; ++q) {
-            uint4 w;
-            w.x = ptx::pack_bf16x2(__uint_as_float(v1[8 * q + 0]) * inv, __uint_as_float(v1[8 * q + 1]) * inv);
-            w.y = ptx::pack_bf16x2(__uint_as_float(v1[8 * q + 2]) * inv, __uint_as_float(v1[8 * q + 3]) * inv);
-            w.z = ptx::pack_bf16x2(__uint_as_float(v1[8 * q + 4]) * inv, __uint_as_float(v1[8 * q + 5]) * inv);
-            w.w = ptx::pack_bf16x2(__uint_as_float(v1[8 * q + 6]) * inv, __uint_as_float(v1[8 * q + 7]) * inv);
-            reinterpret_cast<uint4*>(o)[4 + q] = w;
-          }
+        for (int q = 0; q < 4; ++q) {
+          uint4 w;
+          w.x = ptx::pack_bf16x2(__uint_as_float(v1[8 * q + 0]) * inv, __uint_as_float(v1[8 * q + 1]) * inv);
+          w.y = ptx::pack_bf16x2(__uint_as_float(v1[8 * q + 2]) * inv, __uint_as_float(v1[8 * q + 3]) * inv);
+          w.z = ptx::pack_bf16x2(__uint_as_float(v1[8 * q + 4]) * inv, __uint_as_float(v1[8 * q + 5]) * inv);
+          w.w = ptx::pack_bf16x2(__uint_as_float(v1[8 * q + 6]) * inv, __uint_as_float(v1[8 * q + 7]) * inv);
+          reinterpret_cast<uint4*>(o)[4 + q] = w;
         }
-        if (half == 0) lse[stat_idx(b, h, t, H, T, seq_shift)] = (m_ref + log2f(l)) * kLn2;
+        lse[stat_idx(b, h, t, H, T, seq_shift)] = (m_ref + log2f(l)) * kLn2;
       }
-    };
-    // one chunk (32 score columns) of a step: class dispatch
-    auto chunk = [&](int cls, uint32_t taddr, float neg_m, float& tmax, float& rowsum, uint32_t* pk, uint32_t drop_rk, int kv0) {
-      if (cls == kFull) fwd_chunk<kFull, DROP>(taddr, lane, neg_m, tmax, rowsum, pk, dcfg, drop_rk, kv0);
-      else if (cls == kDiag) fwd_chunk<kDiag, DROP>(taddr, lane, neg_m, tmax, rowsum, pk, dcfg, drop_rk, kv0);
-      else fwd_chunk<kMasked, DROP>(taddr, lane, neg_m, tmax, rowsum, pk, dcfg, drop_rk, kv0);
     };
     auto chunk_max = [&](int cls, uint32_t taddr) -> float {
       if (cls == kFull) return fwd_chunk_max<kFull>(taddr, lane);
@@ -292,102 +264,48 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
         ptx::mbar_wait(&s_full[bsel], (gt >> 1) & 1, 17);
         ptx::tc_fence_after();
         ATTN_STAMP(1);
-        uint32_t pk[32 / NH];
+        uint32_t pk[32];
         float tmax = -1e30f, rowsum = 0.f;
-        if constexpr (NH == 1) {
-          if (!have_ref && (cls0 != kMasked || cls1 != kMasked)) {
-            have_ref = true;
-            // first tile (with packed short sequences: the first tile of this warp's own sequence): the reference exponent
-            // is its true row max (cheap max-only pass, then the exp pass)
-            tmax = fmaxf(chunk_max(cls0, tm_s), chunk_max(cls1, tm_s + 32));
-            m_ref = tmax * kSl2;
-            fwd_tile<DROP>(tm_s, lane, cls0, cls1, -m_ref, tmax, rowsum, pk, dcfg, drop_rk, j * 64, seq_shift);
-          } else {
-            fwd_tile<DROP>(tm_s, lane, cls0, cls1, -m_ref, tmax, rowsum, pk, dcfg, drop_rk, j * 64, seq_shift);
-            const bool need = tmax * kSl2 - m_ref > kRescaleThreshold;
-            if (__any_sync(0xffffffffu, need)) {
-              // rare: raise the reference, rescale the O accumulator in TMEM, recompute this tile's P
-              const float m_new = need ? tmax * kSl2 : m_ref;
-              const float alpha = ex2(m_ref - m_new);
-              ptx::mbar_wait(&p_empty[(gt - 1) & 1], ((gt - 1) >> 1) & 1, 19);  // every earlier P V product has landed in O
-              ptx::tc_fence_after();
-#pragma unroll
-              for (int c = 0; c < 2; ++c) {
-                uint32_t o[32];
-                ptx::tmem_ld32(tm_O + lane_off + c * 32, o);
-                ptx::tmem_ld_wait();
-#pragma unroll
-                for (int i = 0; i < 32; ++i) o[i] = __float_as_uint(__uint_as_float(o[i]) * alpha);
-                ptx::tmem_st32(tm_O + lane_off + c * 32, o);
-              }
-              ptx::tmem_st_wait();
-              l *= alpha;
-              m_ref = m_new;
-              tmax = -1e30f;
-              rowsum = 0.f;
-              fwd_tile<DROP>(tm_s, lane, cls0, cls1, -m_ref, tmax, rowsum, pk, dcfg, drop_rk, j * 64, seq_shift);
-            }
-          }
+        if (!have_ref && (cls0 != kMasked || cls1 != kMasked)) {
+          have_ref = true;
+          // first tile (with packed short sequences: the first tile of this warp's own sequence): the reference exponent
+          // is its true row max (cheap max-only pass, then the exp pass)
+          tmax = fmaxf(chunk_max(cls0, tm_s), chunk_max(cls1, tm_s + 32));
+          m_ref = tmax * kSl2;
+          fwd_tile<DROP>(tm_s, lane, cls0, cls1, -m_ref, tmax, rowsum, pk, dcfg, drop_rk, j * 64, seq_shift);
         } else {
-          // this thread's chunk: columns [64j + 32 half, +32) of its row.  Every step runs exactly one exchange + named barrier
-          // between the two warps of the quarter (parity-double-buffered slots: a slot is rewritten two steps later, after a
-          // barrier that follows every read of it).
-          const int cls = half == 0 ? cls0 : cls1;
-          const uint32_t tm_c = tm_s + half * 32;
-          const int kv0 = real_col(j * 64 + half * 32, seq_shift);
-          float* xm = xch_max + (bsel * 2) * 128;
-          if (!have_ref && (cls0 != kMasked || cls1 != kMasked)) {
-            have_ref = true;
-            xm[half * 128 + r] = chunk_max(cls, tm_c);
-            ptx::bar_sync(1 + quarter, 64);
-            tmax = fmaxf(xm[half * 128 + r], xm[(half ^ 1) * 128 + r]);
-            m_ref = tmax * kSl2;
-            chunk(cls, tm_c, -m_ref, tmax, rowsum, pk, drop_rk, kv0);
-          } else {
-            chunk(cls, tm_c, -m_ref, tmax, rowsum, pk, drop_rk, kv0);
-            const bool need = tmax * kSl2 - m_ref > kRescaleThreshold;
-            const bool wneed = __any_sync(0xffffffffu, need);
-            xm[half * 128 + r] = tmax;
-            if (lane == 0) xch_flag[(bsel * 4 + quarter) * 2 + half] = wneed ? 1u : 0u;
-            ptx::bar_sync(1 + quarter, 64);
-            if (wneed || xch_flag[(bsel * 4 + quarter) * 2 + (half ^ 1)] != 0u) {
-              // rare: raise the reference of the rows that need it (both halves take the same decision from the same two maxima),
-              // rescale this thread's half of the O accumulator in TMEM, recompute this chunk's P
-              const float tm_row = fmaxf(tmax, xm[(half ^ 1) * 128 + r]);
-              const float m_new = (tm_row * kSl2 - m_ref > kRescaleThreshold) ? tm_row * kSl2 : m_ref;
-              const float alpha = ex2(m_ref - m_new);
-              ptx::mbar_wait(&p_empty[(gt - 1) & 1], ((gt - 1) >> 1) & 1, 19);  // every earlier P V product has landed in O
-              ptx::tc_fence_after();
-              {
-                uint32_t o[32];
-                ptx::tmem_ld32(tm_O + lane_off + half * 32, o);
-                ptx::tmem_ld_wait();
+          fwd_tile<DROP>(tm_s, lane, cls0, cls1, -m_ref, tmax, rowsum, pk, dcfg, drop_rk, j * 64, seq_shift);
+          const bool need = tmax * kSl2 - m_ref > kRescaleThreshold;
+          if (__any_sync(0xffffffffu, need)) {
+            // rare: raise the reference, rescale the O accumulator in TMEM, recompute this tile's P
+            const float m_new = need ? tmax * kSl2 : m_ref;
+            const float alpha = ex2(m_ref - m_new);
+            ptx::mbar_wait(&p_empty[(gt - 1) & 1], ((gt - 1) >> 1) & 1, 19);  // every earlier P V product has landed in O
+            ptx::tc_fence_after();
 #pragma unroll
-                for (int i = 0; i < 32; ++i) o[i] = __float_as_uint(__uint_as_float(o[i]) * alpha);
-                ptx::tmem_st32(tm_O + lane_off + half * 32, o);
-              }
-              ptx::tmem_st_wait();
-              l *= alpha;
-              m_ref = m_new;
-              tmax = -1e30f;
-              rowsum = 0.f;
-              chunk(cls, tm_c, -m_ref, tmax, rowsum, pk, drop_rk, kv0);
+            for (int c = 0; c < 2; ++c) {
+              uint32_t o[32];
+              ptx::tmem_ld32(tm_O + lane_off + c * 32, o);
+              ptx::tmem_ld_wait();
+#pragma unroll
+              for (int i = 0; i < 32; ++i) o[i] = __float_as_uint(__uint_as_float(o[i]) * alpha);
+              ptx::tmem_st32(tm_O + lane_off + c * 32, o);
             }
+            ptx::tmem_st_wait();
+            l *= alpha;
+            m_ref = m_new;
+            tmax = -1e30f;
+            rowsum = 0.f;
+            fwd_tile<DROP>(tm_s, lane, cls0, cls1, -m_ref, tmax, rowsum, pk, dcfg, drop_rk, j * 64, seq_shift);
           }
         }
         l += rowsum;
         ATTN_STAMP(2);
         ATTN_STAMP(3);
         // P (64 key columns = 32 packed words) overwrites the first half of this tile's S buffer; the tensor pipe runs in
-        // issue order, so S_{j+2} cannot overwrite it before P V of this tile has consumed it.  NH = 2: every thread overwrites
-        // only S columns it has consumed itself — half 1 puts its 16 words at columns [32, 48) (the P V MMAs of k-steps 2, 3
-        // read their A operand from there), so no thread's store can run into the other half's (re)loads of its own chunk
-        if constexpr (NH == 1) {
-          ptx::tmem_st16(tm_s, pk);
-          ptx::tmem_st16(tm_s + 16, pk + 16);
-        } else {
-          ptx::tmem_st16(tm_s + half * 32, pk);
-        }
+        // issue order, so S_{j+2} cannot overwrite it before P V of this tile has consumed it
+        ptx::tmem_st16(tm_s, pk);
+        ptx::tmem_st16(tm_s + 16, pk + 16);
         ptx::tmem_st_wait();
         ptx::tc_fence_before();
         ptx::mbar_arrive(&p_full[bsel]);
@@ -403,12 +321,8 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
       pend_it = it;
       pend_l = l;
       pend_m = m_ref;
-      if (NH == 2) xch_l[((item_k & 1) * 2 + half) * 128 + r] = l;
     }
-    if (pend) {
-      if (NH == 2) ptx::bar_sync(1 + quarter, 64);
-      epilogue(pend_k, pend_it, pend_l, pend_m);
-    }
+    if (pend) epilogue(pend_k, pend_it, pend_l, pend_m);
 #undef ATTN_STAMP
   }
   ptx::tc_fence_before();
@@ -1092,13 +1006,9 @@ int attn_fwd(const void* qkv, void* out, float* lse, int B, int T, int H, float 
   if ((rc = encode_tmap_2d(&tmQ, qkv, 2, 3ull * C, static_cast<uint64_t>(B) * T, 3ull * C * 2, 64, 128, true))) return rc;
   if ((rc = encode_tmap_2d(&tmKV, qkv, 2, 3ull * C, static_cast<uint64_t>(B) * T, 3ull * C * 2, 64, 64, true))) return rc;
   static bool done = false;
-  static int nh = 1;   // MEASURED (cfg3, 32 x 12 x 1024): NH = 2 0.124-0.125 ms per layer against 0.120-0.122 ms for NH = 1
   if (!done) {
-    if ((rc = set_smem(attn_fwd_kernel<false, 1>, FwdSmem::TOTAL))) return rc;
-    if ((rc = set_smem(attn_fwd_kernel<true, 1>, FwdSmem::TOTAL))) return rc;
-    if ((rc = set_smem(attn_fwd_kernel<false, 2>, FwdSmem::TOTAL))) return rc;
-    if ((rc = set_smem(attn_fwd_kernel<true, 2>, FwdSmem::TOTAL))) return rc;
-    if (const char* e = getenv("ABCGPT_ATTN_FWD_NH")) nh = e[0] == '2' ? 2 : 1;   // experiments: 2 = eight compute warps per CTA
+    if ((rc = set_smem(attn_fwd_kernel<false>, FwdSmem::TOTAL))) return rc;
+    if ((rc = set_smem(attn_fwd_kernel<true>, FwdSmem::TOTAL))) return rc;
     done = true;
   }
   const int BH = B * H, nitems = ((T + 127) / 128) * BH;
@@ -1106,9 +1016,6 @@ int attn_fwd(const void* qkv, void* out, float* lse, int B, int T, int H, float 
   const int grid = nitems < 2 * sm_count() ? nitems : 2 * sm_count();  // persistent: two CTAs per SM
   long long* CT = g_attn_cta_trace;
   __nv_bfloat16* o = reinterpret_cast<__nv_bfloat16*>(out);
-#define ABCGPT_FWD(D, N)                                                                                                          \
-  launch_k(attn_fwd_kernel<D, N>, dim3(grid), dim3(64 + 128 * N), FwdSmem::TOTAL, stream, tmQ, tmKV, o, lse, T, H, C, BH, nitems, \
-           g_attn_trace, dcfg, CT, seq_shift, fBH, fH)
   // Three CTAs per SM with single-buffered S / O (csrc/attn_fwd3.cu) for sequences of >= 256 positions: 0.110 vs 0.120 ms per
   // layer at cfg3, 0.0196 vs 0.0205 ms at cfg2; packed short sequences (T = 32: 0.279 vs 0.273 ms at the cfg4 character level)
   // and the tracing tools keep the two-CTA kernel.  ABCGPT_ATTN_FWD3=0 selects the two-CTA kernel everywhere (A/B runs).
@@ -1118,11 +1025,12 @@ int attn_fwd(const void* qkv, void* out, float* lse, int B, int T, int H, float 
   }();
   if (three_ctas && seq_shift == kNoPack && T >= 256 && g_attn_trace == nullptr && CT == nullptr)
     return attn_fwd3(tmQ, tmKV, out, lse, T, H, C, BH, nitems, dcfg, seq_shift, fBH.d, fBH.m, fH.d, fH.m, stream);
-  // the step traces (abcgpt_debug_attn_trace) instrument the four-warp form
-  const bool two = nh == 2 && g_attn_trace == nullptr;
-  if (dcfg.thr16 == 0) { if (two) ABCGPT_FWD(false, 2); else ABCGPT_FWD(false, 1); }
-  else { if (two) ABCGPT_FWD(true, 2); else ABCGPT_FWD(true, 1); }
-#undef ABCGPT_FWD
+  if (dcfg.thr16 == 0)
+    launch_k(attn_fwd_kernel<false>, dim3(grid), dim3(kThreads), FwdSmem::TOTAL, stream, tmQ, tmKV, o, lse, T, H, C, BH, nitems, g_attn_trace,
+             dcfg, CT, seq_shift, fBH, fH);
+  else
+    launch_k(attn_fwd_kernel<true>, dim3(grid), dim3(kThreads), FwdSmem::TOTAL, stream, tmQ, tmKV, o, lse, T, H, C, BH, nitems, g_attn_trace,
+             dcfg, CT, seq_shift, fBH, fH);
   return launch_status("attn_fwd_kernel");
 }
 

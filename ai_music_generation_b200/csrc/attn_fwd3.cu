@@ -17,32 +17,27 @@
 // Everything a softmax thread computes is the code of the two-CTA kernel (csrc/attn_helpers.cuh), including dropout, packed
 // short sequences and the lazy in-TMEM rescale.
 // MEASURED (cfg3: 32 x 12 heads x 1024, per layer): 0.110 ms against 0.120 ms for the two-CTA kernel (465 vs 430 TFLOP/s of causal
-// FLOPs) — the first change of the round that moved this kernel; FOUR CTAs per SM (Q single-buffered too, 80 registers with a few
-// spills; ABCGPT_ATTN_FWD_CTAS=4) fall back to 0.118 ms.
+// FLOPs) — the first change of the round that moved this kernel.
 #include "attn_helpers.cuh"
-#include <stdlib.h>
 
 namespace abcgpt {
 namespace {
 
 constexpr int kRing3 = 2;
-// NCTA = resident CTAs per SM this instantiation is sized for: 3 (Q double-buffered, <= 112 registers) or 4 (Q single-buffered:
-// 48 KB of shared memory per CTA, <= 80 registers)
-template <int NCTA>
 struct Fwd3Smem {
-  static constexpr int QB = NCTA >= 4 ? 1 : 2;       // Q buffers
+  static constexpr int QB = 2;                       // Q buffers
   static constexpr int Q = 0;                        // QB items x (128 x 64 bf16)
   static constexpr int KV = QB * 16384;              // kRing3 stages x (K 64x64 | V 64x64)
   static constexpr int BAR = KV + kRing3 * 16384;
   static constexpr int TOTAL = BAR + 256 + 1024;
 };
 
-template <bool DROP, int NCTA>
-__global__ void __launch_bounds__(kThreads, NCTA)
+template <bool DROP>
+__global__ void __launch_bounds__(kThreads, 3)
 attn_fwd3_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmKV,
                  __nv_bfloat16* __restrict__ out, float* __restrict__ lse, int T, int H, int C, int BH, int nitems,
                  const DropCfg dcfg, int seq_shift, const FastDiv fBH, const FastDiv fH) {
-  using SM = Fwd3Smem<NCTA>;
+  using SM = Fwd3Smem;
   constexpr int QB = SM::QB;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
@@ -269,23 +264,19 @@ int attn_fwd3(const CUtensorMap& tmQ, const CUtensorMap& tmKV, void* out, float*
               const DropCfg& dcfg, int seq_shift, uint32_t fBH_d, uint32_t fBH_m, uint32_t fH_d, uint32_t fH_m, cudaStream_t stream) {
   const FastDiv fBH{fBH_d, fBH_m}, fH{fH_d, fH_m};   // FastDiv lives in each translation unit's anonymous namespace
   static bool done = false;
-  static int ncta = 3;
   if (!done) {
-    ABCGPT_CUDA(cudaFuncSetAttribute(attn_fwd3_kernel<false, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, Fwd3Smem<3>::TOTAL));
-    ABCGPT_CUDA(cudaFuncSetAttribute(attn_fwd3_kernel<true, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, Fwd3Smem<3>::TOTAL));
-    ABCGPT_CUDA(cudaFuncSetAttribute(attn_fwd3_kernel<false, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, Fwd3Smem<4>::TOTAL));
-    ABCGPT_CUDA(cudaFuncSetAttribute(attn_fwd3_kernel<true, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, Fwd3Smem<4>::TOTAL));
-    if (const char* e = getenv("ABCGPT_ATTN_FWD_CTAS")) ncta = e[0] == '4' ? 4 : 3;
+    ABCGPT_CUDA(cudaFuncSetAttribute(attn_fwd3_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, Fwd3Smem::TOTAL));
+    ABCGPT_CUDA(cudaFuncSetAttribute(attn_fwd3_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Fwd3Smem::TOTAL));
     done = true;
   }
-  const int grid = nitems < ncta * sm_count() ? nitems : ncta * sm_count();  // persistent: ncta CTAs per SM
+  const int grid = nitems < 3 * sm_count() ? nitems : 3 * sm_count();  // persistent: three CTAs per SM
   __nv_bfloat16* o = reinterpret_cast<__nv_bfloat16*>(out);
-#define ABCGPT_FWD3(D, N)                                                                                                        \
-  launch_k(attn_fwd3_kernel<D, N>, dim3(grid), dim3(kThreads), Fwd3Smem<N>::TOTAL, stream, tmQ, tmKV, o, lse, T, H, C, BH, nitems, \
-           dcfg, seq_shift, fBH, fH)
-  if (ncta == 4) { if (dcfg.thr16 == 0) ABCGPT_FWD3(false, 4); else ABCGPT_FWD3(true, 4); }
-  else { if (dcfg.thr16 == 0) ABCGPT_FWD3(false, 3); else ABCGPT_FWD3(true, 3); }
-#undef ABCGPT_FWD3
+  if (dcfg.thr16 == 0)
+    launch_k(attn_fwd3_kernel<false>, dim3(grid), dim3(kThreads), Fwd3Smem::TOTAL, stream, tmQ, tmKV, o, lse, T, H, C, BH, nitems, dcfg,
+             seq_shift, fBH, fH);
+  else
+    launch_k(attn_fwd3_kernel<true>, dim3(grid), dim3(kThreads), Fwd3Smem::TOTAL, stream, tmQ, tmKV, o, lse, T, H, C, BH, nitems, dcfg,
+             seq_shift, fBH, fH);
   return launch_status("attn_fwd3_kernel");
 }
 

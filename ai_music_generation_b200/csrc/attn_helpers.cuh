@@ -41,53 +41,6 @@ __device__ __forceinline__ float ex2(float x) {
   return y;
 }
 
-// 2^x on the FMA pipe (two lanes): Cody-Waite split x = n + f, n = rint(x) through the 1.5 * 2^23 magic add, f in [-0.5, 0.5],
-// 2^f by a cubic fitted for minimal RELATIVE error (7.5e-5, 26 times below bf16's half ulp; the probabilities are rounded to
-// bf16 right after), 2^n by an integer add into the exponent field.  Why: MUFU.EX2 is the bound of all three attention kernels
-// and ONE warp can issue it only every ~16.7 cycles (tools/mufu_bench.py: 1.9 / 2.9 / 3.9 results per clock and scheduler with
-// 1 / 2 / 4 warps) while the same warp's FMA issue slots sit idle in between, so half of the exponentials of every chunk are
-// evaluated here instead (kPolyExp: every second column pair).  Valid for x in [-126, 127]; smaller x is clamped (result ~0).
-// MEASURED (cfg3): parity-green, XU pipe 47 % -> 21 %, and NO change in kernel time (forward 0.118 -> 0.123 ms, backward 0.295 ->
-// 0.302 ms per layer): the ncu source view of the same run shows the compute warps 36 % of their time in the wait for the next
-// score tile, i.e. the step pipeline (three TMEM score buffers, MMA -> softmax -> MMA round trip) is the limit, not the MUFU rate.
-// Off; kept for the day the pipeline is deeper.
-#ifdef ABCGPT_POLY_EXP
-constexpr bool kPolyExp = true;
-constexpr int kPolyEvery = ABCGPT_POLY_EXP;   // every kPolyEvery-th column pair of a chunk goes to the FMA pipe (2 = half of them)
-#else
-constexpr bool kPolyExp = false;
-constexpr int kPolyEvery = 2;
-#endif
-__device__ __forceinline__ float2 ex2_poly2(float2 x) {
-  x.x = fmaxf(x.x, -126.f);
-  x.y = fmaxf(x.y, -126.f);
-  const float2 t = __fadd2_rn(x, make_float2(12582912.f, 12582912.f));
-  const float2 n = __fadd2_rn(t, make_float2(-12582912.f, -12582912.f));
-  const float2 f = __ffma2_rn(n, make_float2(-1.f, -1.f), x);
-  float2 p = __ffma2_rn(f, make_float2(0.0551716685f, 0.0551716685f), make_float2(0.2426111251f, 0.2426111251f));
-  p = __ffma2_rn(p, f, make_float2(0.6932609677f, 0.6932609677f));
-  p = __ffma2_rn(p, f, make_float2(0.9999280572f, 0.9999280572f));
-  return make_float2(__int_as_float(__float_as_int(p.x) + (__float_as_int(t.x) << 23)),
-                     __int_as_float(__float_as_int(p.y) + (__float_as_int(t.y) << 23)));
-}
-// exponentials of column pair i of a chunk: MUFU for even pairs, FMA pipe for odd ones
-__device__ __forceinline__ float2 ex2_pair(float2 t, int i) {
-  if (kPolyExp && (i % kPolyEvery) == kPolyEvery - 1) return ex2_poly2(t);
-  return make_float2(ex2(t.x), ex2(t.y));
-}
-
-// write 32 consecutive bf16 columns (16 packed words) of one row into a [rows x 64] K-major SWIZZLE_128B slab
-__device__ __forceinline__ void st_slab32(uint32_t slab_addr, int row, int c32, const uint32_t* pk) {
-  const uint32_t base = slab_addr + row * 128;
-#pragma unroll
-  for (int q = 0; q < 4; ++q) {
-    const uint32_t addr = base + (((c32 * 4 + q) ^ (row & 7)) << 4);
-    asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(pk[4 * q]), "r"(pk[4 * q + 1]),
-                 "r"(pk[4 * q + 2]), "r"(pk[4 * q + 3])
-                 : "memory");
-  }
-}
-
 // K-major SW128 operand: rows x 64 bf16 slab, 16-column K step k16
 __device__ __forceinline__ uint64_t desc_k(uint32_t slab_addr, int k16) {
   return ptx::umma_smem_desc(slab_addr + k16 * 32, 0, 1024);
@@ -131,42 +84,6 @@ __device__ __forceinline__ float fwd_chunk_max(uint32_t taddr, int lane) {
   return fmaxf(fmaxf(m0, m1), fmaxf(m2, m3));
 }
 
-// forward pass 2: p = 2^(s*sl2 - m), bf16 P into the swizzled slab, returns the fp32 row-sum contribution
-template <int MODE>
-__device__ __forceinline__ float fwd_chunk_exp(uint32_t taddr, int lane, float neg_m, uint32_t slab, int r, int c32) {
-  uint32_t pk[16];
-  if (MODE == kMasked) {
-#pragma unroll
-    for (int i = 0; i < 16; ++i) pk[i] = 0u;
-    st_slab32(slab, r, c32, pk);
-    return 0.f;
-  }
-  uint32_t v[32];
-  ptx::tmem_ld32(taddr, v);
-  ptx::tmem_ld_wait();
-  const float2 sl = make_float2(kSl2, kSl2), nm = make_float2(neg_m, neg_m);
-  float2 acc0 = make_float2(0.f, 0.f), acc1 = make_float2(0.f, 0.f);
-#pragma unroll
-  for (int i = 0; i < 16; i += 2) {
-    const float2 t0 = __ffma2_rn(f2(v[2 * i], v[2 * i + 1]), sl, nm);
-    const float2 t1 = __ffma2_rn(f2(v[2 * i + 2], v[2 * i + 3]), sl, nm);
-    float2 p0 = make_float2(ex2(t0.x), ex2(t0.y));
-    float2 p1 = make_float2(ex2(t1.x), ex2(t1.y));
-    if (MODE == kDiag) {
-      p0.x = (2 * i <= lane) ? p0.x : 0.f;
-      p0.y = (2 * i + 1 <= lane) ? p0.y : 0.f;
-      p1.x = (2 * i + 2 <= lane) ? p1.x : 0.f;
-      p1.y = (2 * i + 3 <= lane) ? p1.y : 0.f;
-    }
-    acc0 = __fadd2_rn(acc0, p0);
-    acc1 = __fadd2_rn(acc1, p1);
-    pk[i] = ptx::pack_bf16x2(p0.x, p0.y);
-    pk[i + 1] = ptx::pack_bf16x2(p1.x, p1.y);
-  }
-  st_slab32(slab, r, c32, pk);
-  return (acc0.x + acc0.y) + (acc1.x + acc1.y);
-}
-
 // prmt.b32 with a selector whose nibbles have bit 3 set replicates the SIGN of the chosen byte: 0xBB99 turns bits 15 / 31
 // into a bf16x2 AND mask, 0x9999 / 0xBBBB into fp32 masks for the even / odd column of a pair (csrc/dropout.cuh)
 __device__ __forceinline__ uint32_t prmt_sign(uint32_t x, uint32_t sel) {
@@ -196,7 +113,7 @@ __device__ __forceinline__ void dq_chunk(uint32_t taddr_s, uint32_t taddr_dp, in
 #pragma unroll
   for (int i = 0; i < 16; ++i) {
     const float2 t = __ffma2_rn(f2(s[2 * i], s[2 * i + 1]), sl, nl);
-    const float2 p = ex2_pair(t, i);
+    const float2 p = make_float2(ex2(t.x), ex2(t.y));
     float2 dpe = f2(dp[2 * i], dp[2 * i + 1]);
     if (DROP) {
       const uint32_t u = attn_drop_signs(attn_drop_fold(drop_s + static_cast<uint32_t>(i) * kDropWeyl, drop_b), dcfg.k15);
@@ -243,7 +160,7 @@ __device__ __forceinline__ void dkv_chunk(uint32_t taddr_s, uint32_t taddr_dp, u
       const float2 nl = h == 0 ? make_float2(l4.x, l4.y) : make_float2(l4.z, l4.w);
       const float2 nd = h == 0 ? make_float2(d4.x, d4.y) : make_float2(d4.z, d4.w);
       const float2 t = __ffma2_rn(f2(s[2 * i], s[2 * i + 1]), sl, nl);
-      float2 p = ex2_pair(t, i);
+      float2 p = make_float2(ex2(t.x), ex2(t.y));
       float2 dpe = f2(dp[2 * i], dp[2 * i + 1]);
       float2 pd = p;  // the (dropped) probabilities that multiply dO in dV
       if (DROP) {
@@ -320,8 +237,8 @@ __device__ __forceinline__ void fwd_chunk(uint32_t taddr, int lane, float neg_m,
     m1 = fmaxf(m1, fmaxf(s2, s3));
     const float2 t0 = __ffma2_rn(make_float2(s0, s1), sl, nm);
     const float2 t1 = __ffma2_rn(make_float2(s2, s3), sl, nm);
-    float2 p0 = ex2_pair(t0, i);  // masked entries: 2^(-huge) = 0
-    float2 p1 = ex2_pair(t1, i + 1);
+    float2 p0 = make_float2(ex2(t0.x), ex2(t0.y));  // masked entries: 2^(-huge) = 0
+    float2 p1 = make_float2(ex2(t1.x), ex2(t1.y));
     acc0 = __fadd2_rn(acc0, p0);
     acc1 = __fadd2_rn(acc1, p1);
     pk[i] = ptx::pack_bf16x2(p0.x, p0.y);

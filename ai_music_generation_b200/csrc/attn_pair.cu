@@ -25,36 +25,29 @@
 // single-CTA kernels (csrc/attn_helpers.cuh); a tile that lies entirely above the diagonal for one CTA of the pair (the first
 // two query steps of the upper key tile, the last two key steps of the lower query tile) takes the "masked" chunk class there.
 #include "attn_helpers.cuh"
-#include <stdlib.h>
 
 namespace abcgpt {
 namespace {
 
 constexpr int kSBuf = 3;          // S/dP score buffers in TMEM (as in csrc/attn.cu)
 constexpr int kRing = 6;          // streamed tiles in flight
-// Thread layout: warp 0 TMA, warp 1 score MMAs, warps 2..17 compute, warp 18 accumulating MMAs.
-// SIXTEEN compute warps (four per scheduler): the single-CTA kernels' two groups of four (two warps per scheduler, each
-// grinding through 64 columns of its row per step) ran at ~4 cycles per instruction — a dependent chain per warp with nothing
-// to switch to — and sat at roughly half of the MUFU rate that bounds these kernels (step traces: ~1100-1300 cycles of compute
-// per 128x64 step against 512 cycles of ex2).  Here a step belongs to one of two step groups (steps alternate between them, as
-// before) and each step group has TWO column halves: a thread owns one row and 32 of the 64 columns of every other step, so
-// twice as many independent instruction streams share each scheduler and the per-thread register footprint halves.
-// MEASURED (cfg3, 32 x 12 heads x 1024): NCH = 2 runs the backward in 0.373 ms per layer against 0.303 ms for NCH = 1 — the
-// kernels are NOT latency-bound: with eight compute warps the steady state already runs at 80-90 % of the MUFU (ex2) rate, and
-// the extra warps only add per-step barrier traffic.  NCH = 1 (eight compute warps, a thread owns a whole row of a step) is the
-// default; the template parameter stays for experiments.
-// NG = number of STEP GROUPS (dQ kernel): group g owns the steps gs with gs % NG == g.  NG = 2 alternates two groups over the
-// three score buffers (the issuer runs one step ahead); NG = 3 gives every score buffer its own group — a third independent
-// instruction stream per SM for the latency gaps of the other two (the forward gained 8 % from a third resident CTA for the
-// same reason, csrc/attn_fwd3.cu).  MEASURED: dQ kernel 0.125 -> 0.118 ms per layer at cfg3 — each group now idles ~60 % of its
-// cycle (3 x 1050 cycles per own step against ~1250 of arithmetic), i.e. the steps are not fed faster than one per ~1050 cycles
-// per SM whatever the number of groups: the score / accumulate MMA chain and its operand re-reads (Q and dO, 4 KB each per
-// MMA, are the shared-memory-bound A operands of eight of the twelve MMAs of a step) are the next thing to look at.
-template <int NCH, int NG = 2> struct PairCfg {
-  static constexpr int kCompWarps = 4 * NG * NCH;
+// Thread layout: warp 0 TMA, warp 1 score MMAs, warps 2 .. 4 NG + 1 compute, warp 4 NG + 2 accumulating MMAs.  The compute
+// warps form NG STEP GROUPS of four (one warp per tensor-memory lane quarter): group g owns the steps gs with gs % NG == g, and a
+// thread owns one row and all 64 columns of each of its steps.  The dK/dV kernel alternates two groups over the three score
+// buffers (the issuer runs one step ahead).  The dQ kernel gives every score buffer its own group: a third independent
+// instruction stream per SM for the latency gaps of the other two (the forward gains from a third resident CTA for the same
+// reason, csrc/attn_fwd3.cu).  More warps per step do not pay: with eight compute warps the steady state already runs at
+// 80-90 % of the MUFU (ex2) rate, and splitting a step's columns over more warps only adds per-step barrier traffic.  In the dQ
+// kernel each group idles ~60 % of its cycle (3 x 1050 cycles per own step against ~1250 of arithmetic): the score / accumulate
+// MMA chain and its operand re-reads (Q and dO, 4 KB each per MMA, are the shared-memory-bound A operands of eight of the
+// twelve MMAs of a step) are the next thing to look at.
+template <int NG> struct PairCfg {
+  static constexpr int kCompWarps = 4 * NG;
   static constexpr int kAccWarp = 2 + kCompWarps;
-  static constexpr int kThreads = (kAccWarp + 1) * 32;   // 352 / 608; NG = 3: 480
+  static constexpr int kThreads = (kAccWarp + 1) * 32;
 };
+using DkvCfg = PairCfg<2>;   // 352 threads
+using DqCfg = PairCfg<3>;    // 480 threads
 
 // static schedule over PAIR items: pair c of G walks items c, 2G-1-c, 2G+c, ... (heaviest first, boustrophedon)
 __device__ __forceinline__ int sched_pair_item(int k, int nitems) {
@@ -84,8 +77,8 @@ struct Dkv2Smem {
   static constexpr int TOTAL = BAR + 512 + 1024;
 };
 
-template <bool DROP, int NCH>
-__global__ void __launch_bounds__(PairCfg<NCH>::kThreads, 1)
+template <bool DROP>
+__global__ void __launch_bounds__(DkvCfg::kThreads, 1)
 attn_bwd_dkv2_kernel(const __grid_constant__ CUtensorMap tmKV128, const __grid_constant__ CUtensorMap tmQ32,
                      const __grid_constant__ CUtensorMap tmDO32, const __grid_constant__ CUtensorMap tmQc,
                      const __grid_constant__ CUtensorMap tmDOc, const float* __restrict__ lse, const float* __restrict__ delta,
@@ -129,10 +122,10 @@ attn_bwd_dkv2_kernel(const __grid_constant__ CUtensorMap tmKV128, const __grid_c
     for (int s = 0; s < kSBuf; ++s) {
       ptx::mbar_init(&s_full[s], 1);
       ptx::mbar_init(&s_free[s], 1);
-      ptx::mbar_init(&pds_full[s], 2 * 4 * NCH);
+      ptx::mbar_init(&pds_full[s], 2 * 4);
     }
     ptx::mbar_init(acc_full, 1);
-    ptx::mbar_init(acc_free, 2 * PairCfg<NCH>::kCompWarps);
+    ptx::mbar_init(acc_free, 2 * DkvCfg::kCompWarps);
     ptx::fence_mbar_init();
   }
   if (warp == 1) {
@@ -213,7 +206,7 @@ attn_bwd_dkv2_kernel(const __grid_constant__ CUtensorMap tmKV128, const __grid_c
       }
     }
     __syncwarp();
-  } else if (warp == PairCfg<NCH>::kAccWarp) {
+  } else if (warp == DkvCfg::kAccWarp) {
     // ---- accumulating MMAs (leader CTA): dV += P^T_n dO_n, dK += dS^T_n Q_n
     if (leader_cta) {
       const bool leader = ptx::elect_one();
@@ -247,23 +240,22 @@ attn_bwd_dkv2_kernel(const __grid_constant__ CUtensorMap tmKV128, const __grid_c
     }
     __syncwarp();
   } else {
-    const int cw = warp - 2;                // 0 .. 8 NCH - 1
-    const int sg = cw / (4 * NCH);          // step group: owns the steps of parity sg
-    const int ch = (cw >> 2) & (NCH - 1);   // NCH = 2: column half of every own step (query columns [32 ch, 32 ch + 32) of the 64)
+    const int cw = warp - 2;                // 0 .. 7
+    const int sg = cw / 4;                  // step group: owns the steps of parity sg
     const int quarter = warp & 3;           // TMEM lane quarter this warp may access
     const int r = quarter * 32 + lane;      // key row inside this CTA's tile
-    const int tid = (cw % (4 * NCH)) * 32 + lane;   // 0 .. 128 NCH - 1 within the step group
+    const int tid = (cw % 4) * 32 + lane;   // 0 .. 127 within the step group
     const uint32_t lane_off = static_cast<uint32_t>(quarter * 32) << 16;
-    // per-step column statistics: threads 0..63 of the step group stage -lse*log2e, 64..127 -delta*scale, 128..191 the dropout
-    // row keys of the step's 64 queries; the RAW value of the next own step is loaded one step ahead
-    const int stat_role = tid >> 6;         // 0: lse, 1: delta (, 2: dropout row keys when NCH = 2; with NCH = 1 role 0 does both)
+    // per-step column statistics: threads 0..63 of the step group stage -lse*log2e and the dropout row keys, 64..127
+    // -delta*scale, of the step's 64 queries; the RAW value of the next own step is loaded one step ahead
+    const int stat_role = tid >> 6;         // 0: lse and dropout row keys, 1: delta
     const float* stat_src = stat_role == 0 ? lse : delta;
     const float stat_coef = stat_role == 0 ? -kLog2e : -kScale;
     int ls_it = -2, ls_q = 0;
     const float* ls_row = stat_src;
     auto load_stat = [&](int it, int n) {
       float v = 0.f;
-      if (it >= 0 && stat_role < 2) {
+      if (it >= 0) {
         if (it != ls_it) {
           int p_, bh_;
           fdivmod(it, fBH, p_, bh_);
@@ -276,7 +268,7 @@ attn_bwd_dkv2_kernel(const __grid_constant__ CUtensorMap tmKV128, const __grid_c
       }
       return v;
     };
-    // item epilogue: step group 0 writes dV, step group 1 dK; each thread 64 / NCH columns of its key row
+    // item epilogue: step group 0 writes dV, step group 1 dK; each thread the 64 columns of its key row
     auto epilogue = [&](int k) {
       const int it = sched_pair_item(k, nitems);
       int p_, bh_, b, h;
@@ -285,18 +277,17 @@ attn_bwd_dkv2_kernel(const __grid_constant__ CUtensorMap tmKV128, const __grid_c
       const int kv_t = (2 * p_ + rank) * 128 + r;
       ptx::mbar_wait(acc_full, k & 1, 67);
       ptx::tc_fence_after();
-      constexpr int NV = 2 / NCH;   // 32-column loads per thread
-      uint32_t v[NV][32];
+      uint32_t v[2][32];
 #pragma unroll
-      for (int c = 0; c < NV; ++c) ptx::tmem_ld32((sg == 0 ? tm_dV : tm_dK) + lane_off + (ch + c) * 32, v[c]);
+      for (int c = 0; c < 2; ++c) ptx::tmem_ld32((sg == 0 ? tm_dV : tm_dK) + lane_off + c * 32, v[c]);
       ptx::tmem_ld_wait();
       ptx::tc_fence_before();
       warp_arrive_leader(acc_free, lane);
       if (kv_t < T) {
         const float sc = (DROP && sg == 0) ? dcfg.inv_keep : 1.0f;  // dV = (P o mask)^T dO / (1-p)
-        __nv_bfloat16* o = dqkv + static_cast<long long>(b * T + kv_t) * (3 * C) + (sg == 0 ? 2 * C : C) + h * HS + ch * 32;
+        __nv_bfloat16* o = dqkv + static_cast<long long>(b * T + kv_t) * (3 * C) + (sg == 0 ? 2 * C : C) + h * HS;
 #pragma unroll
-        for (int c = 0; c < NV; ++c)
+        for (int c = 0; c < 2; ++c)
 #pragma unroll
           for (int q = 0; q < 4; ++q) {
             uint4 w;
@@ -337,16 +328,16 @@ attn_bwd_dkv2_kernel(const __grid_constant__ CUtensorMap tmKV128, const __grid_c
       const int q0 = (4 * p + c_n) * 64;
       const int gs = c_base + c_n;
       float* st_lse = stat + (sg * 2 + (use & 1)) * 192;
-      if (stat_role < 2) st_lse[tid] = raw_cur * stat_coef;
-      if (DROP && stat_role == (NCH == 2 ? 2 : 0))
+      st_lse[tid] = raw_cur * stat_coef;
+      if (DROP && stat_role == 0)
         st_lse[128 + (tid & 63)] = __uint_as_float(drop_row_key(dcfg.key, static_cast<uint32_t>(stat_idx(hb, hh, q0 + (tid & 63), H, T, seq_shift))));
       raw_cur = load_stat(a_it, a_n);  // next own step: consumed at the top of the next iteration
-      ptx::bar_sync(1 + sg, 128 * NCH);
+      ptx::bar_sync(1 + sg, 128);
       ptx::mbar_wait(&s_full[gs % kSBuf], (gs / kSBuf) & 1, 68);
       ptx::tc_fence_after();
       const uint32_t tbuf = tmem_base + lane_off + (gs % kSBuf) * 128;
 #pragma unroll
-      for (int c = ch; c < 2; c += NCH) {
+      for (int c = 0; c < 2; ++c) {
         const int c0 = q0 + c * 32;
         const uint32_t ta_s = tbuf + c * 32, ta_dp = ta_s + 64;
         const uint32_t l2 = ptx::smem_u32(st_lse) + c * 128, d8 = l2 + 256, rkeys = l2 + 512;
@@ -355,8 +346,8 @@ attn_bwd_dkv2_kernel(const __grid_constant__ CUtensorMap tmKV128, const __grid_c
         else if (c0 > r0 && c0 + 31 < T) dkv_chunk<kFull, DROP>(ta_s, ta_dp, l2, d8, c0, kv_t, T, pk_p, pk_ds, dcfg, rkeys, kv_t);
         else dkv_chunk<kDiag, DROP>(ta_s, ta_dp, l2, d8, c0, kv_t, T, pk_p, pk_ds, dcfg, rkeys, kv_t);
         // P^T / dS^T of column half c (16 packed words each) go over the score columns that were just consumed: S^T columns
-        // [32 c, 32 c + 16) and dP^T columns [64 + 32 c, ...) — never into the other half's inputs (with NCH = 2 those belong to
-        // threads that run independently).  The A operand of the accumulating MMAs is two runs of 16 words 32 columns apart.
+        // [32 c, 32 c + 16) and dP^T columns [64 + 32 c, ...) — never into the other half's inputs.  The A operand of the
+        // accumulating MMAs is two runs of 16 words 32 columns apart.
         ptx::tmem_st16(tbuf + c * 32, pk_p);
         ptx::tmem_st16(tbuf + 64 + c * 32, pk_ds);
       }
@@ -387,8 +378,8 @@ struct Dq2Smem {
   static constexpr int TOTAL = BAR + 512 + 1024;
 };
 
-template <bool DROP, int NCH, int NG>
-__global__ void __launch_bounds__(PairCfg<NCH, NG>::kThreads, 1)
+template <bool DROP>
+__global__ void __launch_bounds__(DqCfg::kThreads, 1)
 attn_bwd_dq2_kernel(const __grid_constant__ CUtensorMap tmQ128, const __grid_constant__ CUtensorMap tmDO128,
                     const __grid_constant__ CUtensorMap tmKV32, const __grid_constant__ CUtensorMap tmKc,
                     const float* __restrict__ lse, const float* __restrict__ delta, __nv_bfloat16* __restrict__ dqkv, int T,
@@ -422,7 +413,7 @@ attn_bwd_dq2_kernel(const __grid_constant__ CUtensorMap tmQ128, const __grid_con
       ptx::mbar_init(&qdo_full[s], 1);
       ptx::mbar_init(&qdo_empty[s], 1);
       ptx::mbar_init(&acc_full[s], 1);
-      ptx::mbar_init(&acc_free[s], 2 * PairCfg<NCH, NG>::kCompWarps);
+      ptx::mbar_init(&acc_free[s], 2 * DqCfg::kCompWarps);
     }
     for (int s = 0; s < kRing; ++s) {
       ptx::mbar_init(&kv_full[s], 1);
@@ -431,7 +422,7 @@ attn_bwd_dq2_kernel(const __grid_constant__ CUtensorMap tmQ128, const __grid_con
     for (int s = 0; s < kSBuf; ++s) {
       ptx::mbar_init(&s_full[s], 1);
       ptx::mbar_init(&s_free[s], 1);
-      ptx::mbar_init(&ds_full[s], 2 * 4 * NCH);
+      ptx::mbar_init(&ds_full[s], 2 * 4);
     }
     ptx::fence_mbar_init();
   }
@@ -516,7 +507,7 @@ attn_bwd_dq2_kernel(const __grid_constant__ CUtensorMap tmQ128, const __grid_con
       }
     }
     __syncwarp();
-  } else if (warp == PairCfg<NCH, NG>::kAccWarp) {
+  } else if (warp == DqCfg::kAccWarp) {
     // ---- accumulating MMAs (leader CTA): dQ += dS_j K_j (accumulator double-buffered by item parity)
     if (leader_cta) {
       const bool leader = ptx::elect_one();
@@ -548,9 +539,8 @@ attn_bwd_dq2_kernel(const __grid_constant__ CUtensorMap tmQ128, const __grid_con
     }
     __syncwarp();
   } else {
-    const int cw = warp - 2;                // 0 .. 8 NCH - 1
-    const int sg = cw / (4 * NCH);          // step group: owns the steps gs with gs % NG == sg
-    const int ch = (cw >> 2) & (NCH - 1);   // NCH = 2: column half of every own step (key columns [32 ch, 32 ch + 32) of the 64)
+    const int cw = warp - 2;                // 0 .. 11
+    const int sg = cw / 4;                  // step group: owns the steps gs with gs % 3 == sg
     const int quarter = warp & 3;
     const int r = quarter * 32 + lane;
     const uint32_t lane_off = static_cast<uint32_t>(quarter * 32) << 16;
@@ -568,7 +558,8 @@ attn_bwd_dq2_kernel(const __grid_constant__ CUtensorMap tmQ128, const __grid_con
         raw_d = __ldg(delta + idx);
       }
     };
-    // item epilogue: thread writes columns [32 sg + 16 ch, + 32 / NCH) of its row of this CTA's dQ tile
+    // item epilogue: each step group writes 16-column granules of its row of this CTA's dQ tile: group 0 granules 0 and 1,
+    // groups 1 and 2 one each
     auto epilogue = [&](int k) {
       const int it = sched_pair_item(k, nitems);
       int pr, bh, b, h;
@@ -576,16 +567,13 @@ attn_bwd_dq2_kernel(const __grid_constant__ CUtensorMap tmQ128, const __grid_con
       fdivmod(bh, fH, b, h);
       const int qt = 2 * (npt - 1 - pr) + rank;
       const int t = qt * 128 + r;
-      // 16-column granules of the 64 dQ columns: NG = 2: group sg takes granules [2 sg + ch, + 2 / NCH); NG = 3: group 0 takes
-      // granules 0 and 1, groups 1 and 2 one each
-      const int colq = NG == 3 ? (sg == 0 ? 0 : sg + 1) : 2 * sg + ch;
-      const int nq = NG == 3 ? (sg == 0 ? 2 : 1) : 2 / NCH;
+      const int colq = sg == 0 ? 0 : sg + 1;   // first granule
+      const int nq = sg == 0 ? 2 : 1;          // granules
       ptx::mbar_wait(&acc_full[k & 1], (k >> 1) & 1, 77);
       ptx::tc_fence_after();
-      constexpr int NQ = NG == 3 ? 2 : 2 / NCH;   // 16-column loads per thread (at most)
-      uint32_t v[16 * NQ];
+      uint32_t v[32];
 #pragma unroll
-      for (int c = 0; c < NQ; ++c)
+      for (int c = 0; c < 2; ++c)
         if (c < nq) ptx::tmem_ld16(tm_dQ + (k & 1) * 64 + lane_off + (colq + c) * 16, *reinterpret_cast<uint32_t(*)[16]>(v + 16 * c));
       ptx::tmem_ld_wait();
       ptx::tc_fence_before();
@@ -593,7 +581,7 @@ attn_bwd_dq2_kernel(const __grid_constant__ CUtensorMap tmQ128, const __grid_con
       if (t < T) {
         __nv_bfloat16* o = dqkv + static_cast<long long>(b * T + t) * (3 * C) + h * HS + colq * 16;
 #pragma unroll
-        for (int q = 0; q < 2 * NQ; ++q) {
+        for (int q = 0; q < 4; ++q) {
           if (q >= 2 * nq) break;
           uint4 w;
           w.x = ptx::pack_bf16x2(__uint_as_float(v[8 * q + 0]), __uint_as_float(v[8 * q + 1]));
@@ -604,7 +592,7 @@ attn_bwd_dq2_kernel(const __grid_constant__ CUtensorMap tmQ128, const __grid_con
         }
       }
     };
-    // cursor over this step group's steps: item pass c_k, step c_n inside the item, global step c_base + c_n (parity == sg)
+    // cursor over this step group's steps: item pass c_k, step c_n inside the item, global step c_base + c_n (== sg mod 3)
     int c_k = 0, c_it = sched_pair_item(0, nitems), c_n = sg, c_base = 0, c_nq = c_it >= 0 ? tiles_of(c_it) : 0;
     auto normalize = [&]() {
       while (c_it >= 0 && c_n >= c_nq) {
@@ -636,20 +624,16 @@ attn_bwd_dq2_kernel(const __grid_constant__ CUtensorMap tmQ128, const __grid_con
           drop_rk = drop_row_key(dcfg.key, static_cast<uint32_t>(stat_idx(hb, hh, qt * 128 + r, H, T, seq_shift)));
         }
         stat_k = c_k;
-        int nk = c_k + 1;
-        if (NG == 2) {  // (NG = 3 runs on items of at least four steps: every group owns a step of every item)
-          const int nit = sched_pair_item(nk, nitems);
-          if (nit >= 0 && tiles_of(nit) == 1 && ((c_base + c_nq) & 1) != sg) ++nk;
-        }
-        load_stats(nk, nxt_l, nxt_d);
-        nxt_k = nk;
+        // items have at least four steps (T >= 256), so every group owns a step of every item: the next one is c_k + 1
+        load_stats(c_k + 1, nxt_l, nxt_d);
+        nxt_k = c_k + 1;
       }
       const int gs = c_base + c_n;
       ptx::mbar_wait(&s_full[gs % kSBuf], (gs / kSBuf) & 1, 78);
       ptx::tc_fence_after();
       const uint32_t tbuf = tmem_base + lane_off + (gs % kSBuf) * 128;
 #pragma unroll
-      for (int c = ch; c < 2; c += NCH) {
+      for (int c = 0; c < 2; ++c) {
         const int c0 = c_n * 64 + c * 32;
         const uint32_t ta_s = tbuf + c * 32, ta_dp = ta_s + 64;
         uint32_t pk[16];
@@ -663,7 +647,7 @@ attn_bwd_dq2_kernel(const __grid_constant__ CUtensorMap tmQ128, const __grid_con
       ptx::tc_fence_before();
       warp_arrive_leader(&ds_full[gs % kSBuf], lane);
       while (ep_k < c_k) epilogue(ep_k++);
-      c_n += NG;
+      c_n += 3;
       normalize();
     }
     while (ep_k < c_k) epilogue(ep_k++);
@@ -672,8 +656,6 @@ attn_bwd_dq2_kernel(const __grid_constant__ CUtensorMap tmQ128, const __grid_con
   ptx::cluster_sync_all();
   if (warp == 1) ptx::tmem_dealloc_2sm(tmem_base, 512);
 }
-
-constexpr int kNCH = 1;   // see PairCfg
 
 template <typename K>
 int set_smem(K kern, int bytes) {
@@ -718,21 +700,11 @@ int attn_bwd_pair(const void* qkv, const void* dout, const float* lse, const flo
   if ((rc = encode_tmap_2d(&tmDO32, dout, 2, static_cast<uint64_t>(C), rows, pitch_do, 64, 32, true))) return rc;
   if ((rc = encode_tmap_2d_sw(&tmDOc, dout, 2, static_cast<uint64_t>(C), rows, pitch_do, 32, 64, 64))) return rc;
   static bool done = false;
-  static int nch_dq = kNCH, nch_dkv = kNCH, ng_dq = 3;   // MEASURED (cfg3, per layer): dQ kernel with three step groups 0.118 vs 0.125 ms
   if (!done) {
-    if ((rc = set_smem(attn_bwd_dq2_kernel<false, 1, 2>, Dq2Smem::TOTAL))) return rc;
-    if ((rc = set_smem(attn_bwd_dq2_kernel<true, 1, 2>, Dq2Smem::TOTAL))) return rc;
-    if ((rc = set_smem(attn_bwd_dq2_kernel<false, 1, 3>, Dq2Smem::TOTAL))) return rc;
-    if ((rc = set_smem(attn_bwd_dq2_kernel<true, 1, 3>, Dq2Smem::TOTAL))) return rc;
-    if ((rc = set_smem(attn_bwd_dkv2_kernel<false, 1>, Dkv2Smem::TOTAL))) return rc;
-    if ((rc = set_smem(attn_bwd_dkv2_kernel<true, 1>, Dkv2Smem::TOTAL))) return rc;
-    if ((rc = set_smem(attn_bwd_dq2_kernel<false, 2, 2>, Dq2Smem::TOTAL))) return rc;
-    if ((rc = set_smem(attn_bwd_dq2_kernel<true, 2, 2>, Dq2Smem::TOTAL))) return rc;
-    if ((rc = set_smem(attn_bwd_dkv2_kernel<false, 2>, Dkv2Smem::TOTAL))) return rc;
-    if ((rc = set_smem(attn_bwd_dkv2_kernel<true, 2>, Dkv2Smem::TOTAL))) return rc;
-    if (const char* e = getenv("ABCGPT_ATTN_NCH_DQ")) nch_dq = e[0] == '2' ? 2 : 1;     // experiments: compute warps 8 x NCH
-    if (const char* e = getenv("ABCGPT_ATTN_NCH_DKV")) nch_dkv = e[0] == '2' ? 2 : 1;
-    if (const char* e = getenv("ABCGPT_ATTN_NG_DQ")) ng_dq = e[0] == '2' ? 2 : 3;        // step groups of the dQ kernel
+    if ((rc = set_smem(attn_bwd_dq2_kernel<false>, Dq2Smem::TOTAL))) return rc;
+    if ((rc = set_smem(attn_bwd_dq2_kernel<true>, Dq2Smem::TOTAL))) return rc;
+    if ((rc = set_smem(attn_bwd_dkv2_kernel<false>, Dkv2Smem::TOTAL))) return rc;
+    if ((rc = set_smem(attn_bwd_dkv2_kernel<true>, Dkv2Smem::TOTAL))) return rc;
     done = true;
   }
   const int BH = B * H, nitems = ((T + 255) / 256) * BH;
@@ -740,20 +712,17 @@ int attn_bwd_pair(const void* qkv, const void* dout, const float* lse, const flo
   const int pairs = sm_count() / 2;
   const int grid = 2 * (nitems < pairs ? nitems : pairs);  // persistent: one CTA per SM, SMs paired into clusters
   __nv_bfloat16* dq = reinterpret_cast<__nv_bfloat16*>(dqkv);
-  const bool drop = dcfg.thr16 != 0;
-#define ABCGPT_DKV2(D, N)                                                                                                   \
-  ABCGPT_CUDA(launch_pair(attn_bwd_dkv2_kernel<D, N>, grid, PairCfg<N>::kThreads, Dkv2Smem::TOTAL, stream, tmQKV128, tmQKV32,  \
-                          tmDO32, tmQKVc, tmDOc, lse, delta, dq, T, H, C, BH, nitems, dcfg, fBH, fH))
-#define ABCGPT_DQ2(D, N, G)                                                                                                 \
-  ABCGPT_CUDA(launch_pair(attn_bwd_dq2_kernel<D, N, G>, grid, PairCfg<N, G>::kThreads, Dq2Smem::TOTAL, stream, tmQKV128, tmDO128, \
-                          tmQKV32, tmQKVc, lse, delta, dq, T, H, C, BH, nitems, dcfg, fBH, fH))
-  if (nch_dkv == 2) { if (drop) ABCGPT_DKV2(true, 2); else ABCGPT_DKV2(false, 2); }
-  else { if (drop) ABCGPT_DKV2(true, 1); else ABCGPT_DKV2(false, 1); }
-  if (nch_dq == 2) { if (drop) ABCGPT_DQ2(true, 2, 2); else ABCGPT_DQ2(false, 2, 2); }
-  else if (ng_dq == 3) { if (drop) ABCGPT_DQ2(true, 1, 3); else ABCGPT_DQ2(false, 1, 3); }
-  else { if (drop) ABCGPT_DQ2(true, 1, 2); else ABCGPT_DQ2(false, 1, 2); }
-#undef ABCGPT_DKV2
-#undef ABCGPT_DQ2
+  if (dcfg.thr16 == 0) {
+    ABCGPT_CUDA(launch_pair(attn_bwd_dkv2_kernel<false>, grid, DkvCfg::kThreads, Dkv2Smem::TOTAL, stream, tmQKV128, tmQKV32, tmDO32, tmQKVc,
+                            tmDOc, lse, delta, dq, T, H, C, BH, nitems, dcfg, fBH, fH));
+    ABCGPT_CUDA(launch_pair(attn_bwd_dq2_kernel<false>, grid, DqCfg::kThreads, Dq2Smem::TOTAL, stream, tmQKV128, tmDO128, tmQKV32, tmQKVc,
+                            lse, delta, dq, T, H, C, BH, nitems, dcfg, fBH, fH));
+  } else {
+    ABCGPT_CUDA(launch_pair(attn_bwd_dkv2_kernel<true>, grid, DkvCfg::kThreads, Dkv2Smem::TOTAL, stream, tmQKV128, tmQKV32, tmDO32, tmQKVc,
+                            tmDOc, lse, delta, dq, T, H, C, BH, nitems, dcfg, fBH, fH));
+    ABCGPT_CUDA(launch_pair(attn_bwd_dq2_kernel<true>, grid, DqCfg::kThreads, Dq2Smem::TOTAL, stream, tmQKV128, tmDO128, tmQKV32, tmQKVc,
+                            lse, delta, dq, T, H, C, BH, nitems, dcfg, fBH, fH));
+  }
   return launch_status("attn_bwd pair kernels");
 }
 

@@ -80,22 +80,7 @@ __device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* t
       "l"(reinterpret_cast<uint64_t>(tm)), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
       : "memory");
 }
-__device__ __forceinline__ void tma_load_3d(void* smem_dst, const CUtensorMap* tm, uint64_t* bar, int c0, int c1,
-                                            int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], "
-      "[%2];" ::"r"(smem_u32(smem_dst)),
-      "l"(reinterpret_cast<uint64_t>(tm)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
-}
-// 2D tile store shared -> global (bulk async group)
-__device__ __forceinline__ void tma_store_2d(const CUtensorMap* tm, const void* smem_src, int c0, int c1) {
-  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(
-                   reinterpret_cast<uint64_t>(tm)),
-               "r"(smem_u32(smem_src)), "r"(c0), "r"(c1)
-               : "memory");
-}
-// same, source given as a shared-window address
+// 2D tile store shared -> global (bulk async group), source given as a shared-window address
 __device__ __forceinline__ void tma_store_2d_s(const CUtensorMap* tm, uint32_t smem_src, int c0, int c1) {
   asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(
                    reinterpret_cast<uint64_t>(tm)),
@@ -237,11 +222,6 @@ __device__ __forceinline__ void red_min_shared_cluster_s32(uint32_t cluster_addr
 __device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
   asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
 }
-// release at CLUSTER scope: what this thread wrote (tensor memory included, after tcgen05.wait::st + fence::before_thread_sync)
-// is visible to a thread of the other CTA that observes the phase
-__device__ __forceinline__ void mbar_arrive_release_cluster(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
 // TMA load issued by either CTA of a pair; completion bytes are credited to the mbarrier at `mbar_cluster_addr`
 // (the leader CTA's barrier)
 __device__ __forceinline__ void tma_load_2d_2sm(void* smem_dst, const CUtensorMap* tm, uint32_t mbar_cluster_addr, int c0,
@@ -250,16 +230,6 @@ __device__ __forceinline__ void tma_load_2d_2sm(void* smem_dst, const CUtensorMa
       "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], "
       "[%2];" ::"r"(smem_u32(smem_dst)),
       "l"(reinterpret_cast<uint64_t>(tm)), "r"(mbar_cluster_addr), "r"(c0), "r"(c1)
-      : "memory");
-}
-// multicast variant: the tile lands at the same shared-memory offset in every CTA of cta_mask and the bytes are credited
-// to the barrier at the given offset in the pair leader of each destination CTA
-__device__ __forceinline__ void tma_load_2d_2sm_mc(void* smem_dst, const CUtensorMap* tm, uint32_t mbar_cluster_addr, int c0,
-                                                   int c1, uint16_t cta_mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster "
-      "[%0], [%1, {%3, %4}], [%2], %5;" ::"r"(smem_u32(smem_dst)),
-      "l"(reinterpret_cast<uint64_t>(tm)), "r"(mbar_cluster_addr), "r"(c0), "r"(c1), "h"(cta_mask)
       : "memory");
 }
 __device__ __forceinline__ void tmem_alloc_2sm(uint32_t* smem_dst, uint32_t ncols) {
@@ -387,11 +357,6 @@ __device__ __forceinline__ void stg256(void* p, uint32_t a, uint32_t b, uint32_t
                "r"(f), "r"(g), "r"(h)
                : "memory");
 }
-// register re-balancing between warpgroups (all four warps of a warpgroup execute the same instruction)
-template <int N>
-__device__ __forceinline__ void setmaxnreg_inc() { asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(N)); }
-template <int N>
-__device__ __forceinline__ void setmaxnreg_dec() { asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(N)); }
 __device__ __forceinline__ void bar_sync(int id, int nthreads) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }

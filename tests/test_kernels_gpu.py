@@ -9,7 +9,7 @@ from tools import gpu_probe  # noqa: E402
 FAST_CASES = [
     "gemm_nt_small_bn128", "gemm_nt_small_bn256", "gemm_nn_small_bn128", "gemm_nn_small_bn256",
     "gemm_tn_small_bn128", "gemm_tn_small_bn256", "gemm_nt_k256_bn256", "gemm_nt_ragged", "gemm_nt_f32",
-    "gemm4_nt", "gemm4_nn_dgelu", "gemm4_tn_red", "gemm2_nt_small", "gemm2_nt_k512", "gemm2_nn", "gemm2_tn", "gemm2_tn_red", "gemm2_ragged", "gemm2_gelu", "gemm2_resid",
+    "gemm2_nt_small", "gemm2_nt_k512", "gemm2_nn", "gemm2_tn", "gemm2_tn_red", "gemm2_ragged", "gemm2_gelu", "gemm2_resid",
     "gemm2_dgelu", "gemm2_half_nt", "gemm2_half_nn", "gemm2_half_gelu", "gemm2_half_dgelu", "gemm2_half_resid", "gemm_auto_cfg2_resid", "gemm_auto_cfg2_dgrad", "gemm_auto_cfg2_dgelu", "gemm_auto_cfg2_wgrad", "gemm2_gelu_tanh", "gemm2_dgelu_tanh", "gemm_gelu", "gemm_resid", "gemm_dgelu", "gemm_wgrad_red",
     "attn_spike", "attn_t32", "attn_t32_packed", "attn_t64_packed", "attn_t64", "attn_t128", "attn_t200", "attn_t256", "attn_t1024",
     "ln_384", "ln_768", "ln_768_bias", "ln_1000", "ln_resid_768", "ln_resid_1000_bias", "ce_95", "ce_50304", "colsum_768", "colsum_narrow_130", "adamw", "embed", "embed_bigv",

@@ -1,7 +1,7 @@
 """Build an A/B variant of libabcgpt.so: extra nvcc flags (usually -D switches) for selected sources, output next to the
 product library as libabcgpt_<name>.so.  Select it at run time with ABCGPT_LIB=<path> (ai_music_generation_b200/_C.py).
 
-    python tools/build_variant.py NAME "-DABCGPT_ISSUERS_FIRST" gemm.cu [attn.cu ...]
+    python tools/build_variant.py NAME "-DABCGPT_NO_PDL" gemm.cu [attn.cu ...]
 """
 import os
 import subprocess

@@ -388,10 +388,6 @@ def build_cases():
     cases["gemm2_nn"] = lambda: case_gemm("gemm2_nn", 512, 512, 384, False, True, E.EPI_BF16, 512, timing=False)
     cases["gemm2_tn"] = lambda: case_gemm("gemm2_tn", 512, 512, 1024, True, True, E.EPI_F32, 512, timing=False)
     cases["gemm2_tn_red"] = lambda: case_gemm("gemm2_tn_red", 768, 768, 8192, True, True, E.EPI_F32_RED, 512, timing=False)
-    # clusters of two CTA pairs with TMA-multicast B (tile hint 1024): all three operand-majorness forms
-    cases["gemm4_nt"] = lambda: case_gemm("gemm4_nt", 1024, 768, 512, False, False, E.EPI_BF16, 1024, timing=False)
-    cases["gemm4_nn_dgelu"] = lambda: case_gemm("gemm4_nn_dgelu", 1024, 1536, 384, False, True, E.EPI_DGELU, 1024, timing=False)
-    cases["gemm4_tn_red"] = lambda: case_gemm("gemm4_tn_red", 1536, 768, 8192, True, True, E.EPI_F32_RED, 1024, timing=False)
     cases["gemm2_ragged"] = lambda: case_gemm("gemm2_ragged", 328, 200, 136, False, False, E.EPI_BF16, 512, timing=False)
     cases["gemm2_gelu"] = lambda: case_gemm("gemm2_gelu", 1024, 1536, 384, False, False, E.EPI_GELU, 512, timing=False)
     cases["gemm2_resid"] = lambda: case_gemm("gemm2_resid", 1024, 384, 1536, False, False, E.EPI_RESID, 512, timing=False)
