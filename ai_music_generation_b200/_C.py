@@ -19,7 +19,7 @@ DEBUG_HEADER_PATH = os.path.join(os.path.dirname(HERE), "include", "abcgpt_debug
 
 EPI_BF16, EPI_GELU, EPI_RESID, EPI_DGELU, EPI_F32_RED, EPI_F32 = range(6)
 FN_IDS = {"abcgpt_gemm_bf16": 1, "abcgpt_embed_fwd": 2, "abcgpt_layernorm_fwd": 3, "abcgpt_attn_decode": 4, "abcgpt_argmax": 5,
-          "abcgpt_sample_topk": 6, "abcgpt_attn_decode_hd": 7}
+          "abcgpt_sample_topk": 6, "abcgpt_attn_decode_hd": 7, "abcgpt_sample_top_p": 8}
 ACT_TANH = 0x100  # OR-ed into EPI_GELU / EPI_DGELU: tanh form of GELU (include/abcgpt.h ABCGPT_ACT_TANH)
 
 _P = c_void_p
@@ -61,6 +61,7 @@ _SIGNATURES = {
     "abcgpt_set_dynamic_tiles": (c_int, [c_int]),
     "abcgpt_argmax": (c_int, [_P, c_int64, c_int, _P, c_int64, c_int, _P]),
     "abcgpt_sample_topk": (c_int, [_P, c_int64, c_int, c_float, c_int, _P, c_int64, _P, c_int64, c_int, _P]),
+    "abcgpt_sample_top_p": (c_int, [_P, c_int64, c_int, c_float, c_int, c_float, _P, _P, c_int64, _P, _P, c_int64, c_int, _P]),
 }
 # include/abcgpt_debug.h: only in libabcgpt_debug.so (tools/)
 _DEBUG_SIGNATURES = {

@@ -124,6 +124,12 @@ int abcgpt_sample_topk(const void* logits, int64_t ldl, int V, float temperature
                        int64_t counter, int64_t* out, int64_t out_stride, int B, void* stream) {
   return sample_topk(logits, ldl, V, temperature, top_k, seed, counter, out, out_stride, B, S(stream));
 }
+int abcgpt_sample_top_p(const void* logits, int64_t ldl, int V, float top_p, int top_k, float temperature, const void* seed,
+                        const void* counter_base, int64_t counter, const int64_t* row_id, int64_t* out, int64_t out_stride, int B,
+                        void* stream) {
+  return sample_top_p(logits, ldl, V, top_p, top_k, temperature, seed, counter_base, counter, row_id, out, out_stride, B,
+                      S(stream));
+}
 
 /*
  * Replay of a recorded launch list with position-affine arguments (the decode loop of GPT.generate is launch-bound: ~90
@@ -179,6 +185,11 @@ int abcgpt_replay(const int64_t* prog, int64_t n_words, int64_t k) {
       case ABCGPT_FN_SAMPLE_TOPK:
         if (nargs != 11) return fail(-1, "abcgpt_replay: sample_topk takes 11 arguments");
         rc = abcgpt_sample_topk(P_(0), a[1], I_(2), abcgpt_word_f(a[3]), I_(4), P_(5), a[6], MP_(int64_t, 7), a[8], I_(9), P_(10));
+        break;
+      case ABCGPT_FN_SAMPLE_TOP_P:
+        if (nargs != 14) return fail(-1, "abcgpt_replay: sample_top_p takes 14 arguments");
+        rc = abcgpt_sample_top_p(P_(0), a[1], I_(2), abcgpt_word_f(a[3]), I_(4), abcgpt_word_f(a[5]), P_(6), P_(7), a[8],
+                                 CP_(int64_t, 9), MP_(int64_t, 10), a[11], I_(12), P_(13));
         break;
       default:
         return fail(-1, "abcgpt_replay: unknown function id %lld", (long long)fn);

@@ -65,5 +65,8 @@ int argmax_rows(const void* logits, long long ldl, int V, int64_t* out, long lon
                 cudaStream_t stream);
 int sample_topk(const void* logits, long long ldl, int V, float temperature, int top_k, const void* seed, long long counter,
                 int64_t* out, long long out_stride, int B, cudaStream_t stream);
+int sample_top_p(const void* logits, long long ldl, int V, float top_p, int top_k, float temperature, const void* seed,
+                 const void* counter_base, long long counter, const int64_t* row_id, int64_t* out, long long out_stride, int B,
+                 cudaStream_t stream);
 
 }  // namespace abcgpt

@@ -408,7 +408,194 @@ int sample_topk_cluster(const __nv_bfloat16* logits, long long ldl, int V, float
   return launch_status("sample_topk_cluster_kernel");
 }
 
+// ---- nucleus / top-k / temperature head of the TunesFormer character decoder ------------------------------------------
+// The reference draws each character with the `samplings` package (tunesformer/utils.py:247-250), restated on the host by
+// top_p_filter / top_k_filter / temperature_draw in tunesformer.py.  One CTA per row, V <= 1024 (the character vocabulary
+// is 128), everything in shared memory:
+//   softmax  p = softmax(float(l)) in fp32
+//   rank     every token's position in the order (p descending, lower index first), as numpy's stable argsort(-p)
+//   nucleus  keep ranks 0 .. r* where r* is the first rank whose running sum (in rank order) reaches top_p; all if none does
+//   top-k    keep ranks < top_k (exactly k tokens, ties by lower index; unlike sample_topk_kernel, which keeps ties)
+//   draw     temperature <= 0 or a single kept token with p > 0: the rank-0 token (first maximal index); otherwise weights
+//            (p / p_max)^(1 / temperature) on the kept tokens, inverse CDF in token order with one Philox uniform
+// The renormalisations of the restatement are divisions by one constant per step: they change no order and no cut point
+// (the nucleus cut is taken on the raw p, whose sum is 1), so they are left out.
+constexpr int kTopPThreads = 128;
+constexpr int kTopPMaxV = 1024;  // include/abcgpt.h
+constexpr int kTopPWarps = kTopPThreads / 32;
+
+__device__ __forceinline__ float tp_block_max(float v, float* scratch) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
+  __syncthreads();  // scratch reuse
+  if ((threadIdx.x & 31) == 0) scratch[threadIdx.x >> 5] = v;
+  __syncthreads();
+  float t = scratch[0];
+#pragma unroll
+  for (int w = 1; w < kTopPWarps; ++w) t = fmaxf(t, scratch[w]);
+  return t;
+}
+
+// sum in a fixed order (butterfly inside the warp, warps in order): the same inputs give the same bits in every thread
+__device__ __forceinline__ float tp_block_sum(float v, float* scratch) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  __syncthreads();
+  if ((threadIdx.x & 31) == 0) scratch[threadIdx.x >> 5] = v;
+  __syncthreads();
+  float t = 0.f;
+#pragma unroll
+  for (int w = 0; w < kTopPWarps; ++w) t += scratch[w];
+  return t;
+}
+
+__device__ __forceinline__ int tp_block_min(int v, int* scratch) {
+  v = __reduce_min_sync(0xffffffffu, v);
+  __syncthreads();
+  if ((threadIdx.x & 31) == 0) scratch[threadIdx.x >> 5] = v;
+  __syncthreads();
+  int t = scratch[0];
+#pragma unroll
+  for (int w = 1; w < kTopPWarps; ++w) t = min(t, scratch[w]);
+  return t;
+}
+
+// exclusive prefix of one value per thread over the block (threads in order); *total = the block sum
+__device__ __forceinline__ float tp_block_excl_scan(float v, float* scratch, float* total) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  float incl = v;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const float t = __shfl_up_sync(0xffffffffu, incl, o);
+    if (lane >= o) incl += t;
+  }
+  __syncthreads();
+  if (lane == 31) scratch[warp] = incl;
+  __syncthreads();
+  float off = 0.f, tot = 0.f;
+#pragma unroll
+  for (int w = 0; w < kTopPWarps; ++w) {
+    if (w < warp) off += scratch[w];
+    tot += scratch[w];
+  }
+  *total = tot;
+  return off + incl - v;
+}
+
+__global__ void __launch_bounds__(kTopPThreads)
+sample_top_p_kernel(const __nv_bfloat16* __restrict__ logits, long long ldl, int V, float top_p, int top_k, float temperature,
+                    const unsigned long long* __restrict__ seed, const long long* __restrict__ counter_base, long long counter,
+                    const int64_t* __restrict__ row_id, int64_t* __restrict__ out, long long out_stride) {
+  __shared__ float p[kTopPMaxV];      // softmax in token order, then the weights of the draw
+  __shared__ float sp[kTopPMaxV];     // softmax in rank order
+  __shared__ short tok[kTopPMaxV];    // token at each rank
+  __shared__ short rk[kTopPMaxV];     // rank of each token
+  __shared__ float red_f[kTopPWarps];
+  __shared__ int red_i[kTopPWarps];
+  const int tid = threadIdx.x, row = blockIdx.x;
+  const __nv_bfloat16* lr = logits + static_cast<long long>(row) * ldl;
+
+  // ---- p = softmax(float(l))
+  float mx = -INFINITY;
+  for (int i = tid; i < V; i += kTopPThreads) {
+    const float x = __bfloat162float(lr[i]);
+    p[i] = x;
+    mx = fmaxf(mx, x);
+  }
+  mx = tp_block_max(mx, red_f);
+  float s = 0.f;
+  for (int i = tid; i < V; i += kTopPThreads) {
+    const float e = expf(p[i] - mx);
+    p[i] = e;
+    s += e;
+  }
+  const float z = tp_block_sum(s, red_f);
+  for (int i = tid; i < V; i += kTopPThreads) p[i] = __fdiv_rn(p[i], z);
+  __syncthreads();
+
+  // ---- rank of every token: (p descending, index ascending)
+  for (int i = tid; i < V; i += kTopPThreads) {
+    const float pi = p[i];
+    int r = 0;
+    for (int j = 0; j < V; ++j) {
+      const float pj = p[j];  // the same address in every lane: a broadcast
+      r += (pj > pi || (pj == pi && j < i)) ? 1 : 0;
+    }
+    sp[r] = pi;
+    tok[r] = static_cast<short>(i);
+    rk[i] = static_cast<short>(r);
+  }
+  __syncthreads();
+
+  // ---- nucleus, then top-k: the kept tokens are the ranks [0, n_keep)
+  const int chunk = (V + kTopPThreads - 1) / kTopPThreads;  // contiguous per thread: a prefix over threads is a prefix of V
+  const int c0 = min(V, tid * chunk), c1 = min(V, c0 + chunk);
+  int n_keep = V;
+  if (top_p < 1.f) {
+    float local = 0.f;
+    for (int r = c0; r < c1; ++r) local += sp[r];
+    float total;
+    float acc = tp_block_excl_scan(local, red_f, &total);
+    int first = INT_MAX;
+    for (int r = c0; r < c1; ++r) {
+      acc += sp[r];
+      if (acc >= top_p) { first = r; break; }
+    }
+    first = tp_block_min(first, red_i);  // the first rank at which the running sum reaches top_p
+    n_keep = first == INT_MAX ? V : first + 1;
+  }
+  if (top_k > 0 && top_k < n_keep) n_keep = top_k;
+
+  // ---- greedy: temperature <= 0, or one kept token with p > 0 (zeros sort last)
+  if (temperature <= 0.f || n_keep == 1 || !(sp[1] > 0.f)) {
+    if (tid == 0) out[static_cast<long long>(row) * out_stride] = tok[0];
+    return;
+  }
+
+  // ---- weights (p / p_max)^(1 / temperature) on the kept tokens, one inverse-CDF draw in token order
+  const float inv_t = 1.f / temperature, ptop = sp[0];
+  float local = 0.f;
+  for (int i = c0; i < c1; ++i) {
+    const float w = (rk[i] < n_keep && p[i] > 0.f) ? powf(__fdiv_rn(p[i], ptop), inv_t) : 0.f;
+    p[i] = w;  // only this thread touches [c0, c1) from here on
+    local += w;
+  }
+  float total;
+  const float excl = tp_block_excl_scan(local, red_f, &total);
+  const long long rid = row_id != nullptr ? row_id[row] : row;
+  const uint32_t bits = philox_uniform_bits(*seed, static_cast<uint32_t>(rid), static_cast<uint64_t>(*counter_base + counter));
+  const float u = static_cast<float>(bits >> 8) * (1.0f / 16777216.0f);  // [0, 1)
+  const float target = u * total;
+  int pick = INT_MAX, last = -1;
+  float acc = excl;
+  for (int i = c0; i < c1; ++i) {
+    const float w = p[i];
+    if (w > 0.f) {
+      last = i;
+      acc += w;
+      if (pick == INT_MAX && acc > target && target >= excl) pick = i;
+    }
+  }
+  // rounding may let two neighbouring chunks both claim the target (the smallest wins) or neither (the last kept token)
+  pick = tp_block_min(pick, red_i);
+  last = -tp_block_min(-last, red_i);
+  if (tid == 0) out[static_cast<long long>(row) * out_stride] = pick != INT_MAX ? pick : last;
+}
+
 }  // namespace
+
+int sample_top_p(const void* logits, long long ldl, int V, float top_p, int top_k, float temperature, const void* seed,
+                 const void* counter_base, long long counter, const int64_t* row_id, int64_t* out, long long out_stride, int B,
+                 cudaStream_t stream) {
+  ABCGPT_CHECK_ARG(logits && out && seed && counter_base && B > 0, "sample_top_p: bad arguments");
+  ABCGPT_CHECK_ARG(V >= 1 && V <= kTopPMaxV, "sample_top_p: vocabulary of %d tokens is outside [1, %d]", V, kTopPMaxV);
+  ABCGPT_CHECK_ARG(ldl >= V, "sample_top_p: row stride %lld is below V = %d", ldl, V);
+  sample_top_p_kernel<<<B, kTopPThreads, 0, stream>>>(reinterpret_cast<const __nv_bfloat16*>(logits), ldl, V, top_p, top_k,
+                                                      temperature, reinterpret_cast<const unsigned long long*>(seed),
+                                                      reinterpret_cast<const long long*>(counter_base), counter, row_id, out,
+                                                      out_stride);
+  return launch_status("sample_top_p_kernel");
+}
 
 int sample_topk(const void* logits, long long ldl, int V, float temperature, int top_k, const void* seed, long long counter,
                 int64_t* out, long long out_stride, int B, cudaStream_t stream) {

@@ -170,6 +170,12 @@ class _DecodeState:
         self.stat = e(2, B, dt=f32)
         self.logits = e(B, self.Vpad)
         self.col = torch.zeros(Tmax + 1, B, device=device, dtype=torch.int64)  # token column t = contiguous int64 [B]
+        # set by callers of the other input / output modes of GPT._decode_step (hierarchical decoders): fp32 [B, C] input rows
+        # (`inp` "first" / "embed"), fp32 [B, C] ln_f output rows (`hidden`), and the (seed, counter base, row ids) device
+        # buffers of the ("top_p", ...) sampling head.  Recorded launch lists hold their addresses.
+        self.emb = None
+        self.hidden = None
+        self.sampler = None
         self.plans = {}
         self.affine = {}   # (flags) -> (t0, recorded plan at t0, per-launch argument deltas per position)
 
@@ -852,13 +858,18 @@ class GPT(nn.Module):
             self.train(was_training)
         return out
 
-    def _decode_step(self, st, t, want_logits, head):
+    def _decode_step(self, st, t, want_logits, head, inp="tokens", hidden=False):
         """Position t of every sequence (tokens st.col[t]).  Appends this position's q|k|v to the cache and, if
         want_logits, leaves the next-token logits in st.logits and runs the sampling head, which writes token t + 1 of every
         sequence into st.col[t + 1]: head = None (logits only), ("greedy",) = argmax, ("sample", temperature, top_k) = the
-        fused temperature / top-k / softmax / multinomial kernel (seeded per generate() call through self._sample_seed).
+        fused temperature / top-k / softmax / multinomial kernel (seeded per generate() call through self._sample_seed),
+        ("top_p", top_p, top_k, temperature) = the nucleus / top-k / temperature kernel of the TunesFormer character decoder
+        (seed, counter base and row ids from st.sampler; counter = t).
+        Input and output modes of a decoder fed by another network (TunesFormer): inp = "tokens" (token ids st.col[t]),
+        "first" (t = 0 only: the fp32 row st.emb replaces the token embedding, + wpe[0]) or "embed" (st.emb + wpe[t]);
+        hidden = True writes the fp32 ln_f output of the position to st.hidden (HF last_hidden_state) instead of logits.
         Every argument is static per (t, flags), so the launch list is recorded once and replayed afterwards."""
-        flags = (want_logits, head, torch.cuda.current_stream().cuda_stream)
+        flags = (want_logits, head, torch.cuda.current_stream().cuda_stream, inp, hidden)
         plan_key = (t,) + flags
         plan = st.plans.get(plan_key) if self._plan_cache_enabled else None
         if plan is not None:
@@ -882,7 +893,18 @@ class GPT(nn.Module):
         top = self._arena["top"]
         B, C, H = st.B, cfg.n_embd, cfg.n_head
         x, y = st.x
-        ops.embed_fwd(tokens, top["wte"][0], top["wpe"][0][t:t + 1], x, 1)
+        if inp == "tokens":
+            ops.embed_fwd(tokens, top["wte"][0], top["wpe"][0][t:t + 1], x, 1)
+        elif inp == "first":
+            if t != 0 or st.emb is None:
+                raise _C.AbcgptError("decode step: the 'first' input mode is position 0 of a state with its emb rows set")
+            ops.set_first_pos(st.emb, top["wpe"][0], x, 1)
+        elif inp == "embed":
+            if st.emb is None:
+                raise _C.AbcgptError("decode step: the 'embed' input mode needs the state's emb rows")
+            ops.add_pos(st.emb, top["wpe"][0][t:t + 1], x, 1)
+        else:
+            raise ValueError(f"decode step: unknown input mode {inp!r}")
         for li, lw in enumerate(layers):
             b = lambda name: None if lw[name] is None else lw[name][0]  # noqa: E731
             ops.layernorm_fwd(x, lw["ln_1.weight"][0], b("ln_1.bias"), st.ln, st.stat[0], st.stat[1])
@@ -904,12 +926,19 @@ class GPT(nn.Module):
                      tile_n=128)
             ops.gemm(st.g, lw["mlp.c_proj.weight"][1], epilogue=ops.EPI_RESID, out=x, aux=y, bias=b("mlp.c_proj.bias"),
                      tile_n=128)
-        if want_logits:
+        if hidden and (want_logits or st.hidden is None):
+            raise _C.AbcgptError("decode step: the hidden-state output needs the state's hidden rows and replaces the logits")
+        if want_logits or hidden:
             lnf_b = None if top["ln_f.bias"] is None else top["ln_f.bias"][0]
-            ops.layernorm_fwd(x, top["ln_f.weight"][0], lnf_b, st.ln, st.stat[0], st.stat[1])
+            ops.layernorm_fwd(x, top["ln_f.weight"][0], lnf_b, st.ln, st.stat[0], st.stat[1], y_f32=st.hidden if hidden else None)
+        if want_logits:
             ops.gemm(st.ln, top["wte"][1], N=st.Vpad, epilogue=ops.EPI_BF16, out=st.logits, tile_n=128)
             if head is not None and head[0] == "greedy":
                 ops.argmax(st.logits, cfg.vocab_size, st.col[t + 1], out_stride=1)
+            elif head is not None and head[0] == "top_p":
+                seed, counter_base, row_id = st.sampler
+                ops.sample_top_p(st.logits, cfg.vocab_size, st.col[t + 1], head[1], head[2], head[3], seed, counter_base, t,
+                                 row_id=row_id)
             elif head is not None:
                 ops.sample_topk(st.logits, cfg.vocab_size, st.col[t + 1], head[1], head[2], self._seed_buffer(), t)
         if self._plan_cache_enabled:

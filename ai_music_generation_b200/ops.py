@@ -12,6 +12,7 @@ from ._C import ACT_TANH, EPI_BF16, EPI_DGELU, EPI_F32, EPI_F32_RED, EPI_GELU, E
 
 
 LAUNCHES = 0      # kernels of libabcgpt.so enqueued so far (bench.py reports the delta over its timed region)
+CALLS = 0         # calls into libabcgpt.so that enqueue work (a compiled replay of a whole launch list counts once)
 _PROFILE = None   # optional list collecting (name, meta, start_event, end_event) per C-ABI call
 
 
@@ -104,7 +105,7 @@ def record_callback(fn):
 
 
 def replay(plan, patches=None, keys=None):
-    global LAUNCHES
+    global LAUNCHES, CALLS
     if patches:
         for i, site in patches:
             plan[i][3][-2] = keys[site]
@@ -120,6 +121,7 @@ def replay(plan, patches=None, keys=None):
             e[1]()
             continue
         LAUNCHES += e[1]
+        CALLS += 1
         rc = e[2](*e[3])
         if rc != 0:
             _C.check(rc, e[0])
@@ -176,9 +178,10 @@ def compile_affine(plan, deltas):
 
 
 def replay_compiled(prog, k):
-    global LAUNCHES
+    global LAUNCHES, CALLS
     arr, n, launches = prog
     LAUNCHES += launches
+    CALLS += 1
     rc = _C.lib().abcgpt_replay(arr, n, k)
     if rc != 0:
         _C.check(rc, "abcgpt_replay")
@@ -186,11 +189,12 @@ def replay_compiled(prog, k):
 
 def replay_affine(plan, deltas, k):
     """Replay `plan` with every patched argument advanced by k * delta (see plan_deltas)."""
-    global LAUNCHES
+    global LAUNCHES, CALLS
     if _PROFILE is not None or _RECORD is not None:
         raise _C.AbcgptError("replay_affine: not available while profiling / recording")
     for e, patches in zip(plan, deltas):
         LAUNCHES += e[1]
+        CALLS += 1
         if patches:
             args = list(e[3])
             for i, d in patches:
@@ -203,8 +207,9 @@ def replay_affine(plan, deltas, k):
 
 
 def _call(name, nkernels, meta, fn, *args):
-    global LAUNCHES
+    global LAUNCHES, CALLS
     LAUNCHES += nkernels
+    CALLS += 1
     if _RECORD is not None:
         _RECORD.append((name, nkernels, fn, args, meta))
     if _PROFILE is None:
@@ -405,6 +410,16 @@ def sample_topk(logits, V, out, temperature, top_k, seed, counter, out_stride=1)
     B, ldl = logits.shape[0], logits.stride(0)
     _call("sample_topk", 1, (B, V), _C.lib().abcgpt_sample_topk, logits.data_ptr(), ldl, V, float(temperature),
           int(top_k) if top_k is not None else 0, seed.data_ptr(), int(counter), out.data_ptr(), out_stride, B, _stream())
+
+
+def sample_top_p(logits, V, out, top_p, top_k, temperature, seed, counter_base, counter, row_id=None, out_stride=1):
+    """Nucleus, then top-k, then temperature, one draw per row (include/abcgpt.h: abcgpt_sample_top_p).  seed / counter_base:
+    int64 device scalars; counter: the decode position; row_id: optional int64 [B] device tensor naming each row's stream."""
+    _chk(logits, torch.bfloat16, "sample logits")
+    B, ldl = logits.shape[0], logits.stride(0)
+    _call("sample_top_p", 1, (B, V), _C.lib().abcgpt_sample_top_p, logits.data_ptr(), ldl, V, float(top_p), int(top_k),
+          float(temperature), seed.data_ptr(), counter_base.data_ptr(), int(counter), _ptr(row_id), out.data_ptr(), out_stride, B,
+          _stream())
 
 
 def nvls_allreduce_sumsq(grad_mc_ptr, n, rank, world, partials_mc_ptr, blocks_per_rank, threads=512):

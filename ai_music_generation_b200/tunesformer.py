@@ -18,8 +18,8 @@ import numpy as np
 import torch
 import torch.nn as nn
 
-from . import ops
-from .model import GPT, GPTConfig
+from . import _C, ops
+from .model import GPT, GPTConfig, _DecodeState
 
 PATCH_SIZE = 32      # tunesformer/config.py:2
 PATCH_LENGTH = 128   # tunesformer/config.py:1
@@ -127,15 +127,9 @@ class _PatchEmbed(torch.autograd.Function):
     @staticmethod
     def forward(ctx, anchor, dec, patches):
         M = patches.shape[0]
-        S, V, C = PATCH_SIZE, CHAR_VOCAB, dec.config.n_embd
         dec._ensure_device_state()
-        oh = dec._onehot.get(M)
-        if oh is None:
-            oh = dec._onehot[M] = torch.empty(M, S * V, device=patches.device, dtype=torch.bfloat16)
-        ops.onehot_bf16(patches.contiguous(), oh, V)
-        out = torch.empty(M, C, device=patches.device, dtype=torch.float32)
-        ops.gemm(oh, dec._view("shadow", "patch_embedding.weight"), epilogue=ops.EPI_F32, out=out,
-                 bias=dec._view("flat", "patch_embedding.bias"))
+        out = torch.empty(M, dec.config.n_embd, device=patches.device, dtype=torch.float32)
+        oh = dec.embed_patches(patches.contiguous(), out)
         ctx.dec, ctx.oh = dec, oh
         return out
 
@@ -164,6 +158,18 @@ class PatchLevelDecoder(GPT):
         torch.nn.init.zeros_(self.patch_embedding.bias)
         self._onehot = {}
         self._flatten()
+
+    def embed_patches(self, patches, out):
+        """out fp32 [M, C] = onehot(patches int64 [M, PATCH_SIZE]) W^T + b (one-hot rows, then the GEMM); returns the one-hot
+        rows.  The bf16 weight shadow must be current (_ensure_device_state)."""
+        M = patches.shape[0]
+        oh = self._onehot.get(M)
+        if oh is None:
+            oh = self._onehot[M] = torch.empty(M, PATCH_SIZE * CHAR_VOCAB, device=patches.device, dtype=torch.bfloat16)
+        ops.onehot_bf16(patches, oh, CHAR_VOCAB)
+        ops.gemm(oh, self._view("shadow", "patch_embedding.weight"), epilogue=ops.EPI_F32, out=out,
+                 bias=self._view("flat", "patch_embedding.bias"))
+        return oh
 
     def encode(self, patches):
         """patches int64 [B, P, PATCH_SIZE] -> fp32 [B, P, C] (last_hidden_state)."""
@@ -265,6 +271,251 @@ class TunesFormerShaped(nn.Module):
             remaining = ""
             patches = torch.cat([patches, nxt], dim=1)
         return tune
+
+    # ---- generation on the device ------------------------------------------------------------------------------------
+    @torch.no_grad()
+    def generate_tunes(self, prompts, max_patch=PATCH_LENGTH, top_p=0.8, top_k=8, temperature=1.2, seed=None, batch=64):
+        """`generate_tune` for a list of prompt texts, batched and decoded on the device; returns one tune text per prompt.
+
+        Per tune the loop is that of generate_tune: the prompt is encoded with the same Patchilizer, its unfinished last bar
+        becomes fixed characters of the first generated bar, each bar is spelled until eos or 31 characters, and a tune stops
+        at an end patch, an empty bar or `max_patch` patches.  Both decoders run single-position steps over KV caches
+        (generate_patches), the draw is the nucleus / top-k / temperature kernel (abcgpt_sample_top_p), and the host
+        synchronises once per bar (plus an early-exit check every 8 characters).
+
+        Seeding differs from `generate` / `generate_tune` on purpose: those reproduce the reference's per-draw reseeding of
+        Python's `random` and numpy's generator on the host, which no device kernel can follow.  Here every draw takes a
+        Philox uniform of (seed, index of the tune in `prompts`, patch position, character position), so a tune's random
+        stream does not depend on the batch it lands in.  An int `seed` makes a call reproducible; seed=None draws one seed
+        from torch's CPU generator per call, so `torch.manual_seed` makes it reproducible.  With top_k = 1 every tune equals
+        its greedy generate_tune (up to decisions closer than bf16 rounding)."""
+        pz = Patchilizer()
+        patches, fixed, remaining = [], [], []
+        for prompt in prompts:
+            enc = pz.encode(prompt, add_special_patches=True)[:-1]
+            rest = prompt[len(pz.decode(enc)):]
+            patches.append(enc)
+            remaining.append(rest)
+            fixed.append([ord(c) for c in rest])
+        gen = self.generate_patches(patches, fixed, max_patch=max_patch, top_p=top_p, top_k=top_k, temperature=temperature,
+                                    seed=seed, batch=batch)
+        tunes = []
+        for prompt, bars in zip(prompts, gen):
+            tune = prompt
+            for patch in bars:   # the stop rules of generate_tune: the last patch may be the one that stopped the tune
+                if patch[0] == pz.eos_token_id:
+                    break
+                bar = pz.decode([patch])
+                if bar == "":
+                    break
+                tune += bar
+            tunes.append(tune)
+        return tunes
+
+    @torch.no_grad()
+    def generate_patches(self, prompt_patches, fixed_tokens=None, max_patch=PATCH_LENGTH, top_p=0.8, top_k=8, temperature=1.2,
+                         seed=None, batch=64):
+        """The bar loop of generate_tune on patches, for many tunes at once.
+
+        prompt_patches: one int [P_i, PATCH_SIZE] tensor (or nested list) per tune, starting with the start patch;
+        fixed_tokens: None or one list of character codes per tune that follow bos in the first generated bar (a prompt that
+        ends inside a bar).  Returns, per tune, the generated patches as lists of drawn character codes (each ends at its eos
+        when one was drawn, like `generate`), the last one possibly the end patch or empty bar that stopped the tune.  The
+        patch appended after a bar is bar2patch(fixed + bar) for the first bar and bar2patch(bar) after that.  `batch` tunes
+        share one pass of the loop; tunes are grouped by prompt length first, and the result is in input order.  See
+        generate_tunes for the seeding."""
+        n = len(prompt_patches)
+        pbs, cbs = self.patch_level_decoder.config.block_size, self.char_level_decoder.config.block_size
+        if max_patch > pbs:
+            raise ValueError(f"max_patch ({max_patch}) is above the patch decoder's block_size ({pbs})")
+        prompts = [torch.as_tensor(p, dtype=torch.int64).cpu().reshape(-1, PATCH_SIZE).tolist() for p in prompt_patches]
+        fixed = [[] for _ in range(n)] if fixed_tokens is None else [[int(c) for c in f] for f in fixed_tokens]
+        if len(fixed) != n:
+            raise ValueError("fixed_tokens needs one list per tune")
+        if any(len(p) == 0 for p in prompts):
+            raise ValueError("every prompt needs at least its start patch")
+        if any(len(f) + 1 > min(cbs, PATCH_SIZE) for f in fixed):
+            raise ValueError(f"at most {min(cbs, PATCH_SIZE) - 1} fixed characters per tune")
+        if seed is None:
+            seed = int(torch.randint(0, 2 ** 62, (1,)).item())
+        order = sorted(range(n), key=lambda i: len(prompts[i]))
+        out = [None] * n
+        # counters of the last call (tools/bench_tunesformer_generate.py): bars spelled (one per batch and patch position),
+        # character steps, device->host synchronisations, kernel launches, and launches / C-ABI calls of the character steps
+        self.last_generate_stats = stats = {"bars": 0, "char_steps": 0, "host_syncs": 0, "launches": 0, "char_launches": 0,
+                                            "char_calls": 0}
+        launches0 = ops.LAUNCHES
+        for s in range(0, n, max(1, int(batch))):
+            idx = order[s:s + max(1, int(batch))]
+            res = self._generate_batch([prompts[i] for i in idx], [fixed[i] for i in idx], idx, max_patch, float(top_p),
+                                       int(top_k), float(temperature), seed, stats)
+            for i, r in zip(idx, res):
+                out[i] = r
+        stats["launches"] = ops.LAUNCHES - launches0
+        return out
+
+    def _decode_states(self, B, device):
+        """Per-batch-size decode states of both decoders; the character level's first input rows ARE the patch level's hidden
+        rows (no copy between the two)."""
+        pd, cd = self.patch_level_decoder, self.char_level_decoder
+        key = ("tunes", B)
+        sp = pd._bufs.get(key)
+        if sp is None:
+            sp = pd._bufs[key] = _DecodeState(pd.config, B, pd.config.block_size, device)
+            sp.emb = torch.empty(B, pd.config.n_embd, device=device, dtype=torch.float32)
+            sp.hidden = torch.empty(B, pd.config.n_embd, device=device, dtype=torch.float32)
+        sc = cd._bufs.get(key)
+        if sc is None or sc.emb is not sp.hidden:
+            sc = cd._bufs[key] = _DecodeState(cd.config, B, cd.config.block_size, device)
+            sc.emb = sp.hidden
+            sc.sampler = (torch.zeros(1, device=device, dtype=torch.int64), torch.zeros(1, device=device, dtype=torch.int64),
+                          torch.zeros(B, device=device, dtype=torch.int64))
+        return sp, sc
+
+    def _generate_batch(self, prompts, fixed, row_ids, max_patch, top_p, top_k, temperature, seed, stats):
+        pz = Patchilizer()
+        eos = pz.eos_token_id
+        pd, cd = self.patch_level_decoder, self.char_level_decoder
+        dev = pd._arena["flat"].device
+        if dev.type != "cuda":
+            raise _C.AbcgptError("generate_patches: the model must be on a CUDA device (there is no CPU path)")
+        B, S = len(prompts), PATCH_SIZE
+        pd._ensure_device_state()
+        cd._ensure_device_state()
+        sp, sc = self._decode_states(B, dev)
+        V = cd.config.vocab_size
+        head = ("top_p", top_p, top_k if 0 < top_k < V else 0, temperature)
+        seed_t, counter_base, row_id = sc.sampler
+        seed_t.fill_(int(seed) & ((1 << 63) - 1))
+        row_id.copy_(torch.tensor(row_ids, dtype=torch.int64).pin_memory(), non_blocking=True)
+        # patch rows per position, all prompt patches uploaded at once; generated patches land at their position later
+        rows = torch.zeros(max_patch, B, S, dtype=torch.int64)
+        for i, p in enumerate(prompts):
+            k = min(len(p), max_patch)
+            rows[:k, i] = torch.tensor(p[:k], dtype=torch.int64)
+        patch_rows = rows.pin_memory().to(dev, non_blocking=True)
+        tunes = [len(p) for p in prompts]          # patches so far
+        done = [len(p) >= max_patch for p in prompts]
+        gen = [[] for _ in range(B)]
+        pos = torch.arange(S + 1, device=dev).view(-1, 1)
+        ops.set_pdl(True)
+        try:
+            for p in range(max_patch - 1):
+                if all(done):
+                    break
+                pd.embed_patches(patch_rows[p], sp.emb)
+                pd._decode_step(sp, p, False, None, inp="embed", hidden=True)
+                act = [i for i in range(B) if not done[i] and tunes[i] == p + 1]
+                if not act:
+                    continue                        # every live tune is still inside its prompt
+                # ---- spell one bar for the tunes whose last patch sits at position p
+                t0 = [1 + (len(fixed[i]) if not gen[i] else 0) for i in range(B)]   # first drawn position per tune
+                forced_rows = [i for i in act if t0[i] > 1]
+                n_steps = max(S - 1, max(t0[i] for i in act))
+                t0_dev = torch.tensor(t0, dtype=torch.int64).pin_memory().to(dev, non_blocking=True)
+                if forced_rows:   # a tune whose first bar has fixed characters takes them instead of the draws
+                    fx = torch.zeros(S + 1, B, dtype=torch.int64)
+                    for i in forced_rows:
+                        fx[1:t0[i], i] = torch.tensor(fixed[i], dtype=torch.int64)
+                    fx_dev = fx.pin_memory().to(dev, non_blocking=True)
+                    is_fixed = pos < t0_dev.view(1, -1)
+                    forced_end = max(t0[i] for i in forced_rows)
+                live = torch.zeros(B, dtype=torch.bool)
+                live[act] = True
+                live_dev = live.pin_memory().to(dev, non_blocking=True)
+                counter_base.fill_(p * S)
+                last = n_steps
+                launches0, calls0 = ops.LAUNCHES, ops.CALLS
+                for t in range(n_steps):
+                    cd._decode_step(sc, t, True, head, inp="first" if t == 0 else "tokens")
+                    stats["char_steps"] += 1
+                    if forced_rows and t + 1 < forced_end:
+                        sc.col[t + 1].copy_(torch.where(is_fixed[t + 1], fx_dev[t + 1], sc.col[t + 1]))
+                    if t % 8 == 7 and t + 1 < n_steps:
+                        seen = ((sc.col[:t + 2] == eos) & (pos[:t + 2] >= t0_dev.view(1, -1))).any(dim=0) | ~live_dev
+                        stats["host_syncs"] += 1
+                        if bool(seen.all()):
+                            last = t + 1
+                            break
+                stats["char_launches"] += ops.LAUNCHES - launches0
+                stats["char_calls"] += ops.CALLS - calls0
+                codes = sc.col[:last + 1].t().cpu().tolist()
+                stats["host_syncs"] += 1
+                stats["bars"] += 1
+                new_rows = {}
+                for i in act:
+                    drawn = codes[i][t0[i]:max(t0[i], S - 1) + 1]
+                    if eos in drawn:
+                        drawn = drawn[:drawn.index(eos) + 1]
+                    prefix = "".join(chr(c) for c in fixed[i]) if not gen[i] else ""
+                    gen[i].append(drawn)
+                    bar = pz.decode([drawn])
+                    if drawn[0] == eos or bar == "":
+                        done[i] = True
+                        continue
+                    tunes[i] += 1
+                    if tunes[i] >= max_patch:
+                        done[i] = True
+                    else:
+                        new_rows[i] = pz.bar2patch(prefix + bar)
+                if new_rows:
+                    blk = torch.zeros(B, S, dtype=torch.int64)
+                    for i, r in new_rows.items():
+                        blk[i] = torch.tensor(r, dtype=torch.int64)
+                    mask = torch.zeros(B, dtype=torch.bool)
+                    mask[list(new_rows)] = True
+                    blk_dev = blk.pin_memory().to(dev, non_blocking=True)
+                    mask_dev = mask.pin_memory().to(dev, non_blocking=True)
+                    patch_rows[p + 1].copy_(torch.where(mask_dev.view(-1, 1), blk_dev, patch_rows[p + 1]))
+        finally:
+            ops.set_pdl(False)
+        return gen
+
+    def load_reference_state_dict(self, sd):
+        """Loads a state dict of the reference's `TunesFormer` (tunesformer/utils.py:179-219, HF GPT-2 parameter names): the
+        patch level's `GPT2Model` under `patch_level_decoder.base.`, its `patch_embedding` Linear, the character level's
+        `GPT2LMHeadModel` under `char_level_decoder.base.` (`transformer.*` and `lm_head.weight`).  Conv1D weights ([in, out]
+        there) are transposed, the `attn.bias` / `attn.masked_bias` mask buffers are dropped, the patch level's tied lm_head
+        is set from its wte.  Any other missing or unexpected key, or a shape mismatch, raises with the key named (a
+        checkpoint with shared weights has another key set and is refused)."""
+        conv = GPT._HF_CONV1D
+        mask = (".attn.bias", ".attn.masked_bias")
+        src = {k: v for k, v in sd.items() if not k.endswith(mask)}
+        loads = []
+        for dec, own_prefix in ((self.patch_level_decoder, "patch"), (self.char_level_decoder, "char")):
+            own = dec.state_dict()
+            out = {}
+            for name, ref in own.items():
+                if name == "lm_head.weight" and own_prefix == "patch":
+                    continue   # tied to transformer.wte.weight
+                if own_prefix == "patch":
+                    key = ("patch_level_decoder." + name if name.startswith("patch_embedding.")
+                           else "patch_level_decoder.base." + name.replace("transformer.", "", 1))
+                elif name == "lm_head.weight":
+                    key = "char_level_decoder.base.lm_head.weight"
+                else:
+                    key = "char_level_decoder.base." + name
+                if key not in src:
+                    raise KeyError(f"missing key in the TunesFormer checkpoint: {key}")
+                v = src.pop(key).detach()
+                if key.endswith(conv):
+                    v = v.t()
+                if tuple(v.shape) != tuple(ref.shape):
+                    raise ValueError(f"shape mismatch for {key}: {tuple(v.shape)} vs {tuple(ref.shape)}")
+                out[name] = v.contiguous()
+            if own_prefix == "patch":
+                out["lm_head.weight"] = out["transformer.wte.weight"]
+            else:
+                wte = out["transformer.wte.weight"]
+                if not torch.equal(out["lm_head.weight"], wte):
+                    raise ValueError("char_level_decoder.base.lm_head.weight differs from its tied transformer.wte.weight")
+                out["lm_head.weight"] = wte
+            loads.append((dec, out))
+        if src:
+            raise KeyError(f"unexpected key in the TunesFormer checkpoint: {sorted(src)[0]}")
+        for dec, out in loads:   # nothing is changed unless the whole checkpoint matches
+            dec.load_state_dict(out)
+        return self
 
     def configure_optimizers(self, weight_decay, learning_rate, betas, device_type="cuda"):
         return _Optimizers([self.patch_level_decoder.configure_optimizers(weight_decay, learning_rate, betas, device_type),
