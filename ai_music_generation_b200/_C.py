@@ -34,6 +34,8 @@ _SIGNATURES = {
     "abcgpt_set_first_pos": (c_int, [_P, _P, _P, c_int, c_int, c_int, _P]),
     "abcgpt_pos_bwd": (c_int, [_P, _P, c_int, c_int, c_int, _P]),
     "abcgpt_onehot_bf16": (c_int, [_P, _P, c_int, c_int, c_int, _P]),
+    "abcgpt_add_pos_varlen": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, _P]),
+    "abcgpt_pos_bwd_varlen": (c_int, [_P, _P, _P, c_int, c_int, c_int, _P]),
     "abcgpt_layernorm_fwd": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int, c_int, _P]),
     "abcgpt_layernorm_fwd_resid": (c_int, [_P, _P, _P, _P, _P, _P, _P, _P, c_int, c_int, c_float, c_uint32, _P]),
     "abcgpt_layernorm_bwd": (c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, c_int, c_int, c_float, c_uint32, _P]),
@@ -41,9 +43,14 @@ _SIGNATURES = {
     "abcgpt_attn_bwd": (c_int, [_P, _P, _P, _P, _P, _P, c_int, c_int, c_int, c_float, c_uint32, _P]),
     "abcgpt_attn_fwd_hd": (c_int, [_P, _P, _P, c_int, c_int, c_int, c_int, c_float, c_uint32, _P]),
     "abcgpt_attn_bwd_hd": (c_int, [_P, _P, _P, _P, _P, _P, c_int, c_int, c_int, c_int, c_float, c_uint32, _P]),
+    "abcgpt_attn_varlen_fwd": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_int, c_int, c_float, c_uint32, _P]),
+    "abcgpt_attn_varlen_bwd": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int, c_int, c_int, c_int, c_int, c_float, c_uint32, _P]),
     "abcgpt_ce_fwd": (c_int, [_P, c_int64, _P, _P, c_int, c_int, _P]),
     "abcgpt_ce_finalize": (c_int, [_P, _P, c_int, _P, _P, _P]),
     "abcgpt_ce_bwd": (c_int, [_P, c_int64, _P, _P, _P, _P, c_int, c_int, _P]),
+    "abcgpt_ce_group_weights": (c_int, [_P, _P, c_int, c_int, c_int, _P, _P]),
+    "abcgpt_ce_finalize_weighted": (c_int, [_P, _P, c_int, _P, _P]),
+    "abcgpt_ce_bwd_weighted": (c_int, [_P, c_int64, _P, _P, _P, _P, c_int, c_int, _P]),
     "abcgpt_sumsq": (c_int, [_P, c_int64, _P, _P, _P]),
     "abcgpt_adamw": (c_int, [_P, _P, _P, _P, _P, c_int64, c_float, c_float, c_float, c_float, c_float, c_int, _P,
                              c_float, _P]),

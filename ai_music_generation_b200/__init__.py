@@ -8,7 +8,7 @@ from .model import GPT, GPTConfig  # noqa: F401
 from .optim import FusedAdamW  # noqa: F401
 from .ddp import DDP, TunesFormerDDP  # noqa: F401
 from .data import DeviceTokenStream  # noqa: F401
-from .tunesformer import Patchilizer, TunesFormerShaped  # noqa: F401
+from .tunesformer import Patchilizer, TunesFormerShaped, pack_tunes  # noqa: F401
 
 
 def clip_grad_norm_(model, max_norm):

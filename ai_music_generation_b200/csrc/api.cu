@@ -43,6 +43,13 @@ int abcgpt_pos_bwd(const float* dx, float* dwpe, int M, int T, int C, void* stre
 int abcgpt_onehot_bf16(const int64_t* tok, void* out, int M, int S_, int V, void* stream) {
   return onehot_bf16(tok, out, M, S_, V, S(stream));
 }
+int abcgpt_add_pos_varlen(const float* e, const float* wpe, float* x, const int32_t* cu_seqlens, int n_seqs, int total_rows, int C,
+                          void* stream) {
+  return add_pos_varlen(e, wpe, x, cu_seqlens, n_seqs, total_rows, C, S(stream));
+}
+int abcgpt_pos_bwd_varlen(const float* dx, float* dwpe, const int32_t* cu_seqlens, int n_seqs, int max_len, int C, void* stream) {
+  return pos_bwd_varlen(dx, dwpe, cu_seqlens, n_seqs, max_len, C, S(stream));
+}
 
 int abcgpt_layernorm_fwd(const float* x, const float* weight, const float* bias, void* y_bf16, float* y_f32,
                          float* mean, float* rstd, int M, int C, void* stream) {
@@ -78,6 +85,16 @@ int abcgpt_attn_bwd_hd(const void* qkv, const void* out, const void* dout, const
   if (head_size == 64) return abcgpt_attn_bwd(qkv, out, dout, lse, delta, dqkv, B, T, H, dropout_p, dropout_key, stream);
   return attn_bwd_hd(qkv, out, dout, lse, delta, dqkv, B, T, H, head_size, dropout_p, dropout_key, S(stream));
 }
+int abcgpt_attn_varlen_fwd(const void* qkv, void* out, float* lse, const int32_t* cu_seqlens, int n_seqs, int max_len,
+                           int total_rows, int H, int head_size, float dropout_p, uint32_t dropout_key, void* stream) {
+  return attn_varlen_fwd(qkv, out, lse, cu_seqlens, n_seqs, max_len, total_rows, H, head_size, dropout_p, dropout_key, S(stream));
+}
+int abcgpt_attn_varlen_bwd(const void* qkv, const void* out, const void* dout, const float* lse, float* delta, void* dqkv,
+                           const int32_t* cu_seqlens, int n_seqs, int max_len, int total_rows, int H, int head_size,
+                           float dropout_p, uint32_t dropout_key, void* stream) {
+  return attn_varlen_bwd(qkv, out, dout, lse, delta, dqkv, cu_seqlens, n_seqs, max_len, total_rows, H, head_size, dropout_p,
+                         dropout_key, S(stream));
+}
 
 int abcgpt_ce_fwd(const void* logits, int64_t ldl, const int64_t* targets, float* row_loss, int M, int V,
                   void* stream) {
@@ -90,6 +107,17 @@ int abcgpt_ce_finalize(const float* row_loss, const int64_t* targets, int M, flo
 int abcgpt_ce_bwd(const void* logits, int64_t ldl, const int64_t* targets, const float* loss_sum_count,
                   const float* grad_loss, void* dlogits, int M, int V, void* stream) {
   return ce_bwd(logits, ldl, targets, loss_sum_count, grad_loss, dlogits, M, V, S(stream));
+}
+int abcgpt_ce_group_weights(const int64_t* targets, const int32_t* row_group, int n_groups, int M, int V, float* weights,
+                            void* stream) {
+  return ce_group_weights(targets, row_group, n_groups, M, V, weights, S(stream));
+}
+int abcgpt_ce_finalize_weighted(const float* row_loss, const float* weights, int M, float* loss, void* stream) {
+  return ce_finalize_weighted(row_loss, weights, M, loss, S(stream));
+}
+int abcgpt_ce_bwd_weighted(const void* logits, int64_t ldl, const int64_t* targets, const float* weights, const float* grad_loss,
+                           void* dlogits, int M, int V, void* stream) {
+  return ce_bwd_weighted(logits, ldl, targets, weights, grad_loss, dlogits, M, V, S(stream));
 }
 
 int abcgpt_sumsq(const float* g, int64_t n, float* out, float* workspace, void* stream) {

@@ -599,6 +599,115 @@ __global__ void onehot_bf16_kernel(const int64_t* __restrict__ tok, __nv_bfloat1
   out[(m * S + s) * V + t] = __float2bfloat16(1.0f);
 }
 
+// ---- packed sequences (TunesFormer training on tunes of different lengths) ------------------------------------------------
+// sequence of packed row m: the s with cu[s] <= m < cu[s+1] (cu ascending, cu[0] = 0)
+__device__ __forceinline__ int seq_of_row(const int32_t* __restrict__ cu, int n_seqs, int m) {
+  int lo = 0, hi = n_seqs - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (__ldg(cu + mid) <= m) lo = mid;
+    else hi = mid - 1;
+  }
+  return lo;
+}
+// x[m,:] = e[m,:] + wpe[m - cu[seq(m)],:]: positions restart at every sequence; one block per row
+__global__ void __launch_bounds__(128)
+add_pos_varlen_kernel(const float4* __restrict__ e, const float4* __restrict__ wpe, float4* __restrict__ x,
+                      const int32_t* __restrict__ cu, int n_seqs, int C4) {
+  const int m = blockIdx.x;
+  const int t = m - __ldg(cu + seq_of_row(cu, n_seqs, m));
+  const long long row = static_cast<long long>(m) * C4;
+  for (int c = threadIdx.x; c < C4; c += blockDim.x) {
+    const float4 a = __ldg(e + row + c);
+    const float4 b = __ldg(wpe + static_cast<long long>(t) * C4 + c);
+    x[row + c] = make_float4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w);
+  }
+}
+// dwpe[t,:] += sum over s with len_s > t of dx[cu[s] + t,:]: one thread per (t, 4 columns), sequences summed in index order
+// (no atomics: the position gradient is bitwise reproducible)
+__global__ void __launch_bounds__(128)
+pos_bwd_varlen_kernel(const float4* __restrict__ dx, float4* __restrict__ dwpe, const int32_t* __restrict__ cu, int n_seqs, int C4) {
+  const int t = blockIdx.x;
+  const int c = blockIdx.y * blockDim.x + threadIdx.x;
+  if (c >= C4) return;
+  float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+  int r0 = __ldg(cu);
+  for (int s = 0; s < n_seqs; ++s) {
+    const int r1 = __ldg(cu + s + 1);
+    if (t < r1 - r0) {
+      const float4 v = __ldg(dx + static_cast<long long>(r0 + t) * C4 + c);
+      acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
+    }
+    r0 = r1;
+  }
+  float4* o = dwpe + static_cast<long long>(t) * C4 + c;
+  const float4 p = *o;
+  *o = make_float4(p.x + acc.x, p.y + acc.y, p.z + acc.z, p.w + acc.w);
+}
+// w[m] = 1 / (n_groups * valid rows of group(m)) for a valid target, else 0 (one block: shared-memory integer counts)
+__global__ void __launch_bounds__(1024)
+ce_group_weights_kernel(const int64_t* __restrict__ targets, const int32_t* __restrict__ row_group, int n_groups, int M, int V,
+                        float* __restrict__ w) {
+  extern __shared__ int cnt[];
+  for (int g = threadIdx.x; g < n_groups; g += blockDim.x) cnt[g] = 0;
+  __syncthreads();
+  for (int i = threadIdx.x; i < M; i += blockDim.x) {
+    const long long t = __ldg(targets + i);
+    const int g = __ldg(row_group + i);
+    if (t >= 0 && t < V && g >= 0 && g < n_groups) atomicAdd(&cnt[g], 1);
+  }
+  __syncthreads();
+  const float ng = static_cast<float>(n_groups);
+  for (int i = threadIdx.x; i < M; i += blockDim.x) {
+    const long long t = __ldg(targets + i);
+    const int g = __ldg(row_group + i);
+    w[i] = (t >= 0 && t < V && g >= 0 && g < n_groups) ? 1.0f / (ng * static_cast<float>(cnt[g])) : 0.f;
+  }
+}
+// loss[0] = sum_m w[m] * row_loss[m]; fixed assignment of rows to threads => bitwise reproducible
+__global__ void __launch_bounds__(1024)
+ce_finalize_weighted_kernel(const float* __restrict__ row_loss, const float* __restrict__ w, int M, float* __restrict__ loss) {
+  __shared__ float ssum[32];
+  float s = 0.f;
+  for (int i = threadIdx.x; i < M; i += blockDim.x) s += __ldg(w + i) * row_loss[i];
+  s = warp_sum(s);
+  if ((threadIdx.x & 31) == 0) ssum[threadIdx.x >> 5] = s;
+  __syncthreads();
+  if (threadIdx.x < 32) {
+    s = warp_sum(ssum[threadIdx.x]);
+    if (threadIdx.x == 0) loss[0] = s;
+  }
+}
+// dlogits = (softmax - onehot) * grad_loss * w[m]; zero for ignored rows and the padding columns V..ldl
+__global__ void __launch_bounds__(256)
+ce_bwd_weighted_kernel(const __nv_bfloat16* __restrict__ logits, long long ldl, const int64_t* __restrict__ targets,
+                       const float* __restrict__ w, const float* __restrict__ grad_loss, __nv_bfloat16* __restrict__ dlogits,
+                       int M, int V) {
+  const int lane = threadIdx.x & 31;
+  const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (row >= M) return;
+  const long long tgt = __ldg(targets + row);
+  const __nv_bfloat16* lr = logits + static_cast<long long>(row) * ldl;
+  __nv_bfloat16* dr = dlogits + static_cast<long long>(row) * ldl;
+  const bool valid = tgt >= 0 && tgt < V;
+  const float scale = valid ? __ldg(grad_loss) * __ldg(w + row) : 0.f;
+  float mx = -INFINITY;
+  for (int c = lane; c < V; c += 32) mx = fmaxf(mx, __bfloat162float(lr[c]));
+  mx = warp_max(mx);
+  float s = 0.f;
+  for (int c = lane; c < V; c += 32) s += __expf(__bfloat162float(lr[c]) - mx);
+  s = warp_sum(s);
+  const float inv = 1.0f / s;
+  for (int c = lane; c < static_cast<int>(ldl); c += 32) {
+    float g = 0.f;
+    if (c < V && valid) {
+      const float p = __expf(__bfloat162float(lr[c]) - mx) * inv;
+      g = (p - (c == tgt ? 1.f : 0.f)) * scale;
+    }
+    dr[c] = __float2bfloat16_rn(g);
+  }
+}
+
 }  // namespace
 
 int embed_fwd(const int64_t* idx, const float* wte, const float* wpe, float* x, int M, int T, int C, int V, float drop_p,
@@ -698,6 +807,40 @@ int ce_bwd(const void* logits, long long ldl, const int64_t* targets, const floa
                                                  loss_sum_count, grad_loss, reinterpret_cast<__nv_bfloat16*>(dlogits), M,
                                                  V);
   return launch_status("ce_bwd_kernel");
+}
+
+int add_pos_varlen(const float* e, const float* wpe, float* x, const int32_t* cu_seqlens, int n_seqs, int total_rows, int C,
+                   cudaStream_t stream) {
+  ABCGPT_CHECK_ARG(e && wpe && x && cu_seqlens && n_seqs > 0 && total_rows > 0 && C % 4 == 0, "add_pos_varlen: bad arguments");
+  add_pos_varlen_kernel<<<total_rows, 128, 0, stream>>>(reinterpret_cast<const float4*>(e), reinterpret_cast<const float4*>(wpe),
+                                                       reinterpret_cast<float4*>(x), cu_seqlens, n_seqs, C / 4);
+  return launch_status("add_pos_varlen_kernel");
+}
+int pos_bwd_varlen(const float* dx, float* dwpe, const int32_t* cu_seqlens, int n_seqs, int max_len, int C, cudaStream_t stream) {
+  ABCGPT_CHECK_ARG(dx && dwpe && cu_seqlens && n_seqs > 0 && max_len > 0 && C % 4 == 0, "pos_bwd_varlen: bad arguments");
+  const int C4 = C / 4;
+  pos_bwd_varlen_kernel<<<dim3(max_len, (C4 + 127) / 128), 128, 0, stream>>>(reinterpret_cast<const float4*>(dx),
+                                                                              reinterpret_cast<float4*>(dwpe), cu_seqlens, n_seqs, C4);
+  return launch_status("pos_bwd_varlen_kernel");
+}
+int ce_group_weights(const int64_t* targets, const int32_t* row_group, int n_groups, int M, int V, float* w, cudaStream_t stream) {
+  ABCGPT_CHECK_ARG(targets && row_group && w && M > 0 && V > 0, "ce_group_weights: bad arguments");
+  ABCGPT_CHECK_ARG(n_groups > 0 && n_groups <= kMaxCeGroups, "ce_group_weights: n_groups must lie in [1, %d] (got %d)", kMaxCeGroups,
+                   n_groups);
+  ce_group_weights_kernel<<<1, 1024, n_groups * sizeof(int), stream>>>(targets, row_group, n_groups, M, V, w);
+  return launch_status("ce_group_weights_kernel");
+}
+int ce_finalize_weighted(const float* row_loss, const float* weights, int M, float* loss, cudaStream_t stream) {
+  ABCGPT_CHECK_ARG(row_loss && weights && loss && M > 0, "ce_finalize_weighted: bad arguments");
+  ce_finalize_weighted_kernel<<<1, 1024, 0, stream>>>(row_loss, weights, M, loss);
+  return launch_status("ce_finalize_weighted_kernel");
+}
+int ce_bwd_weighted(const void* logits, long long ldl, const int64_t* targets, const float* weights, const float* grad_loss,
+                    void* dlogits, int M, int V, cudaStream_t stream) {
+  ABCGPT_CHECK_ARG(logits && targets && weights && grad_loss && dlogits && M > 0 && V > 0 && ldl >= V, "ce_bwd_weighted: bad arguments");
+  ce_bwd_weighted_kernel<<<(M + 7) / 8, 256, 0, stream>>>(reinterpret_cast<const __nv_bfloat16*>(logits), ldl, targets, weights,
+                                                          grad_loss, reinterpret_cast<__nv_bfloat16*>(dlogits), M, V);
+  return launch_status("ce_bwd_weighted_kernel");
 }
 
 int sumsq(const float* g, long long n, float* out, float* workspace, cudaStream_t stream) {

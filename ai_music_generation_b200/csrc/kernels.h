@@ -20,6 +20,10 @@ int add_pos(const float* e, const float* wpe, float* x, int M, int T, int C, cud
 int set_first_pos(const float* first, const float* wpe, float* x, int B, int T, int C, cudaStream_t stream);
 int pos_bwd(const float* dx, float* dwpe, int M, int T, int C, cudaStream_t stream);
 int onehot_bf16(const int64_t* tok, void* out, int M, int S, int V, cudaStream_t stream);
+// packed sequences: cu_seqlens int32 [n_seqs + 1] row offsets
+int add_pos_varlen(const float* e, const float* wpe, float* x, const int32_t* cu_seqlens, int n_seqs, int total_rows, int C,
+                   cudaStream_t stream);
+int pos_bwd_varlen(const float* dx, float* dwpe, const int32_t* cu_seqlens, int n_seqs, int max_len, int C, cudaStream_t stream);
 
 int layernorm_fwd(const float* x, const float* weight, const float* bias, void* y_bf16, float* y_f32, float* mean,
                   float* rstd, int M, int C, cudaStream_t stream);
@@ -40,6 +44,12 @@ int attn_fwd_hd(const void* qkv, void* out, float* lse, int B, int T, int H, int
 int attn_bwd_hd(const void* qkv, const void* out, const void* dout, const float* lse, float* delta, void* dqkv, int B, int T,
                 int H, int D, float drop_p, uint32_t drop_key, cudaStream_t stream);
 int attn_decode_hd(const void* qkv_row, void* cache, void* out, int B, int Tmax, int t, int H, int D, cudaStream_t stream);
+// csrc/attn_varlen.cu: packed sequences, head sizes 32, 64 and 128
+int attn_varlen_fwd(const void* qkv, void* out, float* lse, const int32_t* cu_seqlens, int n_seqs, int max_len, int total_rows,
+                    int H, int D, float drop_p, uint32_t drop_key, cudaStream_t stream);
+int attn_varlen_bwd(const void* qkv, const void* out, const void* dout, const float* lse, float* delta, void* dqkv,
+                    const int32_t* cu_seqlens, int n_seqs, int max_len, int total_rows, int H, int D, float drop_p,
+                    uint32_t drop_key, cudaStream_t stream);
 
 int ce_fwd(const void* logits, long long ldl, const int64_t* targets, float* row_loss, int M, int V,
            cudaStream_t stream);
@@ -47,6 +57,11 @@ int ce_finalize(const float* row_loss, const int64_t* targets, int M, float* los
                 cudaStream_t stream);
 int ce_bwd(const void* logits, long long ldl, const int64_t* targets, const float* loss_sum_count,
            const float* grad_loss, void* dlogits, int M, int V, cudaStream_t stream);
+constexpr int kMaxCeGroups = 12288;   // ce_group_weights: one int counter per group in 48 KB of shared memory
+int ce_group_weights(const int64_t* targets, const int32_t* row_group, int n_groups, int M, int V, float* w, cudaStream_t stream);
+int ce_finalize_weighted(const float* row_loss, const float* weights, int M, float* loss, cudaStream_t stream);
+int ce_bwd_weighted(const void* logits, long long ldl, const int64_t* targets, const float* weights, const float* grad_loss,
+                    void* dlogits, int M, int V, cudaStream_t stream);
 
 int sumsq(const float* g, long long n, float* out, float* workspace, cudaStream_t stream);
 int adamw(float* p, const float* g, float* m, float* v, void* shadow_bf16, long long n, float lr, float beta1,

@@ -19,6 +19,7 @@ There is no CPU or eager-PyTorch fallback: a missing extension or a non-CUDA ten
 """
 from __future__ import annotations
 
+import itertools
 import math
 import os
 from dataclasses import dataclass
@@ -134,6 +135,9 @@ class _Buffers:
         self.tgt = torch.empty(B, T, device=device, dtype=torch.int64)   # hold raw pointers
         self.gl = e(1, dt=f32)
         self.hidden = None   # fp32 ln_f output, allocated on first use by the hierarchical (inputs_embeds) path
+        self.cu = None       # packed calls: device sequence table (int32 row offsets) and its (n_seqs, max_len), or None
+        self.varlen = None
+        self.weighted = False   # the loss of the last forward was the per-group mean (weights in self.w)
         self.plans = {}
         self.gen = 0         # bumped by every forward into these buffers; an autograd node remembers the value it saw
         if keep_activations:
@@ -146,6 +150,44 @@ class _Buffers:
             self.dh = e(M, 4 * C)
             self.delta = e(B, H, T, dt=f32)
             self.dlogits = e(M, self.Vpad)
+
+    # packed calls (GPT.forward_hidden_packed, forward_with_first with row groups): the buffers are allocated for the largest
+    # call so far and cut to the rows of each call, so that a run over changing mixes of sequences reuses one buffer set
+    _ROW_ATTRS = ("x", "xmid", "ln1", "ln2", "qkv", "att", "h", "g", "lnf", "ybr", "logits", "row_loss", "hidden", "w", "dx",
+                  "dxb", "dxb2", "dln", "datt", "dqkv", "dh", "dlogits")
+    _SEQ_ATTRS = ("lse", "delta", "idx", "tgt", "last_logits")
+    _COL_ATTRS = ("stat", "statf")
+
+    def add_full(self, name, tensor):
+        """Register a capacity-sized buffer allocated after construction (cut by set_batch like the others)."""
+        setattr(self, name, tensor)
+        self._full[name] = tensor
+
+    def set_batch(self, B):
+        """Cut every per-row buffer to its first B sequences (B * T rows); the full buffers stay allocated."""
+        if not hasattr(self, "_full"):
+            self._full = {k: getattr(self, k, None) for k in self._ROW_ATTRS + self._SEQ_ATTRS + self._COL_ATTRS}
+        M = B * self.T
+        for k, v in self._full.items():
+            if v is None:
+                continue
+            if k in self._COL_ATTRS:
+                cut = lambda t: t[:, :M]  # noqa: E731
+            else:
+                n = B if k in self._SEQ_ATTRS else M
+                cut = lambda t, n=n: t[:n]  # noqa: E731
+            setattr(self, k, [cut(t) for t in v] if isinstance(v, list) else cut(v))
+        self.B, self.M = B, M
+
+
+@dataclass
+class _Pack:
+    """How the rows of a packed call are organised.  seq_lens: the rows are these sequences end to end (positions restart and
+    attention stays inside each one); row_group / n_groups: int32 group of every target row, the loss is the mean over groups
+    of each group's token mean (the reference's per-tune loss)."""
+    seq_lens: tuple = None
+    row_group: torch.Tensor = None
+    n_groups: int = 0
 
 
 class _DecodeState:
@@ -222,9 +264,9 @@ class _GPTEmbedsStep(torch.autograd.Function):
     embedding [B,C] next to token ids.  Returns (loss, fp32 ln_f output); either may be unused."""
 
     @staticmethod
-    def forward(ctx, anchor, model, x_in, idx, targets, want_hidden, mode):
+    def forward(ctx, anchor, model, x_in, idx, targets, want_hidden, mode, pack):
         bufs = model._forward_plan(idx, targets, keep_activations=True, embeds=x_in if mode == 1 else None,
-                                   first=x_in if mode == 2 else None, want_hidden=want_hidden)
+                                   first=x_in if mode == 2 else None, want_hidden=want_hidden, pack=pack)
         B, T, C = bufs.B, bufs.T, model.config.n_embd
         idx_b = None
         if mode == 2:  # the wte gradient must skip position 0 (its embedding was replaced): abcgpt_embed_bwd skips ids < 0
@@ -244,7 +286,7 @@ class _GPTEmbedsStep(torch.autograd.Function):
         d_hidden = grad_hidden.reshape(B * T, C).float() if ctx.want_hidden and ctx.targets is None else None
         dx = ctx.model._backward_plan(ctx.bufs, ctx.idx, ctx.targets, grad_loss, ctx.drop, d_hidden=d_hidden, mode=ctx.mode)
         gx = dx.view(B, T, C).clone() if ctx.mode == 1 else dx.view(B, T, C)[:, 0, :].clone()
-        return None, None, gx, None, None, None, None
+        return None, None, gx, None, None, None, None, None
 
 
 class GPT(nn.Module):
@@ -396,6 +438,36 @@ class GPT(nn.Module):
             self._bufs[key] = _Buffers(self.config, B, T, self._arena["flat"].device, keep)
         return self._bufs[key]
 
+    _PACK_ROWS = 1024   # capacity of the buffers of packed calls: a multiple of this many rows, with 1/8 headroom when grown
+
+    def _packed_buffers(self, B, T, keep, want_hidden, pack):
+        """Buffers of a packed call of B sequences of T rows.  One set per (T, keep), cut to B (see _Buffers.set_batch) and
+        replaced by a larger one only when a call needs more rows than it holds, so a run over changing mixes of similar size
+        allocates a buffer set a few times at most.  The sequence table is staged into the set's device buffer `cu`."""
+        key = ("packed", keep, T)
+        bufs = self._bufs.get(key)
+        device = self._arena["flat"].device
+        if bufs is None or bufs.cap < B:
+            rows = _round_up(B * T + (B * T) // 8, self._PACK_ROWS)
+            bcap = -(-rows // T)
+            self._bufs.pop(key, None)
+            bufs = self._bufs[key] = _Buffers(self.config, bcap, T, device, keep)
+            bufs.set_batch(bcap)
+            bufs.cap = bcap
+            bufs.cu = torch.zeros(bcap * T + 1, device=device, dtype=torch.int32)
+        if want_hidden and bufs._full["hidden"] is None:
+            bufs.add_full("hidden", torch.empty(bufs.cap * T, self.config.n_embd, device=device, dtype=torch.float32))
+        if pack.row_group is not None and bufs._full["w"] is None:
+            bufs.add_full("w", torch.empty(bufs.cap * T, device=device, dtype=torch.float32))
+        bufs.set_batch(B)
+        bufs.varlen = None
+        if pack.seq_lens is not None:
+            lens = list(pack.seq_lens)
+            cu = torch.tensor([0, *itertools.accumulate(lens)], dtype=torch.int32, pin_memory=True)
+            bufs.cu[:len(lens) + 1].copy_(cu, non_blocking=True)   # stream-ordered behind every earlier reader of the table
+            bufs.varlen = (len(lens), max(lens))
+        return bufs
+
     # Programmatic dependent launch pays when the kernels of a step are short (baby GPT, 16 k tokens x 384: 3.02 -> 2.88 ms per
     # step) and costs when every kernel fills the GPU for 25-400 us (GPT-2-small shape at 32 k tokens: -1.8 %), see DESIGN 4.5
     _PDL_MAX_WORK = 8 * 1024 * 1024   # tokens x n_embd
@@ -408,14 +480,14 @@ class GPT(nn.Module):
         if patches is not None:
             bufs.plans[plan_key] = (plan, patches)
 
-    def _forward_plan(self, idx, targets, keep_activations, embeds=None, first=None, want_hidden=False):
+    def _forward_plan(self, idx, targets, keep_activations, embeds=None, first=None, want_hidden=False, pack=None):
         src = idx if idx is not None else embeds
         pdl = src.shape[0] * src.shape[1] * self.config.n_embd <= self._PDL_MAX_WORK
         if not pdl:
-            return self._forward_plan_impl(idx, targets, keep_activations, embeds, first, want_hidden)
+            return self._forward_plan_impl(idx, targets, keep_activations, embeds, first, want_hidden, pack)
         ops.set_pdl(True)
         try:
-            return self._forward_plan_impl(idx, targets, keep_activations, embeds, first, want_hidden)
+            return self._forward_plan_impl(idx, targets, keep_activations, embeds, first, want_hidden, pack)
         finally:
             ops.set_pdl(False)
 
@@ -429,10 +501,11 @@ class GPT(nn.Module):
         finally:
             ops.set_pdl(False)
 
-    def _forward_plan_impl(self, idx, targets, keep_activations, embeds=None, first=None, want_hidden=False):
+    def _forward_plan_impl(self, idx, targets, keep_activations, embeds=None, first=None, want_hidden=False, pack=None):
         """embeds (fp32 [B,T,C]): the decoder is fed embeddings from another network (HF inputs_embeds) instead of token ids;
         first (fp32 [B,C]): token ids, but the first position's embedding is replaced (TunesFormer char decoder);
-        want_hidden: also keep the fp32 ln_f output in bufs.hidden (HF last_hidden_state)."""
+        want_hidden: also keep the fp32 ln_f output in bufs.hidden (HF last_hidden_state);
+        pack (_Pack): a packed call (grow-only buffers; varlen attention / positions and / or the per-group loss)."""
         cfg = self.config
         # Dropout (model.py:39-40,85,129 + SDPA dropout_p :64): counter-based masks, one key per site, derived from a seed
         # drawn from torch's CPU generator for every forward (reproducible under torch.manual_seed); the backward plan
@@ -452,7 +525,10 @@ class GPT(nn.Module):
         top = self._arena["top"]
         B, T = src.shape[0], src.shape[1]
         assert T <= cfg.block_size, f"Cannot forward sequence of length {T}, block size is only {cfg.block_size}"
-        bufs = self._act_buffers(B, T, keep_activations)
+        if pack is not None and p_drop != 0.0:
+            raise _C.AbcgptError("packed calls: dropout is not implemented (use dropout=0)")
+        bufs = self._act_buffers(B, T, keep_activations) if pack is None else self._packed_buffers(B, T, keep_activations,
+                                                                                                    want_hidden, pack)
         bufs.gen += 1
         C, H, V = cfg.n_embd, cfg.n_head, cfg.vocab_size
         if idx is not None:
@@ -478,7 +554,10 @@ class GPT(nn.Module):
         if embeds is not None:
             if p_drop != 0.0:
                 raise _C.AbcgptError("inputs_embeds path: embedding dropout is not implemented (use dropout=0)")
-            ops.add_pos(embeds.contiguous().view(B * T, C), top["wpe"][0], bufs.x[0], T)
+            if bufs.varlen is not None:
+                ops.add_pos_varlen(embeds.contiguous().view(B * T, C), top["wpe"][0], bufs.x[0], bufs.cu, bufs.varlen[0])
+            else:
+                ops.add_pos(embeds.contiguous().view(B * T, C), top["wpe"][0], bufs.x[0], T)
         else:
             ops.embed_fwd(idx, top["wte"][0], top["wpe"][0], bufs.x[0], T, drop_p=p_drop, drop_key=keys[0])
             if first is not None:
@@ -492,8 +571,11 @@ class GPT(nn.Module):
             b = lambda name: None if lw[name] is None else lw[name][0]  # noqa: E731
             ops.layernorm_fwd(x_in, lw["ln_1.weight"][0], b("ln_1.bias"), bufs.ln1[k], st[0], st[1])
             ops.gemm(bufs.ln1[k], lw["attn.c_attn.weight"][1], epilogue=ops.EPI_BF16, out=bufs.qkv[k], bias=b("attn.c_attn.bias"))
-            ops.attn_fwd(bufs.qkv[k], bufs.att[k], bufs.lse[k], B, T, H, drop_p=p_drop, drop_key=keys[1 + 3 * li],
-                         head_size=self._head_size)
+            if bufs.varlen is not None:
+                ops.attn_varlen_fwd(bufs.qkv[k], bufs.att[k], bufs.lse[k], bufs.cu, *bufs.varlen, H, self._head_size)
+            else:
+                ops.attn_fwd(bufs.qkv[k], bufs.att[k], bufs.lse[k], B, T, H, drop_p=p_drop, drop_key=keys[1 + 3 * li],
+                             head_size=self._head_size)
             # attention branch: the K = 768 projection with the residual add in its epilogue was bound by its fp32 residual
             # loads (0.080 ms against 0.038 ms of HBM time at cfg3); the add rides on the LayerNorm pass that follows instead
             # (x_mid = x + drop(c_proj(att)), ln_2(x_mid) in one kernel; the bf16 branch output mostly stays in L2 in between)
@@ -515,10 +597,16 @@ class GPT(nn.Module):
             pass  # a decoder without a head (TunesFormer's patch level): the caller reads bufs.hidden
         elif targets is not None:
             ops.gemm(bufs.lnf, wte_bf16, N=bufs.Vpad, epilogue=ops.EPI_BF16, out=bufs.logits)
-            ops.ce_fwd(bufs.logits, targets.contiguous().view(-1), bufs.row_loss, bufs.sum_count, bufs.loss, V)
+            if pack is not None and pack.row_group is not None:
+                tflat = targets.contiguous().view(-1)
+                ops.ce_group_weights(tflat, pack.row_group, pack.n_groups, bufs.w, V)
+                ops.ce_fwd_weighted(bufs.logits, tflat, bufs.w, bufs.row_loss, bufs.loss, V)
+            else:
+                ops.ce_fwd(bufs.logits, targets.contiguous().view(-1), bufs.row_loss, bufs.sum_count, bufs.loss, V)
         else:  # last position only (model.py:190): strided A operand, no gather copy
             a = bufs.lnf.view(B, T * C)[:, (T - 1) * C:]
             ops.gemm(a, wte_bf16, M=B, N=bufs.Vpad, K=C, epilogue=ops.EPI_BF16, out=bufs.last_logits)
+        bufs.weighted = pack is not None and pack.row_group is not None
         if plan_key is not None:
             self._store_plan(bufs, plan_key, keys, p_drop)
         return bufs
@@ -563,7 +651,10 @@ class GPT(nn.Module):
             ops.begin_record()
         wte, wte_bf16, dwte = top["wte"]
         if targets is not None:
-            ops.ce_bwd(bufs.logits, tflat, bufs.sum_count, gl, bufs.dlogits, V)
+            if bufs.weighted:
+                ops.ce_bwd_weighted(bufs.logits, tflat, bufs.w, gl, bufs.dlogits, V)
+            else:
+                ops.ce_bwd(bufs.logits, tflat, bufs.sum_count, gl, bufs.dlogits, V)
             # lm_head: dW[V,C] += dlogits^T lnf ; d(lnf) = dlogits W
             ops.gemm(bufs.dlogits, bufs.lnf, a_mn=True, b_mn=True, M=V, N=C, K=M, epilogue=ops.EPI_F32_RED, out=dwte)
             ops.gemm(bufs.dlogits, wte_bf16, b_mn=True, M=M, N=C, K=V, epilogue=ops.EPI_BF16, out=bufs.dln)
@@ -627,8 +718,12 @@ class GPT(nn.Module):
             if held is not None:   # the previous layer's bucket goes out beside this layer's attention backward (see below)
                 ops.record_callback(lambda li_=held: sync.layer_done(li_))
                 held = None
-            ops.attn_bwd(bufs.qkv[li], bufs.att[li], bufs.datt, bufs.lse[li], bufs.delta, bufs.dqkv, B, T, H,
-                         drop_p=p_drop, drop_key=keys[1 + 3 * li], head_size=self._head_size)
+            if bufs.varlen is not None:
+                ops.attn_varlen_bwd(bufs.qkv[li], bufs.att[li], bufs.datt, bufs.lse[li], bufs.delta, bufs.dqkv, bufs.cu,
+                                    *bufs.varlen, H, self._head_size)
+            else:
+                ops.attn_bwd(bufs.qkv[li], bufs.att[li], bufs.datt, bufs.lse[li], bufs.delta, bufs.dqkv, B, T, H,
+                             drop_p=p_drop, drop_key=keys[1 + 3 * li], head_size=self._head_size)
             wgrad(bufs.dqkv, bufs.ln1[li], "attn.c_attn", J3)
             ops.gemm(bufs.dqkv, lw["attn.c_attn.weight"][1], b_mn=True, epilogue=ops.EPI_BF16, out=bufs.dln)
             before_overwrite(J0)
@@ -643,7 +738,9 @@ class GPT(nn.Module):
                 else:
                     ops.record_callback(lambda li=li: sync.layer_done(li))
         before_overwrite(J3)           # join: everything the side stream was given has finished before the backward returns
-        if mode == 1:
+        if mode == 1 and bufs.varlen is not None:
+            ops.pos_bwd_varlen(dx, top["wpe"][2], bufs.cu, *bufs.varlen)
+        elif mode == 1:
             ops.pos_bwd(dx, top["wpe"][2], T)
         else:
             ops.embed_bwd(idx.contiguous().view(-1), dx, dwte, top["wpe"][2], T, drop_p=p_drop, drop_key=keys[0])
@@ -691,15 +788,35 @@ class GPT(nn.Module):
                 bufs = self._forward_plan(None, None, keep_activations=False, embeds=inputs_embeds, want_hidden=True)
             return bufs.hidden.view(*inputs_embeds.shape).clone()
         anchor = self._anchor_tensor(inputs_embeds.device)
-        _, hidden = _GPTEmbedsStep.apply(anchor, self, inputs_embeds, None, None, True, 1)
+        _, hidden = _GPTEmbedsStep.apply(anchor, self, inputs_embeds, None, None, True, 1, None)
         return hidden
 
-    def forward_with_first(self, idx, first_embeds, targets):
+    def forward_hidden_packed(self, inputs_embeds, seq_lens):
+        """`forward_hidden` over sequences of different lengths packed end to end: inputs_embeds fp32 [sum(seq_lens), C], every
+        sequence encoded as if alone (positions restart at each one, causal attention never crosses into another).  Returns the
+        fp32 ln_f output [sum(seq_lens), C], differentiable w.r.t. inputs_embeds."""
+        lens = tuple(int(n) for n in seq_lens)
+        M, C = inputs_embeds.shape
+        if not lens or min(lens) < 1 or max(lens) > self.config.block_size or sum(lens) != M:
+            raise ValueError(f"seq_lens must be >= 1, <= block_size ({self.config.block_size}) and sum to the {M} rows")
+        pack = _Pack(seq_lens=lens)
+        x = inputs_embeds.view(M, 1, C)   # one row per "sequence" of the buffer layout; the sequences themselves come from pack
+        if not (torch.is_grad_enabled() and self._arena["params"][0].requires_grad):
+            with torch.no_grad():
+                bufs = self._forward_plan(None, None, keep_activations=False, embeds=x, want_hidden=True, pack=pack)
+            return bufs.hidden.view(M, C).clone()
+        _, hidden = _GPTEmbedsStep.apply(self._anchor_tensor(inputs_embeds.device), self, x, None, None, True, 1, pack)
+        return hidden.view(M, C)
+
+    def forward_with_first(self, idx, first_embeds, targets, row_group=None, n_groups=None):
         """HF `GPT2LMHeadModel(inputs_embeds=cat(first, wte(idx)[:, 1:]), labels=...)`: token embeddings with the first
         position replaced by `first_embeds` [B, C]; returns the loss over `targets` (already shifted by the caller,
-        ignore_index = -1), differentiable w.r.t. first_embeds (tunesformer/utils.py:120-154)."""
+        ignore_index = -1), differentiable w.r.t. first_embeds (tunesformer/utils.py:120-154).
+        row_group (int32 [B * T], device) / n_groups: the loss is the mean over the groups of each group's mean over its valid
+        targets instead of one mean over all of them (a packed batch of tunes; buffers by capacity bucket)."""
+        pack = None if row_group is None else _Pack(row_group=row_group.contiguous(), n_groups=int(n_groups))
         anchor = self._anchor_tensor(idx.device)
-        loss, _ = _GPTEmbedsStep.apply(anchor, self, first_embeds, idx, targets, False, 2)
+        loss, _ = _GPTEmbedsStep.apply(anchor, self, first_embeds, idx, targets, False, 2, pack)
         return loss
 
     def next_logits_with_first(self, idx, first_embeds):

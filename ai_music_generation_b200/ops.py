@@ -293,6 +293,31 @@ def pos_bwd(dx, dwpe, T):
     _call("pos_bwd", 1, (M, C), _C.lib().abcgpt_pos_bwd, dx.data_ptr(), dwpe.data_ptr(), M, T, C, _stream())
 
 
+def _chk_cu(cu_seqlens, n_seqs):
+    _chk(cu_seqlens, torch.int32, "cu_seqlens")
+    if not cu_seqlens.is_contiguous() or cu_seqlens.numel() < n_seqs + 1:
+        raise _C.AbcgptError(f"cu_seqlens: expected a contiguous int32 tensor of at least n_seqs + 1 = {n_seqs + 1} entries")
+
+
+def add_pos_varlen(e, wpe, x, cu_seqlens, n_seqs):
+    """x[m] = e[m] + wpe[m - cu_seqlens[seq(m)]] (fp32): positions restart at every packed sequence."""
+    _chk(e, torch.float32, "add_pos_varlen e")
+    _chk(x, torch.float32, "add_pos_varlen x")
+    _chk_cu(cu_seqlens, n_seqs)
+    M, C = x.shape
+    _call("add_pos_varlen", 1, (M, C), _C.lib().abcgpt_add_pos_varlen, e.data_ptr(), wpe.data_ptr(), x.data_ptr(),
+          cu_seqlens.data_ptr(), int(n_seqs), M, C, _stream())
+
+
+def pos_bwd_varlen(dx, dwpe, cu_seqlens, n_seqs, max_len):
+    """dwpe[t] += sum over the packed sequences longer than t of dx[cu_seqlens[s] + t] (fixed order, no atomics)."""
+    _chk(dx, torch.float32, "pos_bwd_varlen dx")
+    _chk_cu(cu_seqlens, n_seqs)
+    M, C = dx.shape
+    _call("pos_bwd_varlen", 1, (n_seqs, max_len, C), _C.lib().abcgpt_pos_bwd_varlen, dx.data_ptr(), dwpe.data_ptr(),
+          cu_seqlens.data_ptr(), int(n_seqs), int(max_len), C, _stream())
+
+
 def onehot_bf16(tok, out, V):
     """out[m, s * V + tok[m, s]] = 1 (bf16), everything else 0: the rows TunesFormer's patch embedding Linear sees."""
     _chk(tok, torch.int64, "onehot tok")
@@ -360,6 +385,64 @@ def attn_bwd(qkv, out, dout, lse, delta, dqkv, B, T, H, drop_p=0.0, drop_key=0, 
     else:
         _call("attn_bwd", 3, (B, T, H, head_size), _C.lib().abcgpt_attn_bwd_hd, qkv.data_ptr(), out.data_ptr(), dout.data_ptr(),
               lse.data_ptr(), delta.data_ptr(), dqkv.data_ptr(), B, T, H, int(head_size), drop_p, drop_key, _stream())
+
+
+def attn_varlen_fwd(qkv, out, lse, cu_seqlens, n_seqs, max_len, H, head_size, drop_p=0.0, drop_key=0):
+    """Causal attention over packed sequences (rows [cu_seqlens[s], cu_seqlens[s+1]) of qkv [total_rows, 3C]); lse fp32
+    [H, total_rows].  max_len >= the longest sequence; head sizes 32, 64, 128; drop_p must be 0."""
+    _chk(qkv, torch.bfloat16, "attn_varlen qkv")
+    _chk(out, torch.bfloat16, "attn_varlen out")
+    _chk(lse, torch.float32, "attn_varlen lse")
+    _chk_cu(cu_seqlens, n_seqs)
+    M = qkv.shape[0]
+    _call("attn_varlen_fwd", 1, (n_seqs, max_len, M, H, head_size), _C.lib().abcgpt_attn_varlen_fwd, qkv.data_ptr(),
+          out.data_ptr(), lse.data_ptr(), cu_seqlens.data_ptr(), int(n_seqs), int(max_len), M, H, int(head_size), drop_p,
+          drop_key, _stream())
+
+
+def attn_varlen_bwd(qkv, out, dout, lse, delta, dqkv, cu_seqlens, n_seqs, max_len, H, head_size, drop_p=0.0, drop_key=0):
+    _chk(qkv, torch.bfloat16, "attn_varlen qkv")
+    _chk(dout, torch.bfloat16, "attn_varlen dout")
+    _chk(dqkv, torch.bfloat16, "attn_varlen dqkv")
+    _chk(delta, torch.float32, "attn_varlen delta")
+    _chk_cu(cu_seqlens, n_seqs)
+    M = qkv.shape[0]
+    _call("attn_varlen_bwd", 3, (n_seqs, max_len, M, H, head_size), _C.lib().abcgpt_attn_varlen_bwd, qkv.data_ptr(),
+          out.data_ptr(), dout.data_ptr(), lse.data_ptr(), delta.data_ptr(), dqkv.data_ptr(), cu_seqlens.data_ptr(),
+          int(n_seqs), int(max_len), M, H, int(head_size), drop_p, drop_key, _stream())
+
+
+def ce_group_weights(targets, row_group, n_groups, weights, V):
+    """weights[m] = 1 / (n_groups * valid rows of group row_group[m]) for a valid target, else 0: the loss becomes the mean
+    over groups of each group's token mean."""
+    _chk(targets, torch.int64, "ce targets")
+    _chk(row_group, torch.int32, "ce row_group")
+    _chk(weights, torch.float32, "ce weights")
+    M = targets.numel()
+    if row_group.numel() < M or weights.numel() < M:
+        raise _C.AbcgptError("ce_group_weights: row_group and weights need one entry per target")
+    _call("ce_group_weights", 1, (M, n_groups), _C.lib().abcgpt_ce_group_weights, targets.data_ptr(), row_group.data_ptr(),
+          int(n_groups), M, V, weights.data_ptr(), _stream())
+
+
+def ce_fwd_weighted(logits, targets, weights, row_loss, loss, V):
+    """loss[0] = sum_m weights[m] * (-log softmax(logits[m])[targets[m]])."""
+    _chk(logits, torch.bfloat16, "ce logits")
+    _chk(targets, torch.int64, "ce targets")
+    _chk(weights, torch.float32, "ce weights")
+    M, ldl = logits.shape[0], logits.stride(0)
+    L = _C.lib()
+    _call("ce_fwd", 1, (M, V), L.abcgpt_ce_fwd, logits.data_ptr(), ldl, targets.data_ptr(), row_loss.data_ptr(), M, V,
+          _stream())
+    _call("ce_finalize_weighted", 1, (M,), L.abcgpt_ce_finalize_weighted, row_loss.data_ptr(), weights.data_ptr(), M,
+          loss.data_ptr(), _stream())
+
+
+def ce_bwd_weighted(logits, targets, weights, grad_loss, dlogits, V):
+    _chk(weights, torch.float32, "ce weights")
+    M, ldl = logits.shape[0], logits.stride(0)
+    _call("ce_bwd_weighted", 1, (M, V), _C.lib().abcgpt_ce_bwd_weighted, logits.data_ptr(), ldl, targets.data_ptr(),
+          weights.data_ptr(), grad_loss.data_ptr(), dlogits.data_ptr(), M, V, _stream())
 
 
 def ce_fwd(logits, targets, row_loss, sum_count, loss, V):

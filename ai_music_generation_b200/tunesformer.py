@@ -24,6 +24,7 @@ from .model import GPT, GPTConfig, _DecodeState
 PATCH_SIZE = 32      # tunesformer/config.py:2
 PATCH_LENGTH = 128   # tunesformer/config.py:1
 CHAR_VOCAB = 128     # one-hot width per character (utils.py:102)
+_C_MAX_GROUPS = 12288   # tunes per packed call: abcgpt_ce_group_weights counts each group in shared memory
 
 
 class Patchilizer:
@@ -125,11 +126,11 @@ class _PatchEmbed(torch.autograd.Function):
     """out[m,:] = onehot(patch m) W^T + b as a GEMM on the one-hot rows; backward = weight / bias gradients only."""
 
     @staticmethod
-    def forward(ctx, anchor, dec, patches):
+    def forward(ctx, anchor, dec, patches, packed=False):
         M = patches.shape[0]
         dec._ensure_device_state()
         out = torch.empty(M, dec.config.n_embd, device=patches.device, dtype=torch.float32)
-        oh = dec.embed_patches(patches.contiguous(), out)
+        oh = dec.embed_patches(patches.contiguous(), out, packed)
         ctx.dec, ctx.oh = dec, oh
         return out
 
@@ -145,7 +146,7 @@ class _PatchEmbed(torch.autograd.Function):
         sync = dec._grad_sync
         if sync is not None and dec.require_backward_grad_sync:
             sync.finalize()   # this arena's last gradients: wte/wpe, the patch embedding and the 1-D tail go out now
-        return None, None, None
+        return None, None, None, None
 
 
 class PatchLevelDecoder(GPT):
@@ -159,11 +160,20 @@ class PatchLevelDecoder(GPT):
         self._onehot = {}
         self._flatten()
 
-    def embed_patches(self, patches, out):
+    def embed_patches(self, patches, out, packed=False):
         """out fp32 [M, C] = onehot(patches int64 [M, PATCH_SIZE]) W^T + b (one-hot rows, then the GEMM); returns the one-hot
-        rows.  The bf16 weight shadow must be current (_ensure_device_state)."""
+        rows.  The bf16 weight shadow must be current (_ensure_device_state).  packed: M changes from call to call, the rows
+        live in one buffer that only grows (like the packed activation buffers of GPT._packed_buffers)."""
         M = patches.shape[0]
-        oh = self._onehot.get(M)
+        if packed:
+            oh = self._onehot.get("packed")
+            if oh is None or oh.shape[0] < M:
+                rows = -(-(M + M // 8) // 1024) * 1024
+                self._onehot.pop("packed", None)
+                oh = self._onehot["packed"] = torch.empty(rows, PATCH_SIZE * CHAR_VOCAB, device=patches.device, dtype=torch.bfloat16)
+            oh = oh[:M]
+        else:
+            oh = self._onehot.get(M)
         if oh is None:
             oh = self._onehot[M] = torch.empty(M, PATCH_SIZE * CHAR_VOCAB, device=patches.device, dtype=torch.bfloat16)
         ops.onehot_bf16(patches, oh, CHAR_VOCAB)
@@ -175,8 +185,35 @@ class PatchLevelDecoder(GPT):
         """patches int64 [B, P, PATCH_SIZE] -> fp32 [B, P, C] (last_hidden_state)."""
         B, P, S = patches.shape
         assert S == PATCH_SIZE and P <= self.config.block_size
-        emb = _PatchEmbed.apply(self._anchor_tensor(patches.device), self, patches.reshape(B * P, S))
+        emb = _PatchEmbed.apply(self._anchor_tensor(patches.device), self, patches.reshape(B * P, S), False)
         return self.forward_hidden(emb.view(B, P, -1))
+
+    def encode_packed(self, patches, patch_counts):
+        """patches int64 [sum(patch_counts), PATCH_SIZE], the tunes end to end -> fp32 [sum(patch_counts), C], every tune encoded
+        as if alone."""
+        emb = _PatchEmbed.apply(self._anchor_tensor(patches.device), self, patches, True)
+        return self.forward_hidden_packed(emb, patch_counts)
+
+
+def packed_decode_rows(patch_counts):
+    """Row tables of a packed batch: the character level decodes patch j + 1 of a tune from the encoding of its patch j, so
+    it takes every packed row but each tune's last.  Returns (int64 source rows, int32 tune index of each of them)."""
+    counts = np.asarray(patch_counts, dtype=np.int64)
+    starts = np.concatenate([[0], np.cumsum(counts)[:-1]])
+    src = np.concatenate([np.arange(s0, s0 + c - 1) for s0, c in zip(starts, counts)])
+    tune = np.repeat(np.arange(len(counts), dtype=np.int32), counts - 1)
+    return src.astype(np.int64), tune
+
+
+def pack_tunes(tunes):
+    """Packed layout of TunesFormerShaped.forward(patches, patch_counts): `tunes` is a sequence of int [P_i, PATCH_SIZE] tensors
+    (or nested lists, e.g. Patchilizer.encode output); returns (int64 [sum P_i, PATCH_SIZE] on the device of the first tensor,
+    [P_i])."""
+    parts = [torch.as_tensor(t, dtype=torch.int64).reshape(-1, PATCH_SIZE) for t in tunes]
+    if not parts:
+        raise ValueError("pack_tunes: no tunes")
+    dev = parts[0].device
+    return torch.cat([p.to(dev) for p in parts], dim=0), [int(p.shape[0]) for p in parts]
 
 
 class TunesFormerShaped(nn.Module):
@@ -187,9 +224,18 @@ class TunesFormerShaped(nn.Module):
         self.char_level_decoder = GPT(char_config)
         self.pad_token_id = 0
 
-    def forward(self, patches):
+    def forward(self, patches, patch_counts=None):
         """patches int64 [B, P, PATCH_SIZE] (pad id 0 at the tail of every patch) -> mean next-character loss over the
-        non-pad characters of patches 1..P-1, each decoded from the encoding of the patches before it (utils.py:210-219)."""
+        non-pad characters of patches 1..P-1, each decoded from the encoding of the patches before it (utils.py:210-219).
+
+        patch_counts (a sequence of ints P_i): tunes of different lengths, packed.  patches is then int64
+        [sum P_i, PATCH_SIZE], the tunes' patches end to end with no pad patches (pack_tunes builds it).  The patch level
+        encodes every tune alone, the character level decodes patches 1..P_i-1 of every tune from the encoding of the
+        previous patch of the same tune, and the loss is the mean over tunes of each tune's mean over its non-pad characters:
+        the reference's objective, one tune per DataParallel replica (tunesformer/train.py:77-82).  Every P_i must lie in
+        [2, patch-level block_size]; dropout in either decoder is not supported here.  Raises ValueError before any launch."""
+        if patch_counts is not None:
+            return self._forward_packed(patches, patch_counts)
         B, P, S = patches.shape
         encoded = self.patch_level_decoder.encode(patches)                  # [B, P, C]
         first = encoded[:, :-1, :].reshape(B * (P - 1), -1)
@@ -198,6 +244,44 @@ class TunesFormerShaped(nn.Module):
         y[:, :-1] = chars[:, 1:]
         y[y == self.pad_token_id] = -1                                       # labels -100 at pads (utils.py:128-129)
         return self.char_level_decoder.forward_with_first(chars, first, y)
+
+    def _check_packed(self, patches, patch_counts):
+        counts = [int(c) for c in patch_counts]
+        pbs = self.patch_level_decoder.config.block_size
+        if not counts:
+            raise ValueError("patch_counts is empty")
+        if min(counts) < 2:
+            raise ValueError(f"every tune needs at least 2 patches (one to condition on, one to predict); got {min(counts)}")
+        if max(counts) > pbs:
+            raise ValueError(f"a tune of {max(counts)} patches exceeds the patch-level block_size {pbs}")
+        if patches.dim() != 2 or patches.shape[1] != PATCH_SIZE:
+            raise ValueError(f"packed patches must be int64 [sum(patch_counts), {PATCH_SIZE}], got {tuple(patches.shape)}")
+        if sum(counts) != patches.shape[0]:
+            raise ValueError(f"patch_counts sum to {sum(counts)} but patches has {patches.shape[0]} rows")
+        if len(counts) > _C_MAX_GROUPS:
+            raise ValueError(f"at most {_C_MAX_GROUPS} tunes per packed call")
+        for name, dec in (("patch", self.patch_level_decoder), ("char", self.char_level_decoder)):
+            if dec.config.dropout > 0.0:
+                raise ValueError(f"packed training does not support dropout (the {name}-level decoder has dropout="
+                                 f"{dec.config.dropout})")
+        return counts
+
+    def _forward_packed(self, patches, patch_counts):
+        counts = self._check_packed(patches, patch_counts)
+        S, n = PATCH_SIZE, len(counts)
+        src, tune = packed_decode_rows(counts)
+        dev = patches.device
+        src_d = torch.from_numpy(src).pin_memory().to(dev, non_blocking=True)
+        tune_d = torch.from_numpy(tune).pin_memory().to(dev, non_blocking=True)
+        patches = patches.contiguous()
+        encoded = self.patch_level_decoder.encode_packed(patches, counts)    # [sum P_i, C]
+        first = encoded.index_select(0, src_d)
+        chars = patches.index_select(0, src_d + 1)
+        y = torch.full_like(chars, -1)
+        y[:, :-1] = chars[:, 1:]
+        y[y == self.pad_token_id] = -1
+        row_group = tune_d.view(-1, 1).expand(-1, S).reshape(-1)
+        return self.char_level_decoder.forward_with_first(chars, first, y, row_group=row_group, n_groups=n)
 
     @torch.no_grad()
     def generate(self, patches, tokens=None, top_p=1.0, top_k=0, temperature=1.0, seed=None):
