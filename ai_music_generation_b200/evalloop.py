@@ -33,3 +33,27 @@ def estimate_loss(model, get_batch, eval_iters, device, *, shard=False, group=No
         out[split] = (acc / (n_local * world)).cpu()[0]
     model.train(was_training)
     return out
+
+
+@torch.no_grad()
+def estimate_tunes_loss(model, batches, device, group=None):
+    """Mean loss over every evaluated tune of the hierarchical model: sum_b loss_b * n_b / sum_b n_b, where batch b holds n_b
+    tunes and loss_b is the packed forward's mean over them.  `batches` yields (patches, patch_counts) of this rank, in the
+    layout of `TunesFormerShaped.forward(patches, patch_counts)`; an empty shard is skipped.  Always without patch sampling.
+    The per-rank sums stay on the device, ranks are combined with one all-reduce of the two scalars, and the call
+    synchronises with the host once.  Returns a float (nan when no rank evaluated a tune)."""
+    world = dist.get_world_size(group) if dist.is_initialized() else 1
+    was_training = model.training
+    model.eval()
+    acc = torch.zeros(2, device=device, dtype=torch.float32)
+    for patches, counts in batches:
+        if len(counts) == 0:
+            continue
+        loss = model(patches, counts)
+        acc[0] += loss.detach().float() * len(counts)
+        acc[1] += len(counts)
+    if world > 1:
+        dist.all_reduce(acc, group=group)
+    model.train(was_training)
+    total, n = acc.cpu().tolist()
+    return total / n if n > 0 else float("nan")

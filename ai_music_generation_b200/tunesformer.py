@@ -54,6 +54,11 @@ class Patchilizer:
     def patch2bar(self, patch):
         return "".join(chr(t) for t in patch if t > self.eos_token_id)
 
+    @staticmethod
+    def is_header(line):
+        """An information field ("K:G", "M:6/8", ...) or a %%score line: one patch of its own rather than bars."""
+        return len(line) > 1 and ((line[0].isalpha() and line[1] == ":") or line.startswith("%%score"))
+
     def encode(self, abc_code, patch_length=PATCH_LENGTH, patch_size=PATCH_SIZE, add_special_patches=False):
         try:
             from unidecode import unidecode
@@ -68,8 +73,7 @@ class Patchilizer:
                 patches.append(self.bar2patch(bar + "\n" if (last_newline and i == len(bars) - 1) else bar, patch_size))
 
         for line in (ln for ln in abc_code.split("\n") if ln):
-            header = len(line) > 1 and ((line[0].isalpha() and line[1] == ":") or line.startswith("%%score"))
-            if header:
+            if self.is_header(line):
                 if body:
                     flush(True)
                     body = ""
@@ -205,6 +209,24 @@ def packed_decode_rows(patch_counts):
     return src.astype(np.int64), tune
 
 
+def sampled_decode_rows(patch_counts, k, generator=None):
+    """`packed_decode_rows` with patch sampling (the reference's `patch_sampling_batch_size`): a tune with more than k decoded
+    rows keeps k of them, drawn uniformly without replacement (torch.randperm on the host `generator`) and kept in row order;
+    k = 0 keeps every row.  The tunes are drawn one after another, in batch order.  Returns the same (src, tune) arrays."""
+    src, tune = packed_decode_rows(patch_counts)
+    if k <= 0:
+        return src, tune
+    keep, r0 = [], 0
+    for n in (int(c) - 1 for c in patch_counts):
+        if n > k:
+            keep.append(r0 + torch.randperm(n, generator=generator)[:k].sort().values.numpy())
+        else:
+            keep.append(np.arange(r0, r0 + n))
+        r0 += n
+    keep = np.concatenate(keep)
+    return src[keep], tune[keep]
+
+
 def pack_tunes(tunes):
     """Packed layout of TunesFormerShaped.forward(patches, patch_counts): `tunes` is a sequence of int [P_i, PATCH_SIZE] tensors
     (or nested lists, e.g. Patchilizer.encode output); returns (int64 [sum P_i, PATCH_SIZE] on the device of the first tensor,
@@ -224,7 +246,7 @@ class TunesFormerShaped(nn.Module):
         self.char_level_decoder = GPT(char_config)
         self.pad_token_id = 0
 
-    def forward(self, patches, patch_counts=None):
+    def forward(self, patches, patch_counts=None, patch_sampling=0, generator=None):
         """patches int64 [B, P, PATCH_SIZE] (pad id 0 at the tail of every patch) -> mean next-character loss over the
         non-pad characters of patches 1..P-1, each decoded from the encoding of the patches before it (utils.py:210-219).
 
@@ -233,9 +255,16 @@ class TunesFormerShaped(nn.Module):
         encodes every tune alone, the character level decodes patches 1..P_i-1 of every tune from the encoding of the
         previous patch of the same tune, and the loss is the mean over tunes of each tune's mean over its non-pad characters:
         the reference's objective, one tune per DataParallel replica (tunesformer/train.py:77-82).  Every P_i must lie in
-        [2, patch-level block_size]; dropout in either decoder is not supported here.  Raises ValueError before any launch."""
+        [2, patch-level block_size]; dropout in either decoder is not supported here.  Raises ValueError before any launch.
+
+        patch_sampling k > 0 (packed only; the reference's `patch_sampling_batch_size`): the character level decodes only k of
+        the rows of every tune that has more than k, chosen by `sampled_decode_rows` from the host torch.Generator `generator`
+        (torch's default generator when None); the loss is then each tune's mean over its selected rows' non-pad characters,
+        averaged over tunes.  The selection is per tune because the reference runs one tune per DataParallel replica."""
         if patch_counts is not None:
-            return self._forward_packed(patches, patch_counts)
+            return self._forward_packed(patches, patch_counts, patch_sampling, generator)
+        if patch_sampling:
+            raise ValueError("patch_sampling needs the packed path (patch_counts)")
         B, P, S = patches.shape
         encoded = self.patch_level_decoder.encode(patches)                  # [B, P, C]
         first = encoded[:, :-1, :].reshape(B * (P - 1), -1)
@@ -266,10 +295,12 @@ class TunesFormerShaped(nn.Module):
                                  f"{dec.config.dropout})")
         return counts
 
-    def _forward_packed(self, patches, patch_counts):
+    def _forward_packed(self, patches, patch_counts, patch_sampling=0, generator=None):
         counts = self._check_packed(patches, patch_counts)
         S, n = PATCH_SIZE, len(counts)
-        src, tune = packed_decode_rows(counts)
+        if patch_sampling < 0:
+            raise ValueError(f"patch_sampling must be >= 0, got {patch_sampling}")
+        src, tune = sampled_decode_rows(counts, int(patch_sampling), generator)
         dev = patches.device
         src_d = torch.from_numpy(src).pin_memory().to(dev, non_blocking=True)
         tune_d = torch.from_numpy(tune).pin_memory().to(dev, non_blocking=True)
@@ -358,7 +389,8 @@ class TunesFormerShaped(nn.Module):
 
     # ---- generation on the device ------------------------------------------------------------------------------------
     @torch.no_grad()
-    def generate_tunes(self, prompts, max_patch=PATCH_LENGTH, top_p=0.8, top_k=8, temperature=1.2, seed=None, batch=64):
+    def generate_tunes(self, prompts, max_patch=PATCH_LENGTH, top_p=0.8, top_k=8, temperature=1.2, seed=None, batch=64,
+                       tune_ids=None):
         """`generate_tune` for a list of prompt texts, batched and decoded on the device; returns one tune text per prompt.
 
         Per tune the loop is that of generate_tune: the prompt is encoded with the same Patchilizer, its unfinished last bar
@@ -372,7 +404,11 @@ class TunesFormerShaped(nn.Module):
         Philox uniform of (seed, index of the tune in `prompts`, patch position, character position), so a tune's random
         stream does not depend on the batch it lands in.  An int `seed` makes a call reproducible; seed=None draws one seed
         from torch's CPU generator per call, so `torch.manual_seed` makes it reproducible.  With top_k = 1 every tune equals
-        its greedy generate_tune (up to decisions closer than bf16 rounding)."""
+        its greedy generate_tune (up to decisions closer than bf16 rounding).
+
+        tune_ids (one int per prompt, default 0..len(prompts)-1): the tune index of the Philox key.  A process that holds a
+        slice of a larger prompt list passes the slice's global indices and draws exactly what one process given the whole
+        list draws for those tunes."""
         pz = Patchilizer()
         patches, fixed, remaining = [], [], []
         for prompt in prompts:
@@ -382,7 +418,7 @@ class TunesFormerShaped(nn.Module):
             remaining.append(rest)
             fixed.append([ord(c) for c in rest])
         gen = self.generate_patches(patches, fixed, max_patch=max_patch, top_p=top_p, top_k=top_k, temperature=temperature,
-                                    seed=seed, batch=batch)
+                                    seed=seed, batch=batch, tune_ids=tune_ids)
         tunes = []
         for prompt, bars in zip(prompts, gen):
             tune = prompt
@@ -398,7 +434,7 @@ class TunesFormerShaped(nn.Module):
 
     @torch.no_grad()
     def generate_patches(self, prompt_patches, fixed_tokens=None, max_patch=PATCH_LENGTH, top_p=0.8, top_k=8, temperature=1.2,
-                         seed=None, batch=64):
+                         seed=None, batch=64, tune_ids=None):
         """The bar loop of generate_tune on patches, for many tunes at once.
 
         prompt_patches: one int [P_i, PATCH_SIZE] tensor (or nested list) per tune, starting with the start patch;
@@ -407,7 +443,7 @@ class TunesFormerShaped(nn.Module):
         when one was drawn, like `generate`), the last one possibly the end patch or empty bar that stopped the tune.  The
         patch appended after a bar is bar2patch(fixed + bar) for the first bar and bar2patch(bar) after that.  `batch` tunes
         share one pass of the loop; tunes are grouped by prompt length first, and the result is in input order.  See
-        generate_tunes for the seeding."""
+        generate_tunes for the seeding and `tune_ids`."""
         n = len(prompt_patches)
         pbs, cbs = self.patch_level_decoder.config.block_size, self.char_level_decoder.config.block_size
         if max_patch > pbs:
@@ -418,6 +454,9 @@ class TunesFormerShaped(nn.Module):
             raise ValueError("fixed_tokens needs one list per tune")
         if any(len(p) == 0 for p in prompts):
             raise ValueError("every prompt needs at least its start patch")
+        ids = list(range(n)) if tune_ids is None else [int(i) for i in tune_ids]
+        if len(ids) != n or any(i < 0 for i in ids):
+            raise ValueError("tune_ids needs one non-negative id per tune")
         if any(len(f) + 1 > min(cbs, PATCH_SIZE) for f in fixed):
             raise ValueError(f"at most {min(cbs, PATCH_SIZE) - 1} fixed characters per tune")
         if seed is None:
@@ -431,8 +470,8 @@ class TunesFormerShaped(nn.Module):
         launches0 = ops.LAUNCHES
         for s in range(0, n, max(1, int(batch))):
             idx = order[s:s + max(1, int(batch))]
-            res = self._generate_batch([prompts[i] for i in idx], [fixed[i] for i in idx], idx, max_patch, float(top_p),
-                                       int(top_k), float(temperature), seed, stats)
+            res = self._generate_batch([prompts[i] for i in idx], [fixed[i] for i in idx], [ids[i] for i in idx], max_patch,
+                                       float(top_p), int(top_k), float(temperature), seed, stats)
             for i, r in zip(idx, res):
                 out[i] = r
         stats["launches"] = ops.LAUNCHES - launches0
@@ -600,6 +639,24 @@ class TunesFormerShaped(nn.Module):
         for dec, out in loads:   # nothing is changed unless the whole checkpoint matches
             dec.load_state_dict(out)
         return self
+
+    def reference_state_dict(self):
+        """The inverse of `load_reference_state_dict`: this model's parameters under the reference TunesFormer's HF GPT-2 names,
+        Conv1D weights transposed back to [in, out], as detached CPU tensors.  It loads with strict=True into the reference's
+        arrangement (a `patch_level_decoder` holding `patch_embedding` and `base = GPT2Model`, a `char_level_decoder` holding
+        `base = GPT2LMHeadModel`).  The attention mask buffers are not written (transformers leaves them out of state_dict()
+        too) and the patch level's tied lm_head has no HF counterpart; the character level's tied `lm_head.weight` is kept."""
+        conv = GPT._HF_CONV1D
+        out = {}
+        for name, v in self.patch_level_decoder.state_dict().items():
+            if name == "lm_head.weight":
+                continue
+            key = ("patch_level_decoder." + name if name.startswith("patch_embedding.")
+                   else "patch_level_decoder.base." + name.replace("transformer.", "", 1))
+            out[key] = v
+        for name, v in self.char_level_decoder.state_dict().items():
+            out["char_level_decoder.base." + name] = v
+        return {k: (v.t() if k.endswith(conv) else v).detach().to("cpu", copy=True).contiguous() for k, v in out.items()}
 
     def configure_optimizers(self, weight_decay, learning_rate, betas, device_type="cuda"):
         return _Optimizers([self.patch_level_decoder.configure_optimizers(weight_decay, learning_rate, betas, device_type),
