@@ -158,6 +158,12 @@ int abcgpt_sample_top_p(const void* logits, int64_t ldl, int V, float top_p, int
   return sample_top_p(logits, ldl, V, top_p, top_k, temperature, seed, counter_base, counter, row_id, out, out_stride, B,
                       S(stream));
 }
+int abcgpt_sample_top_p_cluster(const void* logits, int64_t ldl, int V, float top_p, int top_k, float temperature,
+                                const void* seed, const void* counter_base, int64_t counter, const int64_t* row_id, int64_t* out,
+                                int64_t out_stride, int B, void* stream) {
+  return sample_top_p_cluster(logits, ldl, V, top_p, top_k, temperature, seed, counter_base, counter, row_id, out, out_stride, B,
+                              S(stream));
+}
 
 /*
  * Replay of a recorded launch list with position-affine arguments (the decode loop of GPT.generate is launch-bound: ~90
@@ -218,6 +224,11 @@ int abcgpt_replay(const int64_t* prog, int64_t n_words, int64_t k) {
         if (nargs != 14) return fail(-1, "abcgpt_replay: sample_top_p takes 14 arguments");
         rc = abcgpt_sample_top_p(P_(0), a[1], I_(2), abcgpt_word_f(a[3]), I_(4), abcgpt_word_f(a[5]), P_(6), P_(7), a[8],
                                  CP_(int64_t, 9), MP_(int64_t, 10), a[11], I_(12), P_(13));
+        break;
+      case ABCGPT_FN_SAMPLE_TOP_P_CLUSTER:
+        if (nargs != 14) return fail(-1, "abcgpt_replay: sample_top_p_cluster takes 14 arguments");
+        rc = abcgpt_sample_top_p_cluster(P_(0), a[1], I_(2), abcgpt_word_f(a[3]), I_(4), abcgpt_word_f(a[5]), P_(6), P_(7), a[8],
+                                         CP_(int64_t, 9), MP_(int64_t, 10), a[11], I_(12), P_(13));
         break;
       default:
         return fail(-1, "abcgpt_replay: unknown function id %lld", (long long)fn);

@@ -216,6 +216,11 @@ __device__ __forceinline__ uint32_t ld_shared_cluster_u32(uint32_t cluster_addr)
   asm volatile("ld.shared::cluster.u32 %0, [%1];" : "=r"(v) : "r"(cluster_addr) : "memory");
   return v;
 }
+__device__ __forceinline__ unsigned long long ld_shared_cluster_u64(uint32_t cluster_addr) {
+  unsigned long long v;
+  asm volatile("ld.shared::cluster.u64 %0, [%1];" : "=l"(v) : "r"(cluster_addr) : "memory");
+  return v;
+}
 __device__ __forceinline__ void red_min_shared_cluster_s32(uint32_t cluster_addr, int v) {
   asm volatile("red.shared::cluster.min.s32 [%0], %1;" ::"r"(cluster_addr), "r"(v) : "memory");
 }

@@ -582,7 +582,404 @@ sample_top_p_kernel(const __nv_bfloat16* __restrict__ logits, long long ldl, int
   if (tid == 0) out[static_cast<long long>(row) * out_stride] = pick != INT_MAX ? pick : last;
 }
 
+// ---- nucleus / top-k / temperature for large vocabularies: one cluster per row ----------------------------------------
+// The contract of sample_top_p_kernel for 8 <= V <= 786 432, with the slice layout of sample_topk_cluster_kernel (8 CTAs,
+// each holding a contiguous slice of the row as bf16 bits).  Tokens are ranked by the 16-bit order key of their logit:
+// p = exp(l - max) / Z is strictly increasing in l, so (key descending, index ascending) is (p descending, index ascending)
+// for the exact softmax.  Masses are 64-bit fixed point, e = expf(l - max) in units of 2^-43 (the row maximum weighs exactly
+// 2^43; V * 2^43 < 2^63): integer sums are exact and order-free, so every combination over threads and CTAs gives the same
+// bits whatever the order of arrival.
+//   load     slice into shared memory; slice max and first index; 256-bin token count on the key's high byte | barrier 1
+//   top-k    (0 < top_k < V) high byte of the rank-top_k key from the summed counts
+//   mass     Z and a 256-bin mass histogram on the high byte; top-k: counts on the low byte under its high byte | barrier 2
+//            nucleus: the high byte where the mass from the top reaches ceil(top_p * Z); top-k: its exact key
+//   low      nucleus: mass and count histograms on the low byte under that high byte                        | barrier 3
+//            nucleus cut key k and the number of its ties, in index order, the cut needs
+//   cut      the first n = min(nucleus size, top_k) ranks: every key above the cut key, and the first j tokens (by index) of
+//            the cut key's tie class
+//   draw     per-thread contiguous chunks: weight above the cut and tie count, CTA scans, CTA totals            | barrier 4
+//            exclusive prefix of the 8 CTA totals (tie tokens are kept while their index-order rank is below j); the one
+//            thread whose integer interval holds floor(u * W) walks its chunk and writes the token
+//   exit     barrier 5: no CTA leaves while a peer may still read its shared memory
+// Against sample_top_p_kernel (which sums fp32 p in rank order):
+//   * the nucleus cut: expf is within 2 ulp and the fixed point within 2^-44 per token, so the mass fraction of any prefix is
+//     within 1e-6 of the exact softmax's.  The two kernels can pick different cuts only where the running sum lies within
+//     that, plus the one-CTA kernel's own fp32 rounding, of top_p.
+//   * ties: the one-CTA kernel ranks by its fp32 p, which can round two distinct logits to one value and then orders them by
+//     index; here they are ordered by logit.  fp32 p separates logits that differ by more than about 2^-22 (every pair of
+//     distinct bf16 logits with |l| >= 2^-14) while p is a normal float (l > max - 87); the order can differ only inside such
+//     a merged pair, and only matters when a cut falls between its two tokens.
+//   * the draw: weights exp((l - max) / temperature) (= (p / p_max)^(1 / temperature)), zero where fp32 exp(l - max) is
+//     zero, as a zero p is in the one-CTA kernel; the same uniform u picks the smallest kept token whose running weight
+//     exceeds floor(u * W), so the tokens differ only where u lies within rounding of a CDF boundary.
+constexpr int kTopPClusterMinV = kClusterCtas;
+constexpr float kFixedOne = 8796093022208.f;  // 2^43
+
+__device__ __forceinline__ unsigned long long to_fixed(float w) { return __float2ull_rn(w * kFixedOne); }
+
+// bits of a logit as ranked here: -0 as +0, so that equal values have equal keys
+__device__ __forceinline__ uint32_t logit_bits(__nv_bfloat16 l) {
+  const uint32_t b = __bfloat16_as_ushort(l);
+  return b == 0x8000u ? 0u : b;
+}
+
+__device__ __forceinline__ uint32_t key16_bits(uint32_t key) { return (key & 0x8000u) ? (key & 0x7fffu) : (~key & 0xffffu); }
+
+__device__ __forceinline__ unsigned long long mass_fixed(uint32_t b, float mx) { return to_fixed(expf(bits_to_float(b) - mx)); }
+
+__device__ __forceinline__ unsigned long long weight_fixed(uint32_t b, float mx, float inv_t) {
+  const float d = bits_to_float(b) - mx;
+  return expf(d) > 0.f ? to_fixed(expf(d * inv_t)) : 0ull;
+}
+
+// Masses are accumulated with native 32-bit shared atomics as three 15-bit pieces (m = p0 + p1 << 15 + p2 << 30, m <= 2^43):
+// a piece summed over a slice of at most 98 304 tokens stays below 2^32.  (A 64-bit shared atomicAdd is a compare-and-swap
+// loop, and combining lanes with __reduce_add_sync under a per-lane mask compiles to a loop over the distinct masks; both
+// serialise under the contention of the few populated key bins.)
+__device__ __forceinline__ void add_mass(uint32_t* hist, uint32_t bin, unsigned long long m) {
+  const uint32_t p0 = static_cast<uint32_t>(m & 0x7fffu), p1 = static_cast<uint32_t>((m >> 15) & 0x7fffu),
+                 p2 = static_cast<uint32_t>(m >> 30);
+  if (p0) atomicAdd(&hist[bin], p0);
+  if (p1) atomicAdd(&hist[256 + bin], p1);
+  if (p2) atomicAdd(&hist[512 + bin], p2);
+}
+
+// Cluster-wide sums of the CTAs' 256-bin histograms `hist` (kPieces = 1: counts; 3: masses in 15-bit pieces), read through
+// distributed shared memory, one bin per thread: above[b] = the sum over the bins above b.  Returns the total in every thread.
+template <int kPieces>
+__device__ __forceinline__ unsigned long long cluster_bins_above(const uint32_t* hist, unsigned long long* above,
+                                                                 unsigned long long* scan_w) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const uint32_t bin = 255 - tid;  // descending bins: a prefix over threads is a suffix over bins
+  unsigned long long c = 0;
+#pragma unroll
+  for (int k = 0; k < kPieces; ++k) {
+    const uint32_t addr = ptx::smem_u32(hist + 256 * k + bin);
+    unsigned long long ck = 0;
+#pragma unroll
+    for (int r = 0; r < kClusterCtas; ++r) ck += ptx::ld_shared_cluster_u32(ptx::mapa(addr, r));
+    c += ck << (15 * k);
+  }
+  unsigned long long incl = c;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const unsigned long long v = __shfl_up_sync(0xffffffffu, incl, o);
+    if (lane >= o) incl += v;
+  }
+  __syncthreads();  // scan_w reuse
+  if (lane == 31) scan_w[warp] = incl;
+  __syncthreads();
+  unsigned long long off = 0, total = 0;
+#pragma unroll
+  for (int w = 0; w < kClusterWarps; ++w) {
+    if (w < warp) off += scan_w[w];
+    total += scan_w[w];
+  }
+  above[bin] = off + incl - c;
+  __syncthreads();
+  return total;
+}
+
+// The bin b with above[b] < target <= above[b] + (sum of bin b), for 1 <= target <= total; in every thread.
+__device__ __forceinline__ uint32_t select_bin(const unsigned long long* above, unsigned long long total,
+                                               unsigned long long target, int* sel) {
+  const uint32_t b = threadIdx.x;
+  if (above[b] < target && target <= (b > 0 ? above[b - 1] : total)) *sel = static_cast<int>(b);
+  __syncthreads();
+  const uint32_t r = static_cast<uint32_t>(*sel);
+  __syncthreads();  // sel reuse
+  return r;
+}
+
+// exclusive prefix over the block (threads in order) of one u64 and one int per thread; totals in *tw / *tc
+__device__ __forceinline__ void block_excl_scan2(unsigned long long w, int c, unsigned long long* scan_w, int* scan_c,
+                                                 unsigned long long* ew, int* ec, unsigned long long* tw, int* tc) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  unsigned long long iw = w;
+  int ic = c;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const unsigned long long vw = __shfl_up_sync(0xffffffffu, iw, o);
+    const int vc = __shfl_up_sync(0xffffffffu, ic, o);
+    if (lane >= o) { iw += vw; ic += vc; }
+  }
+  __syncthreads();
+  if (lane == 31) { scan_w[warp] = iw; scan_c[warp] = ic; }
+  __syncthreads();
+  unsigned long long ow = 0, sw = 0;
+  int oc = 0, sc = 0;
+#pragma unroll
+  for (int k = 0; k < kClusterWarps; ++k) {
+    if (k < warp) { ow += scan_w[k]; oc += scan_c[k]; }
+    sw += scan_w[k];
+    sc += scan_c[k];
+  }
+  *ew = ow + iw - w;
+  *ec = oc + ic - c;
+  *tw = sw;
+  *tc = sc;
+}
+
+__global__ void __launch_bounds__(kClusterThreads)
+sample_top_p_cluster_kernel(const __nv_bfloat16* __restrict__ logits, long long ldl, int V, int slice, float top_p, int top_k,
+                            float temperature, const unsigned long long* __restrict__ seed,
+                            const long long* __restrict__ counter_base, long long counter, const int64_t* __restrict__ row_id,
+                            int64_t* __restrict__ out, long long out_stride) {
+  static_assert(kClusterThreads == 256, "one histogram bin per thread");
+  extern __shared__ __align__(16) uint16_t xb[];  // [slice] logit bits
+  // read by the peers (each between two consecutive cluster barriers)
+  __shared__ uint32_t cnt_hi[256], cnt_lo_k[256], cnt_lo_p[256];
+  __shared__ uint32_t mass_hi[3 * 256], mass_lo[3 * 256];  // 15-bit pieces (add_mass)
+  __shared__ float slice_max;
+  __shared__ int slice_arg, slice_ties;
+  __shared__ unsigned long long slice_w;
+  // this CTA only
+  __shared__ unsigned long long above_cnt[256], above_a[256], above_b[256];
+  __shared__ unsigned long long scan_w[kClusterWarps];
+  __shared__ float red_f[kClusterWarps], cta_f[kClusterCtas];
+  __shared__ int red_i[kClusterWarps], scan_c[kClusterWarps], cta_i[kClusterCtas], sel;
+  __shared__ unsigned long long cta_w[kClusterCtas];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int rank = static_cast<int>(ptx::cluster_ctarank());
+  const int row = blockIdx.x / kClusterCtas;
+  const int base = rank * slice;
+  const int n = max(0, min(slice, V - base));
+  const __nv_bfloat16* lr = logits + static_cast<long long>(row) * ldl + base;
+  // every CTA of the cluster takes the same branches: the barriers below are reached by all of them
+  const bool greedy = temperature <= 0.f || top_k == 1;
+  const bool nucleus = !greedy && top_p < 1.f;
+  const bool crop = !greedy && top_k > 0 && top_k < V;
+
+  cnt_hi[tid] = 0u;
+  cnt_lo_k[tid] = 0u;
+  cnt_lo_p[tid] = 0u;
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    mass_hi[256 * k + tid] = 0u;
+    mass_lo[256 * k + tid] = 0u;
+  }
+  __syncthreads();
+
+  // ---- load: logit bits into shared memory, slice max and its first index, high-byte token counts
+  float mx = -INFINITY;
+  int mi = INT_MAX;  // every thread visits its indices in increasing order, so a strict > keeps the first maximum
+  const bool count = nucleus || crop;
+  const int n8 = (reinterpret_cast<uintptr_t>(lr) & 15u) == 0 ? n / 8 : 0;
+  for (int v = tid; v < n8; v += kClusterThreads) {
+    const uint4 raw = __ldg(reinterpret_cast<const uint4*>(lr) + v);
+    const __nv_bfloat16* l8 = reinterpret_cast<const __nv_bfloat16*>(&raw);
+    uint32_t w[4];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      const uint32_t b = logit_bits(l8[j]);
+      const float x = bits_to_float(b);
+      if (x > mx) { mx = x; mi = v * 8 + j; }
+      if (count) atomicAdd(&cnt_hi[order_key16(b) >> 8], 1u);
+      if (j & 1) w[j >> 1] |= b << 16; else w[j >> 1] = b;
+    }
+    reinterpret_cast<uint4*>(xb)[v] = make_uint4(w[0], w[1], w[2], w[3]);
+  }
+  for (int i = n8 * 8 + tid; i < n; i += kClusterThreads) {
+    const uint32_t b = logit_bits(lr[i]);
+    const float x = bits_to_float(b);
+    xb[i] = static_cast<uint16_t>(b);
+    if (x > mx) { mx = x; mi = i; }
+    if (count) atomicAdd(&cnt_hi[order_key16(b) >> 8], 1u);
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const float om = __shfl_xor_sync(0xffffffffu, mx, o);
+    const int oi = __shfl_xor_sync(0xffffffffu, mi, o);
+    if (om > mx || (om == mx && oi < mi)) { mx = om; mi = oi; }
+  }
+  if (lane == 0) { red_f[warp] = mx; red_i[warp] = mi; }
+  __syncthreads();
+  if (tid == 0) {
+#pragma unroll
+    for (int w = 1; w < kClusterWarps; ++w)
+      if (red_f[w] > mx || (red_f[w] == mx && red_i[w] < mi)) { mx = red_f[w]; mi = red_i[w]; }
+    slice_max = mx;
+    slice_arg = mi == INT_MAX ? INT_MAX : base + mi;
+  }
+  ptx::cluster_sync_all();  // 1
+
+  // ---- row max and its first index (the rank-0 token): the slices in rank order hold increasing indices
+  if (tid < kClusterCtas) {
+    cta_f[tid] = __uint_as_float(ptx::ld_shared_cluster_u32(ptx::mapa(ptx::smem_u32(&slice_max), tid)));
+    cta_i[tid] = static_cast<int>(ptx::ld_shared_cluster_u32(ptx::mapa(ptx::smem_u32(&slice_arg), tid)));
+  }
+  __syncthreads();
+  mx = cta_f[0];
+  mi = cta_i[0];
+#pragma unroll
+  for (int r = 1; r < kClusterCtas; ++r)
+    if (cta_f[r] > mx) { mx = cta_f[r]; mi = cta_i[r]; }
+
+  int n_keep = V;        // kept ranks
+  uint32_t cut = 0u;     // kept: key > cut, and the first `ties` tokens (by index) with key == cut
+  int ties = INT_MAX;
+  if (count) {
+    cluster_bins_above<1>(cnt_hi, above_cnt, scan_w);
+    // ---- top-k: high byte of the rank-top_k key
+    uint32_t hc = 0u;
+    if (crop) hc = select_bin(above_cnt, V, top_k, &sel);
+    // ---- mass histogram on the high byte; top-k: counts on the low byte under hc
+    const float mxv = mx;
+    for (int v = tid; v * 8 < n; v += kClusterThreads) {
+      const uint4 q = reinterpret_cast<const uint4*>(xb)[v];
+      const uint32_t w[4] = {q.x, q.y, q.z, q.w};
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {
+        if (v * 8 + j >= n) break;
+        const uint32_t b = (w[j >> 1] >> (16 * (j & 1))) & 0xffffu, key = order_key16(b);
+        if (nucleus) add_mass(mass_hi, key >> 8, mass_fixed(b, mxv));
+        if (crop && (key >> 8) == hc) atomicAdd(&cnt_lo_k[key & 0xffu], 1u);
+      }
+    }
+    ptx::cluster_sync_all();  // 2
+    if (crop) {
+      const unsigned long long in_hc = cluster_bins_above<1>(cnt_lo_k, above_b, scan_w);
+      const unsigned long long k_in = top_k - above_cnt[hc];  // rank of the cut inside bin hc, from 1
+      const uint32_t lc = select_bin(above_b, in_hc, k_in, &sel);
+      cut = (hc << 8) | lc;
+      ties = static_cast<int>(k_in - above_b[lc]);
+      n_keep = top_k;
+    }
+    uint32_t hb = 0u;
+    unsigned long long need = 0;
+    if (nucleus) {
+      const unsigned long long z = cluster_bins_above<3>(mass_hi, above_a, scan_w);
+      const unsigned long long target = max(1ull, static_cast<unsigned long long>(ceil(static_cast<double>(top_p) * static_cast<double>(z))));
+      hb = select_bin(above_a, z, target, &sel);
+      need = target - above_a[hb];
+      // ---- mass and counts on the low byte under hb
+      for (int v = tid; v * 8 < n; v += kClusterThreads) {
+        const uint4 q = reinterpret_cast<const uint4*>(xb)[v];
+        const uint32_t w[4] = {q.x, q.y, q.z, q.w};
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          if (v * 8 + j >= n) break;
+          const uint32_t b = (w[j >> 1] >> (16 * (j & 1))) & 0xffffu, key = order_key16(b);
+          if ((key >> 8) == hb) {
+            atomicAdd(&cnt_lo_p[key & 0xffu], 1u);
+            add_mass(mass_lo, key & 0xffu, mass_fixed(b, mxv));
+          }
+        }
+      }
+    }
+    ptx::cluster_sync_all();  // 3
+    if (nucleus) {
+      const unsigned long long in_hb = cluster_bins_above<3>(mass_lo, above_a, scan_w);
+      const uint32_t lb = select_bin(above_a, in_hb, need, &sel);
+      const unsigned long long rest = need - above_a[lb];
+      const uint32_t key = (hb << 8) | lb;
+      const unsigned long long m = mass_fixed(key16_bits(key), mx);  // every token of the tie class weighs m > 0
+      const int j = static_cast<int>((rest + m - 1) / m);
+      cluster_bins_above<1>(cnt_lo_p, above_b, scan_w);
+      const int n_nuc = static_cast<int>(above_cnt[hb] + above_b[lb]) + j;
+      if (!crop || n_nuc <= top_k) {
+        cut = key;
+        ties = j;
+        n_keep = n_nuc;
+      }
+    }
+  }
+
+  if (greedy || n_keep == 1) {
+    ptx::cluster_sync_all();  // exit
+    if (rank == 0 && tid == 0) out[static_cast<long long>(row) * out_stride] = mi;
+    return;
+  }
+
+  // ---- draw: weights above the cut and tie counts over a contiguous chunk per thread
+  const float inv_t = 1.f / temperature;
+  const int chunk = (n + kClusterThreads - 1) / kClusterThreads;
+  const int i0 = min(n, tid * chunk), i1 = min(n, i0 + chunk);
+  unsigned long long local_w = 0;
+  int local_t = 0;
+  for (int i = i0; i < i1; ++i) {
+    const uint32_t b = xb[i], key = order_key16(b);
+    if (key > cut) local_w += weight_fixed(b, mx, inv_t);
+    else if (key == cut) ++local_t;
+  }
+  unsigned long long excl_w, cta_total_w;
+  int excl_t, cta_total_t;
+  block_excl_scan2(local_w, local_t, scan_w, scan_c, &excl_w, &excl_t, &cta_total_w, &cta_total_t);
+  if (tid == 0) { slice_w = cta_total_w; slice_ties = cta_total_t; }
+  ptx::cluster_sync_all();  // 4
+  if (tid < kClusterCtas) {
+    cta_w[tid] = ptx::ld_shared_cluster_u64(ptx::mapa(ptx::smem_u32(&slice_w), tid));
+    cta_i[tid] = static_cast<int>(ptx::ld_shared_cluster_u32(ptx::mapa(ptx::smem_u32(&slice_ties), tid)));
+  }
+  __syncthreads();
+  const unsigned long long w_tie = weight_fixed(key16_bits(cut), mx, inv_t);
+  unsigned long long w_before = 0, w_total = 0;
+  int t_before = 0, t_seen = 0;
+#pragma unroll
+  for (int r = 0; r < kClusterCtas; ++r) {
+    const int kept = min(cta_i[r], max(0, ties - t_seen));
+    const unsigned long long wr = cta_w[r] + w_tie * static_cast<unsigned long long>(kept);
+    if (r < rank) { w_before += wr; t_before += cta_i[r]; }
+    w_total += wr;
+    t_seen += cta_i[r];
+  }
+  const int ties_left = max(0, ties - t_before - excl_t);  // tie tokens this thread and the ones after it may still keep
+  const unsigned long long lo = w_before + excl_w + w_tie * static_cast<unsigned long long>(min(excl_t, max(0, ties - t_before)));
+  const unsigned long long hi = lo + local_w + w_tie * static_cast<unsigned long long>(min(local_t, ties_left));
+
+  const long long rid = row_id != nullptr ? row_id[row] : row;
+  const uint32_t bits = philox_uniform_bits(*seed, static_cast<uint32_t>(rid), static_cast<uint64_t>(*counter_base + counter));
+  const unsigned long long target = __umul64hi(w_total, static_cast<unsigned long long>(bits >> 8) << 40);  // floor(u * W)
+  if (lo <= target && target < hi) {  // exactly one thread of the cluster
+    unsigned long long acc = lo;
+    int left = ties_left, pick = i1 - 1;
+    for (int i = i0; i < i1; ++i) {
+      const uint32_t b = xb[i], key = order_key16(b);
+      unsigned long long w = 0;
+      if (key > cut) w = weight_fixed(b, mx, inv_t);
+      else if (key == cut && left > 0) { w = w_tie; --left; }
+      acc += w;
+      if (acc > target) { pick = i; break; }
+    }
+    out[static_cast<long long>(row) * out_stride] = base + pick;
+  }
+  ptx::cluster_sync_all();  // 5
+}
+
 }  // namespace
+
+int sample_top_p_cluster(const void* logits, long long ldl, int V, float top_p, int top_k, float temperature, const void* seed,
+                         const void* counter_base, long long counter, const int64_t* row_id, int64_t* out, long long out_stride,
+                         int B, cudaStream_t stream) {
+  ABCGPT_CHECK_ARG(logits && out && seed && counter_base && B > 0, "sample_top_p_cluster: bad arguments");
+  ABCGPT_CHECK_ARG(V >= kTopPClusterMinV && V <= kClusterMaxV,
+                   "sample_top_p_cluster: vocabulary of %d tokens is outside [%d, %d]", V, kTopPClusterMinV, kClusterMaxV);
+  ABCGPT_CHECK_ARG(ldl >= V, "sample_top_p_cluster: row stride %lld is below V = %d", ldl, V);
+  ABCGPT_CHECK_ARG(B <= INT_MAX / kClusterCtas, "sample_top_p_cluster: %d rows do not fit one grid", B);
+  const int slice = ((V + kClusterCtas - 1) / kClusterCtas + 7) / 8 * 8;  // a multiple of 8: 16-byte aligned slices
+  static bool configured = false;
+  if (!configured) {
+    ABCGPT_CUDA(cudaFuncSetAttribute(sample_top_p_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                     kClusterSliceMax * static_cast<int>(sizeof(uint16_t))));
+    configured = true;
+  }
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(static_cast<unsigned>(B) * kClusterCtas);
+  cfg.blockDim = dim3(kClusterThreads);
+  cfg.dynamicSmemBytes = static_cast<size_t>(slice) * sizeof(uint16_t);
+  cfg.stream = stream;
+  cudaLaunchAttribute at[1];
+  at[0].id = cudaLaunchAttributeClusterDimension;
+  at[0].val.clusterDim.x = kClusterCtas;
+  at[0].val.clusterDim.y = 1;
+  at[0].val.clusterDim.z = 1;
+  cfg.attrs = at;
+  cfg.numAttrs = 1;
+  ABCGPT_CUDA(cudaLaunchKernelEx(&cfg, sample_top_p_cluster_kernel, reinterpret_cast<const __nv_bfloat16*>(logits), ldl, V,
+                                 slice, top_p, top_k, temperature, reinterpret_cast<const unsigned long long*>(seed),
+                                 reinterpret_cast<const long long*>(counter_base), counter, row_id, out, out_stride));
+  return launch_status("sample_top_p_cluster_kernel");
+}
 
 int sample_top_p(const void* logits, long long ldl, int V, float top_p, int top_k, float temperature, const void* seed,
                  const void* counter_base, long long counter, const int64_t* row_id, int64_t* out, long long out_stride, int B,

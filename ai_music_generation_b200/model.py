@@ -89,6 +89,8 @@ def _round_up(x, m):
 
 
 HEAD_SIZES = (32, 64, 128)   # head sizes the sm_100a attention kernels are built for (csrc/attn.cu: 64, csrc/attn_hd.cu: 32, 128)
+_TOP_P_CTA_MAX_V = 1024      # nucleus head: one CTA per row up to here (abcgpt_sample_top_p), one cluster above
+_TOP_P_MAX_V = 786432        # ... up to here (abcgpt_sample_top_p_cluster)
 
 
 def head_size_of(cfg: GPTConfig) -> int:
@@ -924,7 +926,7 @@ class GPT(nn.Module):
         flops_per_iter = flops_per_token * T * fwdbwd_per_iter
         return flops_per_iter * (1.0 / dt) / flops_promised
 
-    def _generate_ragged(self, idx, prompt_lens, max_new_tokens, temperature, top_k, stop_token, stop_check_every):
+    def _generate_ragged(self, idx, prompt_lens, max_new_tokens, head, stop_token, stop_check_every, seed, row_ids):
         if not idx.is_cuda:
             raise _C.AbcgptError("GPT.generate: idx must be a CUDA tensor (there is no CPU path)")
         B, Tmax = idx.shape
@@ -952,8 +954,7 @@ class GPT(nn.Module):
             forced = torch.zeros(total, B, device=idx.device, dtype=torch.int64)
             forced[:lmax] = idx[:, :lmax].t()
             st.col[:lmin].copy_(forced[:lmin])
-            head = self._head(temperature, top_k)
-            self._reseed_sampler()
+            self._arm_sampler(head, seed, row_ids, B, idx.device, st)
             last = total - 1
             ops.set_pdl(True)
             for t in range(last):
@@ -1054,8 +1055,9 @@ class GPT(nn.Module):
                 ops.argmax(st.logits, cfg.vocab_size, st.col[t + 1], out_stride=1)
             elif head is not None and head[0] == "top_p":
                 seed, counter_base, row_id = st.sampler
-                ops.sample_top_p(st.logits, cfg.vocab_size, st.col[t + 1], head[1], head[2], head[3], seed, counter_base, t,
-                                 row_id=row_id)
+                top_p_kernel = ops.sample_top_p if cfg.vocab_size <= _TOP_P_CTA_MAX_V else ops.sample_top_p_cluster
+                top_p_kernel(st.logits, cfg.vocab_size, st.col[t + 1], head[1], head[2], head[3], seed, counter_base, t,
+                             row_id=row_id)
             elif head is not None:
                 ops.sample_topk(st.logits, cfg.vocab_size, st.col[t + 1], head[1], head[2], self._seed_buffer(), t)
         if self._plan_cache_enabled:
@@ -1080,23 +1082,65 @@ class GPT(nn.Module):
         tunes reproducible, and consecutive calls see different random streams."""
         self._seed_buffer().fill_(int(torch.randint(0, 2 ** 62, (1,)).item()))
 
-    def _head(self, temperature, top_k):
+    def _head(self, temperature, top_k, top_p=None):
         V = self.config.vocab_size
+        if top_p is not None:
+            # TunesFormer's chain: nucleus, then top-k, then temperature (abcgpt_sample_top_p / _cluster)
+            if not 0.0 < top_p <= 1.0:
+                raise ValueError(f"top_p must lie in (0, 1] (got {top_p})")
+            if V > _TOP_P_MAX_V:
+                raise ValueError(f"nucleus sampling supports vocabularies of up to {_TOP_P_MAX_V} tokens (got {V})")
+            k = 0 if top_k is None or int(top_k) >= V else max(0, int(top_k))
+            return ("top_p", float(top_p), k, float(temperature))
         if top_k is not None and min(top_k, V) == 1:
             return ("greedy",)   # top_k = 1: the softmax over one surviving token is 1, the draw is its argmax
         k = 0 if top_k is None else min(int(top_k), V)
         return ("sample", float(temperature), 0 if k >= V else k)
 
-    def _sample(self, logits_bf16, out_col, out_stride, head, counter):
+    def _arm_sampler(self, head, seed, row_ids, B, device, st=None):
+        """Sets the random stream of one generate() call.  seed: an int, or None for one draw from torch's CPU generator.
+        The ("top_p", ...) head reads (seed, counter base, row ids) device buffers: the decode state's own (recorded launch
+        lists hold their addresses), or a per-batch-size set when there is no state; the counter base is 1, so that with
+        counter = position of the last input token every draw is keyed by the absolute position of the token it draws.
+        Returns those buffers (None for the other heads)."""
+        if seed is None:
+            self._reseed_sampler()
+        else:
+            self._seed_buffer().fill_(int(seed) & ((1 << 63) - 1))
+        if head[0] != "top_p":
+            if row_ids is not None:
+                raise ValueError("row_ids name the random streams of the top_p head; pass top_p as well")
+            return None
+        ids = list(range(B)) if row_ids is None else [int(i) for i in row_ids]
+        if len(ids) != B or min(ids) < 0:
+            raise ValueError(f"row_ids needs one non-negative int per row ({B} rows)")
+        smp = st.sampler if st is not None else None
+        if smp is None:
+            smp = self._bufs.get(("sampler", B))
+            if smp is None:
+                z = lambda n: torch.zeros(n, device=device, dtype=torch.int64)  # noqa: E731
+                smp = self._bufs[("sampler", B)] = (z(1), z(1), z(B))
+            if st is not None:
+                st.sampler = smp
+        smp[0].copy_(self._seed_buffer())
+        smp[1].fill_(1)
+        smp[2].copy_(torch.tensor(ids, dtype=torch.int64))
+        return smp
+
+    def _sample(self, logits_bf16, out_col, out_stride, head, counter, sampler=None):
         V = self.config.vocab_size
         if head[0] == "greedy":
             ops.argmax(logits_bf16, V, out_col, out_stride=out_stride)
+        elif head[0] == "top_p":
+            top_p_kernel = ops.sample_top_p if V <= _TOP_P_CTA_MAX_V else ops.sample_top_p_cluster
+            top_p_kernel(logits_bf16, V, out_col, head[1], head[2], head[3], sampler[0], sampler[1], counter,
+                         row_id=sampler[2], out_stride=out_stride)
         else:
             ops.sample_topk(logits_bf16, V, out_col, head[1], head[2], self._seed_buffer(), counter, out_stride=out_stride)
 
     @torch.no_grad()
     def generate(self, idx, max_new_tokens, temperature=1.0, top_k=None, use_cache=True, stop_token=None, stop_check_every=64,
-                 prompt_lens=None):
+                 prompt_lens=None, top_p=None, seed=None, row_ids=None):
         """Reference semantics (model.py:305-330): feed the sequence back max_new_tokens times, last-position logits,
         temperature, optional top-k, sample, append; the context is cropped to block_size.
 
@@ -1117,9 +1161,19 @@ class GPT(nn.Module):
         prompt instead of the sampler (its prefix is fed through the same single-position steps an equal-length batch
         uses, so each row's tokens are those of generating it alone).  Row i of the result holds its prompt followed by
         max_new_tokens generated tokens; anything after that is filled with stop_token (0 if None).  Needs
-        max(prompt_lens) + max_new_tokens <= block_size + 1 (the window may not slide)."""
+        max(prompt_lens) + max_new_tokens <= block_size + 1 (the window may not slide).
+
+        top_p (extension, default None = the head above): 0 < top_p <= 1 samples with TunesFormer's chain instead — nucleus
+        (the most probable tokens up to and including the one whose running probability reaches top_p), then the first
+        top_k of those (None: no cut), then weights p^(1 / temperature) (temperature <= 0: the argmax); one CTA per row for
+        V <= 1024 (abcgpt_sample_top_p), one cluster of 8 CTAs above (abcgpt_sample_top_p_cluster, V <= 786 432).  Every
+        draw is keyed by (seed, row id, absolute position of the drawn token), on the cached, ragged and slid-window paths
+        alike, so a row draws the same tokens wherever it sits in a batch.  row_ids: one non-negative int per row naming its
+        stream (default 0 .. B-1).
+        seed (extension): an int makes the call reproducible under either head; None takes one draw from torch's generator."""
+        head = self._head(temperature, top_k, top_p)
         if prompt_lens is not None:
-            return self._generate_ragged(idx, prompt_lens, max_new_tokens, temperature, top_k, stop_token, stop_check_every)
+            return self._generate_ragged(idx, prompt_lens, max_new_tokens, head, stop_token, stop_check_every, seed, row_ids)
         if not idx.is_cuda:
             raise _C.AbcgptError("GPT.generate: idx must be a CUDA tensor (there is no CPU path)")
         B, T0 = idx.shape
@@ -1131,14 +1185,15 @@ class GPT(nn.Module):
         self.eval()
         try:
             self._ensure_device_state()
-            head = self._head(temperature, top_k)
-            self._reseed_sampler()
             t = 0
+            st = None
             if use_cache and T0 <= bs:
                 key = ("decode", B, bs)
                 if key not in self._bufs:
                     self._bufs[key] = _DecodeState(self.config, B, bs, idx.device)
                 st = self._bufs[key]
+            sampler = self._arm_sampler(head, seed, row_ids, B, idx.device, st)
+            if st is not None:
                 last = min(total - 1, bs)   # positions 0 .. last-1 can be decoded with the cache
                 st.col[:T0].copy_(idx.t())
                 stopped = False
@@ -1161,7 +1216,7 @@ class GPT(nn.Module):
                 lo = max(0, pos + 1 - bs)
                 cond = out[:, lo:pos + 1].contiguous()
                 bufs = self._forward_plan(cond, None, keep_activations=False)
-                self._sample(bufs.last_logits, out[:, pos + 1:], out.stride(0), head, pos)
+                self._sample(bufs.last_logits, out[:, pos + 1:], out.stride(0), head, pos, sampler)
         finally:
             ops.set_pdl(False)
             self.train(was_training)

@@ -505,6 +505,16 @@ def sample_top_p(logits, V, out, top_p, top_k, temperature, seed, counter_base, 
           _stream())
 
 
+def sample_top_p_cluster(logits, V, out, top_p, top_k, temperature, seed, counter_base, counter, row_id=None, out_stride=1):
+    """sample_top_p for 8 <= V <= 786 432: one cluster of 8 CTAs per row (include/abcgpt.h: abcgpt_sample_top_p_cluster).
+    Same arguments; a V outside that range raises before any launch."""
+    _chk(logits, torch.bfloat16, "sample logits")
+    B, ldl = logits.shape[0], logits.stride(0)
+    _call("sample_top_p_cluster", 1, (B, V), _C.lib().abcgpt_sample_top_p_cluster, logits.data_ptr(), ldl, V, float(top_p),
+          int(top_k), float(temperature), seed.data_ptr(), counter_base.data_ptr(), int(counter), _ptr(row_id), out.data_ptr(),
+          out_stride, B, _stream())
+
+
 def nvls_allreduce_sumsq(grad_mc_ptr, n, rank, world, partials_mc_ptr, blocks_per_rank, threads=512):
     """include/abcgpt.h abcgpt_nvls_allreduce_sumsq: mean of the replicas' gradient arenas + norm partials, over multicast memory."""
     _call("nvls_allreduce_sumsq", 1, (n, world), _C.lib().abcgpt_nvls_allreduce_sumsq, int(grad_mc_ptr), int(n), int(rank), int(world),

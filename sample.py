@@ -7,6 +7,10 @@ construction from a validation set (first `n_conditional_measures` bars; sample.
 (cut at '$', trim to the last bar line; sample.py:158-169).  Difference: prompts are decoded in batches through GPT.generate,
 also when their lengths differ (prompt_lens; the reference decodes them one at a time through the same batch-generic API,
 model.py:305-330).
+
+top_p > 0 draws with TunesFormer's recipe instead of the reference's head (e.g. --top_p=0.8 --top_k=8 --temperature=1.2).
+The run's random stream is `seed`, and each prompt draws from its own stream named by its index in the prompt list, so the
+files do not depend on `batch` or on how the prompts are grouped.
 """
 from __future__ import annotations
 
@@ -27,6 +31,7 @@ DEFAULTS = dict(
     temperature=0.8, top_k=200, seed=1337, device="cuda", dtype="bfloat16", compile=False,
     batch=64,          # new knob: prompts of equal length are decoded together (the reference decodes one at a time)
     early_stop=True,   # new knob: stop a batch once every tune has produced its end symbol '$' (files are cut there anyway)
+    top_p=0.0,         # new knob: 0 < top_p <= 1 samples with TunesFormer's nucleus / top-k / temperature chain; 0 = off
 )
 
 
@@ -101,8 +106,10 @@ def main():
     abc = s["tokens_format"] == "char" and s["dataset"] == "irishman"
     out_dir = os.path.join(s["out_dir"], "samples")
     os.makedirs(out_dir, exist_ok=True)
-    todo = [(key, text, encode(text)) for key, text in prompts_from(s)]
+    todo = [(key, text, encode(text), i) for i, (key, text) in enumerate(prompts_from(s))]
     top_k = s["top_k"] if s["top_k"] > 0 else None
+    # the nucleus head: one seed per run, each prompt's stream named by its place in prompts_from (before the sort below)
+    nucleus = dict(top_p=s["top_p"], seed=s["seed"]) if s["top_p"] > 0 else {}
     block = model.config.block_size
     # prompts sorted by length and cut into batches; a batch of different lengths is decoded together (prompt_lens: rows
     # still inside their prompt are fed its tokens) as long as the longest prompt + max_new_tokens fits the context window,
@@ -111,7 +118,7 @@ def main():
     chunks = []
     for i in range(0, len(todo), s["batch"]):
         chunk = todo[i:i + s["batch"]]
-        lens = [len(ids) for _, _, ids in chunk]
+        lens = [len(ids) for _, _, ids, _ in chunk]
         if len(set(lens)) == 1 or max(lens) + s["max_new_tokens"] <= block + 1:
             chunks.append(chunk)
         else:
@@ -121,18 +128,23 @@ def main():
             chunks.extend(group for _, group in sorted(by_len.items()))
     with torch.no_grad():
         for chunk in chunks:
-            lens = [len(ids) for _, _, ids in chunk]
+            lens = [len(ids) for _, _, ids, _ in chunk]
             if len(set(lens)) == 1:
-                x = torch.tensor([ids for _, _, ids in chunk], dtype=torch.long, device=s["device"])
-                y = model.generate(x, s["max_new_tokens"], temperature=s["temperature"], top_k=top_k, stop_token=stop).tolist()
+                x = torch.tensor([ids for _, _, ids, _ in chunk], dtype=torch.long, device=s["device"])
+                if nucleus:
+                    nucleus["row_ids"] = [i for _, _, _, i in chunk]
+                y = model.generate(x, s["max_new_tokens"], temperature=s["temperature"], top_k=top_k, stop_token=stop,
+                                   **nucleus).tolist()
             else:
                 x = torch.zeros(len(chunk), max(lens), dtype=torch.long)
-                for r, (_, _, ids) in enumerate(chunk):
+                for r, (_, _, ids, _) in enumerate(chunk):
                     x[r, :len(ids)] = torch.tensor(ids, dtype=torch.long)
+                if nucleus:
+                    nucleus["row_ids"] = [i for _, _, _, i in chunk]
                 y = model.generate(x.to(s["device"]), s["max_new_tokens"], temperature=s["temperature"], top_k=top_k,
-                                   stop_token=stop, prompt_lens=lens).tolist()
+                                   stop_token=stop, prompt_lens=lens, **nucleus).tolist()
                 y = [row[:n + s["max_new_tokens"]] for row, n in zip(y, lens)]
-            for (key, text, _), ids in zip(chunk, y):
+            for (key, text, _, _), ids in zip(chunk, y):
                 res = decode(ids)
                 print(f"\nPrefix: {text}\nGeneration: {res}\n" + "-" * 50)
                 name = f"sample_{key}.abc" if abc else f"sample_{key}.txt"
