@@ -66,7 +66,6 @@ _SIGNATURES = {
     "abcgpt_event_wait": (c_int, [c_int, _P]),
     "abcgpt_nvls_allreduce_sumsq": (c_int, [_P, c_int64, c_int, c_int, c_float, _P, c_int, c_int, _P]),
     "abcgpt_sumsq_partials": (c_int, [_P, c_int, _P, _P]),
-    "abcgpt_set_dynamic_tiles": (c_int, [c_int]),
     "abcgpt_argmax": (c_int, [_P, c_int64, c_int, _P, c_int64, c_int, _P]),
     "abcgpt_sample_topk": (c_int, [_P, c_int64, c_int, c_float, c_int, _P, c_int64, _P, c_int64, c_int, _P]),
     "abcgpt_sample_top_p": (c_int, [_P, c_int64, c_int, c_float, c_int, c_float, _P, _P, c_int64, _P, _P, c_int64, c_int, _P]),
@@ -76,8 +75,6 @@ _SIGNATURES = {
 # include/abcgpt_debug.h: only in libabcgpt_debug.so (tools/)
 _DEBUG_SIGNATURES = {
     "abcgpt_debug_gemm_stats": (c_int, [_P]),
-    "abcgpt_debug_attn_trace": (c_int, [_P]),
-    "abcgpt_debug_attn_cta_trace": (c_int, [_P]),
     "abcgpt_debug_mma_bench": (c_int, [_P, c_int, c_int, c_int, _P]),
     "abcgpt_debug_tmem_ld_bench": (c_int, [_P, c_int, c_int, c_int, _P]),
     "abcgpt_debug_pair_probe": (c_int, [_P, _P, _P, c_int, _P]),

@@ -292,13 +292,4 @@ int abcgpt_sumsq_partials(const float* partials, int nparts, float* out, void* s
   return sumsq_partials(partials, nparts, out, S(stream));
 }
 
-/* Ticket-based tile scheduler of the CTA-pair GEMM for the launches that follow (0 = static round-robin, the default): resident
- * pairs absorb the tiles of pairs that share their SM with another stream's kernel — with the gradient exchange running in a few
- * small CTAs beside the backward a static schedule waits for the slowest SM (+13..48 % per GEMM, tools/coresidency_probe.py), the
- * dynamic one loses 3-7 %. */
-int abcgpt_set_dynamic_tiles(int on) {
-  abcgpt::set_dynamic_tiles(on != 0);
-  return 0;
-}
-
 }  // extern "C"

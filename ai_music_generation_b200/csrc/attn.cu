@@ -12,18 +12,15 @@
 //                         dK += dS^T Q (TMEM acc).  Two kernels instead of atomics on dQ: deterministic gradients.
 // The forward runs two CTAs per SM so that one CTA's softmax (MUFU-bound) overlaps the other's MMAs.
 #include "attn_helpers.cuh"
-#include <stdlib.h>
 
 namespace abcgpt {
 
-long long* g_attn_trace = nullptr;  // debug only (abcgpt_debug_attn_trace): per-phase clock64 stamps of one CTA
-long long* g_attn_cta_trace = nullptr;
-// csrc/attn_pair.cu: the same backward on CTA pairs (cta_group::2 MMAs) for unpacked sequences of >= 256 positions
+// csrc/attn_pair.cu: the same backward on CTA pairs (cta_group::2 MMAs) for unpacked sequences of >= 512 positions
 int attn_bwd_pair(const void* qkv, const void* dout, const float* lse, const float* delta, void* dqkv, int B, int T, int H,
                   const DropCfg& dcfg, cudaStream_t stream);
 // csrc/attn_fwd3.cu: the forward with three CTAs per SM (single-buffered S / O in 128 tensor-memory columns)
 int attn_fwd3(const CUtensorMap& tmQ, const CUtensorMap& tmKV, void* out, float* lse, int T, int H, int C, int BH, int nitems,
-              const DropCfg& dcfg, int seq_shift, uint32_t fBH_d, uint32_t fBH_m, uint32_t fH_d, uint32_t fH_m, cudaStream_t stream);  // debug only (abcgpt_debug_attn_cta_trace): {start ns, end ns, SM id, steps} per CTA
+              const DropCfg& dcfg, int seq_shift, uint32_t fBH_d, uint32_t fBH_m, uint32_t fH_d, uint32_t fH_m, cudaStream_t stream);
 
 namespace {
 
@@ -53,8 +50,7 @@ template <bool DROP>
 __global__ void __launch_bounds__(kThreads, 2)
 attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmKV,
                 __nv_bfloat16* __restrict__ out, float* __restrict__ lse, int T, int H, int C, int BH, int nitems,
-                long long* trace, const DropCfg dcfg, long long* cta_trace, int seq_shift, const FastDiv fBH, const FastDiv fH) {
-  const long long cta_t0 = cta_trace ? globaltimer_ns() : 0;
+                const DropCfg dcfg, int seq_shift, const FastDiv fBH, const FastDiv fH) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + FwdSmem::BAR);
@@ -71,10 +67,6 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
 
   const int warp = ptx::uniform(threadIdx.x >> 5), lane = threadIdx.x & 31;
   const int nqt = (T + 127) / 128;
-  const bool tr = trace != nullptr && blockIdx.x == 0 && threadIdx.x == 64;
-  int total_steps = 0;
-// debug stamps (abcgpt_debug_attn_trace): the first 120 steps of CTA 0's row-0 thread; slot 5 = item ordinal, 6 = tile, 7 = globaltimer
-#define ATTN_STAMP(k) do { if (tr && gt < 120) { trace[gt * 8 + (k)] = clock64(); if ((k) == 0) { trace[gt * 8 + 5] = item_k; trace[gt * 8 + 6] = j; trace[gt * 8 + 7] = globaltimer_ns(); } } } while (0)
 
   if (warp == 0 && lane == 0) {
     ptx::prefetch_tmap(&tmQ);
@@ -246,7 +238,6 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
       if (it < 0) break;
       const int qt = nqt - 1 - fdiv(it, fBH), bh = fmodi(it, fBH);
       const int num_kv = tiles_of(it);
-      total_steps += num_kv;
       const uint32_t tm_O = tmem_base + 128 + (item_k & 1) * 64;
       const int r0 = qt * 128 + quarter * 32;  // first query row of this warp (relative to the sequence)
       float m_ref = 0.f, l = 0.f;
@@ -260,10 +251,8 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
         const int c0 = j * 64, c1 = j * 64 + 32;
         const int cls0 = !same_seq(c0, r0, seq_shift) ? kMasked : ((c0 + 31 <= r0) ? kFull : ((c0 > r0 + 31) ? kMasked : kDiag));
         const int cls1 = !same_seq(c1, r0, seq_shift) ? kMasked : ((c1 + 31 <= r0) ? kFull : ((c1 > r0 + 31) ? kMasked : kDiag));
-        ATTN_STAMP(0);
         ptx::mbar_wait(&s_full[bsel], (gt >> 1) & 1, 17);
         ptx::tc_fence_after();
-        ATTN_STAMP(1);
         uint32_t pk[32];
         float tmax = -1e30f, rowsum = 0.f;
         if (!have_ref && (cls0 != kMasked || cls1 != kMasked)) {
@@ -300,8 +289,6 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
           }
         }
         l += rowsum;
-        ATTN_STAMP(2);
-        ATTN_STAMP(3);
         // P (64 key columns = 32 packed words) overwrites the first half of this tile's S buffer; the tensor pipe runs in
         // issue order, so S_{j+2} cannot overwrite it before P V of this tile has consumed it
         ptx::tmem_st16(tm_s, pk);
@@ -309,7 +296,6 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
         ptx::tmem_st_wait();
         ptx::tc_fence_before();
         ptx::mbar_arrive(&p_full[bsel]);
-        ATTN_STAMP(4);
         if (pend) {
           epilogue(pend_k, pend_it, pend_l, pend_m);
           pend = false;
@@ -323,12 +309,10 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
       pend_m = m_ref;
     }
     if (pend) epilogue(pend_k, pend_it, pend_l, pend_m);
-#undef ATTN_STAMP
   }
   ptx::tc_fence_before();
   __syncthreads();
   if (warp == 1) ptx::tmem_dealloc(tmem_base, 256);
-  if (threadIdx.x == 64) cta_trace_write(cta_trace, cta_t0, total_steps);
 }
 
 // ======================================================================================================
@@ -387,10 +371,7 @@ __global__ void __launch_bounds__(kBwdThreads, 1)
 attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap tmQKV128, const __grid_constant__ CUtensorMap tmQKV64,
                    const __grid_constant__ CUtensorMap tmDO128, const float* __restrict__ lse,
                    const float* __restrict__ delta, __nv_bfloat16* __restrict__ dqkv, int T, int H, int C, int BH,
-                   int nitems, long long* trace, const DropCfg dcfg, long long* cta_trace, int seq_shift, const FastDiv fBH, const FastDiv fH) {
-  const long long cta_t0 = cta_trace ? globaltimer_ns() : 0;
-  const bool tr = trace != nullptr && blockIdx.x == 0 && threadIdx.x == 64;
-#define DQ_STAMP(k) do { if (tr && use < 64) trace[use * 8 + (k)] = clock64(); } while (0)
+                   int nitems, const DropCfg dcfg, int seq_shift, const FastDiv fBH, const FastDiv fH) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + DqSmem::BAR);
@@ -408,7 +389,6 @@ attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap tmQKV128, const __grid_co
 
   const int warp = ptx::uniform(threadIdx.x >> 5), lane = threadIdx.x & 31;
   const int nqt = (T + 127) / 128;
-  int total_steps = 0;
 
   if (warp == 0 && lane == 0) {
     ptx::prefetch_tmap(&tmQKV128);
@@ -593,13 +573,12 @@ attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap tmQKV128, const __grid_co
       }
     };
     normalize();
-    int ep_k = 0, stat_k = -1, nxt_k = c_k, use = 0;
+    int ep_k = 0, stat_k = -1, nxt_k = c_k;
     int r0 = 0;
     uint32_t drop_rk = 0;
     float neg_l = 0.f, neg_d = 0.f, nxt_l, nxt_d;
     load_stats(c_k, nxt_l, nxt_d);
     while (c_it >= 0) {
-      DQ_STAMP(0);
       if (stat_k != c_k) {  // first own step in a new item: decode it once, take its row statistics, prefetch the next item's
         if (nxt_k != c_k) load_stats(c_k, nxt_l, nxt_d);  // (prefetch guessed another item: never at the shapes in use)
         neg_l = -nxt_l * kLog2e;
@@ -618,10 +597,8 @@ attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap tmQKV128, const __grid_co
         nxt_k = nk;
       }
       const int gs = c_base + c_n;
-      DQ_STAMP(1);
       ptx::mbar_wait(&s_full[gs % kSBuf], (gs / kSBuf) & 1, 28);
       ptx::tc_fence_after();
-      DQ_STAMP(2);
       const uint32_t tbuf = tmem_base + lane_off + (gs % kSBuf) * 128;
 #pragma unroll
       for (int c = 0; c < 2; ++c) {
@@ -635,28 +612,21 @@ attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap tmQKV128, const __grid_co
         // dS chunk c (32 key columns = 16 packed words) overwrites score columns that this thread has already consumed
         ptx::tmem_st16(tbuf + c * 16, pk);
       }
-      DQ_STAMP(3);
       ptx::tmem_st_wait();
       ptx::tc_fence_before();
       ptx::mbar_arrive(&ds_full[gs % kSBuf]);
-      DQ_STAMP(4);
-      if (tr && use < 64) { trace[use * 8 + 5] = c_k; trace[use * 8 + 6] = c_n; }
-      ++use;
-      ++total_steps;
       // earlier items are drained AFTER this group's first step in a later item: by then their last MMAs (which wait for
       // the other group's final step) have completed, so the drain does not stall the step pipeline
       while (ep_k < c_k) epilogue(ep_k++);
       c_n += 2;
       normalize();
     }
-#undef DQ_STAMP
     // items not yet drained (c_k is now one past the last item of this CTA)
     while (ep_k < c_k) epilogue(ep_k++);
   }
   ptx::tc_fence_before();
   __syncthreads();
   if (warp == 1) ptx::tmem_dealloc(tmem_base, 512);
-  if (threadIdx.x == 64) cta_trace_write(cta_trace, cta_t0, 2 * total_steps);
 }
 
 struct DkvSmem {
@@ -673,10 +643,7 @@ __global__ void __launch_bounds__(kBwdThreads, 1)
 attn_bwd_dkv_kernel(const __grid_constant__ CUtensorMap tmQKV128, const __grid_constant__ CUtensorMap tmQKV64,
                     const __grid_constant__ CUtensorMap tmDO64, const float* __restrict__ lse,
                     const float* __restrict__ delta, __nv_bfloat16* __restrict__ dqkv, int T, int H, int C, int BH,
-                    int nitems, long long* trace, const DropCfg dcfg, long long* cta_trace, int seq_shift, const FastDiv fBH, const FastDiv fH) {
-  const long long cta_t0 = cta_trace ? globaltimer_ns() : 0;
-  const bool tr = trace != nullptr && blockIdx.x == 0 && threadIdx.x == 64;
-#define DKV_STAMP(k) do { if (tr && use < 64) trace[512 + use * 8 + (k)] = clock64(); } while (0)
+                    int nitems, const DropCfg dcfg, int seq_shift, const FastDiv fBH, const FastDiv fH) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + DkvSmem::BAR);
@@ -694,7 +661,6 @@ attn_bwd_dkv_kernel(const __grid_constant__ CUtensorMap tmQKV128, const __grid_c
 
   const int warp = ptx::uniform(threadIdx.x >> 5), lane = threadIdx.x & 31;
   const int nq64 = (T + 63) / 64;
-  int total_steps = 0;
 
   if (warp == 0 && lane == 0) {
     ptx::prefetch_tmap(&tmQKV128);
@@ -906,7 +872,6 @@ attn_bwd_dkv_kernel(const __grid_constant__ CUtensorMap tmQKV128, const __grid_c
     int ep_k = 0, use = 0, dec_k = -1;
     int kt = 0, bh = 0;
     while (c_it >= 0) {
-      DKV_STAMP(0);
       if (dec_k != c_k) {  // decode the item once
         kt = fdiv(c_it, fBH);
         bh = fmodi(c_it, fBH);
@@ -922,11 +887,9 @@ attn_bwd_dkv_kernel(const __grid_constant__ CUtensorMap tmQKV128, const __grid_c
         st_lse[128 + tid] = __uint_as_float(
             drop_row_key(dcfg.key, static_cast<uint32_t>(stat_idx(fdiv(bh, fH), fmodi(bh, fH), q0 + tid, H, T, seq_shift))));
       raw_cur = load_stat(a_it, a_n);  // next own step: consumed at the top of the next iteration
-      DKV_STAMP(1);
       ptx::bar_sync(1 + g, 128);
       ptx::mbar_wait(&s_full[gs % kSBuf], (gs / kSBuf) & 1, 38);
       ptx::tc_fence_after();
-      DKV_STAMP(2);
       const uint32_t tbuf = tmem_base + lane_off + (gs % kSBuf) * 128;
 #pragma unroll
       for (int c = 0; c < 2; ++c) {
@@ -942,14 +905,10 @@ attn_bwd_dkv_kernel(const __grid_constant__ CUtensorMap tmQKV128, const __grid_c
         ptx::tmem_st16(tbuf + c * 16, pk_p);
         ptx::tmem_st16(tbuf + 64 + c * 16, pk_ds);
       }
-      DKV_STAMP(3);
       ptx::tmem_st_wait();
       ptx::tc_fence_before();
       ptx::mbar_arrive(&pds_full[gs % kSBuf]);
-      DKV_STAMP(4);
-      if (tr && use < 64) { trace[512 + use * 8 + 5] = c_k; trace[512 + use * 8 + 6] = c_n; }
       ++use;
-      ++total_steps;
       // earlier items are drained AFTER this group's first step in a later item (their last MMAs wait for the other
       // group's final step; by now they have completed): the drain does not stall the step pipeline
       while (ep_k < c_k) epilogue(ep_k++);
@@ -957,13 +916,11 @@ attn_bwd_dkv_kernel(const __grid_constant__ CUtensorMap tmQKV128, const __grid_c
       a_n += 2;
       normalize(a_k, a_it, a_n, a_base, a_nq);
     }
-#undef DKV_STAMP
     while (ep_k < c_k) epilogue(ep_k++);  // c_k is now one past the last item of this CTA
   }
   ptx::tc_fence_before();
   __syncthreads();
   if (warp == 1) ptx::tmem_dealloc(tmem_base, 512);
-  if (threadIdx.x == 64) cta_trace_write(cta_trace, cta_t0, 2 * total_steps);
 }
 
 template <typename K>
@@ -1014,23 +971,18 @@ int attn_fwd(const void* qkv, void* out, float* lse, int B, int T, int H, float 
   const int BH = B * H, nitems = ((T + 127) / 128) * BH;
   const FastDiv fBH = make_fastdiv(static_cast<uint32_t>(BH), static_cast<uint64_t>(nitems)), fH = make_fastdiv(static_cast<uint32_t>(H), BH);
   const int grid = nitems < 2 * sm_count() ? nitems : 2 * sm_count();  // persistent: two CTAs per SM
-  long long* CT = g_attn_cta_trace;
   __nv_bfloat16* o = reinterpret_cast<__nv_bfloat16*>(out);
   // Three CTAs per SM with single-buffered S / O (csrc/attn_fwd3.cu) for sequences of >= 256 positions: 0.110 vs 0.120 ms per
   // layer at cfg3, 0.0196 vs 0.0205 ms at cfg2; packed short sequences (T = 32: 0.279 vs 0.273 ms at the cfg4 character level)
-  // and the tracing tools keep the two-CTA kernel.  ABCGPT_ATTN_FWD3=0 selects the two-CTA kernel everywhere (A/B runs).
-  static const bool three_ctas = [] {
-    const char* e = getenv("ABCGPT_ATTN_FWD3");
-    return e == nullptr || e[0] != '0';
-  }();
-  if (three_ctas && seq_shift == kNoPack && T >= 256 && g_attn_trace == nullptr && CT == nullptr)
+  // keep the two-CTA kernel.
+  if (seq_shift == kNoPack && T >= 256)
     return attn_fwd3(tmQ, tmKV, out, lse, T, H, C, BH, nitems, dcfg, seq_shift, fBH.d, fBH.m, fH.d, fH.m, stream);
   if (dcfg.thr16 == 0)
-    launch_k(attn_fwd_kernel<false>, dim3(grid), dim3(kThreads), FwdSmem::TOTAL, stream, tmQ, tmKV, o, lse, T, H, C, BH, nitems, g_attn_trace,
-             dcfg, CT, seq_shift, fBH, fH);
+    launch_k(attn_fwd_kernel<false>, dim3(grid), dim3(kThreads), FwdSmem::TOTAL, stream, tmQ, tmKV, o, lse, T, H, C, BH, nitems, dcfg,
+             seq_shift, fBH, fH);
   else
-    launch_k(attn_fwd_kernel<true>, dim3(grid), dim3(kThreads), FwdSmem::TOTAL, stream, tmQ, tmKV, o, lse, T, H, C, BH, nitems, g_attn_trace,
-             dcfg, CT, seq_shift, fBH, fH);
+    launch_k(attn_fwd_kernel<true>, dim3(grid), dim3(kThreads), FwdSmem::TOTAL, stream, tmQ, tmKV, o, lse, T, H, C, BH, nitems, dcfg,
+             seq_shift, fBH, fH);
   return launch_status("attn_fwd_kernel");
 }
 
@@ -1064,32 +1016,25 @@ int attn_bwd(const void* qkv, const void* out, const void* dout, const float* ls
     if ((rc = launch_status("attn_delta_kernel"))) return rc;
   }
   // CTA-pair kernels (csrc/attn_pair.cu) for sequences of >= 512 positions (at T = 256 a pair item has only 4 steps and the
-  // single-CTA kernels are 10 % faster: 0.057 vs 0.063 ms at cfg2); ABCGPT_ATTN_PAIR=0 keeps the single-CTA kernels everywhere
-  // (A/B measurements).  The tracing tools (abcgpt_debug_attn_*) instrument the single-CTA kernels only.
-  static const bool use_pair = [] {
-    const char* e = getenv("ABCGPT_ATTN_PAIR");
-    return e == nullptr || e[0] != '0';
-  }();
-  if (use_pair && seq_shift == kNoPack && T >= 512 && g_attn_trace == nullptr && g_attn_cta_trace == nullptr)
+  // single-CTA kernels are 10 % faster: 0.057 vs 0.063 ms at cfg2).
+  if (seq_shift == kNoPack && T >= 512)
     return attn_bwd_pair(qkv, dout, lse, delta, dqkv, B, T, H, dcfg, stream);
   const int BH = B * H, nitems = ((T + 127) / 128) * BH;
   const FastDiv fBH = make_fastdiv(static_cast<uint32_t>(BH), static_cast<uint64_t>(nitems)), fH = make_fastdiv(static_cast<uint32_t>(H), BH);
   const int grid = nitems < sm_count() ? nitems : sm_count();  // persistent: one CTA per SM
   __nv_bfloat16* dq = reinterpret_cast<__nv_bfloat16*>(dqkv);
-  long long* CT1 = g_attn_cta_trace ? g_attn_cta_trace + 4 * 1024 : nullptr;
-  long long* CT2 = g_attn_cta_trace ? g_attn_cta_trace + 8 * 1024 : nullptr;
   if (dcfg.thr16 == 0) {
     launch_k(attn_bwd_dkv_kernel<false>, dim3(grid), dim3(kBwdThreads), DkvSmem::TOTAL, stream, tmQKV128, tmQKV64, tmDO64, lse, delta, dq, T, H, C,
-                                                                              BH, nitems, g_attn_trace, dcfg, CT1, seq_shift, fBH, fH);
+                                                                              BH, nitems, dcfg, seq_shift, fBH, fH);
     if ((rc = launch_status("attn_bwd_dkv_kernel"))) return rc;
     launch_k(attn_bwd_dq_kernel<false>, dim3(grid), dim3(kBwdThreads), DqSmem::TOTAL, stream, tmQKV128, tmQKV64, tmDO128, lse, delta, dq, T, H, C,
-                                                                            BH, nitems, g_attn_trace, dcfg, CT2, seq_shift, fBH, fH);
+                                                                            BH, nitems, dcfg, seq_shift, fBH, fH);
   } else {
     launch_k(attn_bwd_dkv_kernel<true>, dim3(grid), dim3(kBwdThreads), DkvSmem::TOTAL, stream, tmQKV128, tmQKV64, tmDO64, lse, delta, dq, T, H, C,
-                                                                             BH, nitems, g_attn_trace, dcfg, CT1, seq_shift, fBH, fH);
+                                                                             BH, nitems, dcfg, seq_shift, fBH, fH);
     if ((rc = launch_status("attn_bwd_dkv_kernel"))) return rc;
     launch_k(attn_bwd_dq_kernel<true>, dim3(grid), dim3(kBwdThreads), DqSmem::TOTAL, stream, tmQKV128, tmQKV64, tmDO128, lse, delta, dq, T, H, C,
-                                                                           BH, nitems, g_attn_trace, dcfg, CT2, seq_shift, fBH, fH);
+                                                                           BH, nitems, dcfg, seq_shift, fBH, fH);
   }
   return launch_status("attn_bwd_dq_kernel");
 }

@@ -3,7 +3,7 @@
 // Why.  A forward step (128 query rows x 64 keys) of the two-CTA kernel is ~1640 cycles of one CTA, of which ~1170 are the softmax
 // (64 MUFU instructions per warp at the ~18 cycles each that two warps sharing a scheduler's MUFU get) and ~470-650 are latencies
 // in which that CTA issues no MUFU work at all: the hand-over of P, the wait for the next S, tensor-memory round trips, loop
-// bookkeeping (tools/attn_trace.py).  Measured this round: the time does not move when the per-thread work is halved (eight
+// bookkeeping (per-phase clock stamps of one CTA).  Measured this round: the time does not move when the per-thread work is halved (eight
 // compute warps), nor when MUFU work is traded for FMA work (1/8, 1/4, 1/2 of the exponentials as polynomials), and the clean
 // MUFU benchmark (tools/mufu2_bench.py) shows ONE warp per scheduler can saturate the unit (15.6 of 16 results per clock): the
 // SM simply has too few independent instruction streams — with two CTAs both are regularly inside their gaps at once and the

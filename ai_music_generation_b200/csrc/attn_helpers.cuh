@@ -21,20 +21,6 @@ __host__ __device__ constexpr float scale_of(int D) { return D == 32 ? 0.1767766
 __host__ __device__ constexpr float sl2_of(int D) { return D == HS ? kSl2 : scale_of(D) * kLog2e; }
 constexpr int kThreads = 192;  // warp 0 TMA, warp 1 MMA, warps 2..5 one thread per tile row
 
-__device__ __forceinline__ long long globaltimer_ns() {
-  long long t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  return t;
-}
-__device__ __forceinline__ void cta_trace_write(long long* cta_trace, long long t0, int steps) {
-  if (cta_trace != nullptr) {
-    uint32_t smid;
-    asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-    long long* o = cta_trace + 4ll * blockIdx.x;
-    o[0] = t0; o[1] = globaltimer_ns(); o[2] = smid; o[3] = steps;
-  }
-}
-
 __device__ __forceinline__ float ex2(float x) {
   float y;
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));

@@ -1,5 +1,4 @@
 #include "common.h"
-#include <stdlib.h>
 
 #include <unordered_map>
 
@@ -12,19 +11,12 @@ char* last_error_buf() {
   return buf;
 }
 
-// ABCGPT_PDL=0 / 1 forces the attribute off / on for every launch; otherwise the caller decides (abcgpt_set_pdl): on for
-// the chain of small kernels of a decoded token (+11 % tokens/s), off for the training step, where every kernel fills the
-// GPU for 25-400 us and the early-resident CTAs cost more than the hidden launch latency (measured -1.8 %).
-static int g_pdl_request = 0;
-void set_pdl(bool on) { g_pdl_request = on ? 1 : 0; }
-bool pdl_enabled() {
-  static int forced = -2;
-  if (forced == -2) {
-    const char* e = getenv("ABCGPT_PDL");
-    forced = (e == nullptr || e[0] == '\0') ? -1 : (e[0] == '0' ? 0 : 1);
-  }
-  return forced >= 0 ? forced == 1 : g_pdl_request == 1;
-}
+// The caller decides (abcgpt_set_pdl): on for the chain of small kernels of a decoded token (+11 % tokens/s), off for the
+// training step, where every kernel fills the GPU for 25-400 us and the early-resident CTAs cost more than the hidden launch
+// latency (measured -1.8 %).
+static bool g_pdl = false;
+void set_pdl(bool on) { g_pdl = on; }
+bool pdl_enabled() { return g_pdl; }
 
 int sm_count() {
   static int cached[64] = {0};

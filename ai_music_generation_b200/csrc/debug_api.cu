@@ -6,8 +6,6 @@
 
 namespace abcgpt {
 extern unsigned long long* g_gemm_stats;
-extern long long* g_attn_trace;
-extern long long* g_attn_cta_trace;
 int tmem_ld_bench(long long*, int, int, int, cudaStream_t);
 int mma_bench(long long*, int, int, int, cudaStream_t);
 int mma2_bench(long long*, int, int, cudaStream_t);
@@ -24,12 +22,6 @@ extern "C" {
 /* debug: device pointer to 8 uint64 cycle counters filled by subsequent GEMM launches (NULL disables) */
 int abcgpt_debug_gemm_stats(void* device_counters) {
   abcgpt::g_gemm_stats = reinterpret_cast<unsigned long long*>(device_counters);
-  return 0;
-}
-
-/* debug: 3 x (CTAs of one attention launch) x 4 int64 {start ns, end ns, SM id, steps}: forward, dK/dV, dQ kernels */
-int abcgpt_debug_attn_cta_trace(void* device_records) {
-  abcgpt::g_attn_cta_trace = reinterpret_cast<long long*>(device_records);
   return 0;
 }
 
@@ -63,11 +55,6 @@ int abcgpt_debug_tmem_mma_bench(void* out, int iters, int nwarps, int x16, int i
 /* debug: MUFU.EX2 rate by operand format, compile-time modes (csrc/microbench.cu mufu2_bench_kernel); out[warp] = cycles */
 int abcgpt_debug_mufu2_bench(void* out, void* sink, int iters, int warps, int mode, void* stream) {
   return abcgpt::mufu2_bench(reinterpret_cast<long long*>(out), reinterpret_cast<float*>(sink), iters, warps, mode, S(stream));
-}
-
-int abcgpt_debug_attn_trace(void* device_stamps) {
-  abcgpt::g_attn_trace = reinterpret_cast<long long*>(device_stamps);
-  return 0;
 }
 
 }  // extern "C"

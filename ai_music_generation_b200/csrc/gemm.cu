@@ -13,9 +13,6 @@
 // The accumulator is double-buffered in TMEM (2 x BN columns) so the epilogue of tile i overlaps the
 // main loop of tile i+1.
 #include "common.h"
-#include <stdlib.h>
-#include <mutex>
-#include <vector>
 #include "dropout.cuh"
 #include "kernels.h"
 #include "ptx.cuh"
@@ -23,8 +20,6 @@
 namespace abcgpt {
 
 unsigned long long* g_gemm_stats = nullptr;  // debug only: set through abcgpt_debug_gemm_stats
-bool g_dynamic_tiles = false;                // abcgpt_set_dynamic_tiles: ticket-based tile scheduler for the pair GEMM launches that follow
-void set_dynamic_tiles(bool on) { g_dynamic_tiles = on; }
 
 namespace {
 
@@ -61,7 +56,6 @@ struct GemmParams {
   long long head_stride;  // BF16 epilogue: != 0 -> column c of a row goes to (c / 64) * head_stride + c % 64 (head-major KV cache)
   int half_from, half_extra;  // pair kernel: tiles >= half_from are processed as two 256 x 128 half tiles (work items
                               // half_from + 2 j, + 2 j + 1 of tile half_from + j): see "Half tiles" above gemm2_kernel
-  int* sched;  // pair kernel: global ticket counter of the dynamic tile scheduler (nullptr = static round-robin)
   unsigned long long* stats;  // optional debug counters (cycles): [0] producer empty-wait, [1] mma full-wait,
                               // [2] mma tmem-empty wait, [3] epilogue tmem-full wait, [4] epilogue busy, [5] cta total
 };
@@ -579,7 +573,6 @@ struct Cfg2 {
   static constexpr int B_BYTES = (BN / 2) * BK * 2;   // 128 of the 256 B rows per CTA
   static constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
   static constexpr int TMEM_COLS = 512;
-  static constexpr int SCHED_SLOTS = 16;               // ring of published work ids (dynamic tile scheduler)
 };
 // TMA-store epilogues (TS): every epilogue warp owns TWO staging buffers of one 32-row x 32-column bf16 chunk each (2 KB,
 // SWIZZLE_64B): one per output stream for the GELU epilogue (h and gelu(h)), alternating by chunk for the single-stream ones.
@@ -597,19 +590,6 @@ struct Cfg2S {
   static_assert(SMEM_BYTES <= 232448, "pair GEMM: shared memory budget");
 };
 
-// Dynamic tile scheduler (opt-in: ABCGPT_DYNAMIC_TILES=1).  The static round-robin `w = pair, pair + num_pairs, ...`
-// assumes every CTA pair is resident from the start; a pair that starts late (its SMs held by another stream's kernel, e.g.
-// an NCCL all-reduce) delays the whole GEMM.  Here the first tile of a pair stays static (no atomic round trip on a launch's
-// critical path: with it the 147 GEMM launches of a step lost 0.4 ms), from the second on the leader's producer warp draws
-// tickets from a global counter while it issues the previous tile's loads and publishes them to both CTAs through a 16-slot
-// shared-memory ring with one mbarrier per slot (plain store + arrive locally; st.async + complete_tx to the peer, so every
-// waiter uses an ordinary CTA-scope wait — a cluster-scope acquire wait costs a CCTL.IVALL per waiter); the value is
-// broadcast with __shfl_sync so the issue loops stay on the uniform datapath.  Producer, MMA and epilogue warps read the
-// ring at their own pace (never more than ~9 tiles apart: operand ring + two accumulators + the prefetched ticket).
-// Resident pairs absorb the tiles of late ones; every pair draws exactly one end ticket, so the pair holding the last one
-// resets the counter for the next launch.  MEASURED: parity-green, but no gain — 4-GPU DDP step 26.0 ms with either
-// schedule (the all-reduce cost that overlap fails to hide, ~0.9 of 1.1 ms, is therefore NOT late GEMM pairs), one GPU
-// 25.65 vs 25.48 ms.  Kept for experiments with other co-running kernels.
 // 18 warps: ptxas caps the kernel at 96 registers per thread, and that IS the hardware limit (registers are allocated per warp
 // in units of 512: 112 per thread rounds to 4096 per warp, x 18 > 65 536 — a __maxnreg__(112) build fails to launch).
 template <bool A_MN, bool B_MN, int EPI, bool TS>
@@ -626,8 +606,6 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
   uint64_t* tfull = empty + C::STAGES;
   uint64_t* tempty = tfull + 2;
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty + 2);
-  uint32_t* sched_id = reinterpret_cast<uint32_t*>(ctrl + 192);     // [SCHED_SLOTS]
-  uint64_t* sched_full = reinterpret_cast<uint64_t*>(ctrl + 256);  // [SCHED_SLOTS]
 
   const int warp = ptx::uniform(threadIdx.x >> 5);  // provably warp-uniform: the issuer loops below stay on the uniform datapath
   const int lane = threadIdx.x & 31;
@@ -655,7 +633,6 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
       ptx::mbar_init(&tfull[s], 1);
       ptx::mbar_init(&tempty[s], 2 * kNumEpiWarps);
     }
-    for (int s = 0; s < C::SCHED_SLOTS; ++s) ptx::mbar_init(&sched_full[s], 1);
     ptx::fence_mbar_init();
   }
   if (warp == kMmaWarp) {
@@ -686,23 +663,7 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
   const long long t_start = p.stats ? clock64() : 0;
   long long w0 = 0, w1 = 0;
   const int num_pairs = gridDim.x / 2;
-  // dynamic scheduling from the SECOND tile of a pair on: the first one is static (w = pair index), so a launch does not
-  // start with an atomic round trip plus a message to the peer CTA on its critical path (147 GEMM launches per step)
-  const bool dyn = p.sched != nullptr && total_work > num_pairs;
-  const int dyn_work = total_work - num_pairs;  // tickets [0, dyn_work) map to work items num_pairs + ticket
-  // work item of iteration `it` of this pair (-1: none left)
-  auto next_work = [&](int it) -> int {
-    if (!dyn) {
-      const int w = pair_id + it * num_pairs;
-      return w < total_work ? w : -1;
-    }
-    if (it == 0) return pair_id;
-    const int slot = it & (C::SCHED_SLOTS - 1);
-    ptx::mbar_wait(&sched_full[slot], (it / C::SCHED_SLOTS) & 1, 45);
-    // a value loaded from shared memory is not provably warp-uniform: without the broadcast the TMA / MMA issue loops that
-    // derive coordinates and trip counts from it fall off the uniform datapath (ptx.cuh, "Warp-uniform issue")
-    return static_cast<int>(ptx::uniform(ptx::ld_shared_u32_volatile(&sched_id[slot])));
-  };
+  // static round-robin: iteration `it` of a pair processes work item pair_id + it * num_pairs
 
   if (warp == kProdWarp) {
     // ===================== TMA producer (both CTAs) =====================
@@ -710,41 +671,7 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
       const bool issue = ptx::elect_one();  // whole warp runs the loop, one elected lane issues (uniform operands)
       int stage = 0;
       uint32_t phase = 0;
-      // leader: a ticket is drawn while the previous tile's loads are being issued and published (to both CTAs) once they
-      // are: the atomic's round trip is never waited for (its result is first touched a whole tile after it was issued)
-      bool drew_end = false;
-      int pending = -1;
-      auto draw = [&]() -> int {
-        if (drew_end) return -1;
-        return atomicAdd(p.sched, 1);
-      };
-      auto post = [&](int i, int w) {  // work id of iteration i -> both CTAs' rings
-        const int slot = i & (C::SCHED_SLOTS - 1);
-        ptx::st_shared_u32_volatile(&sched_id[slot], static_cast<uint32_t>(w));
-        ptx::mbar_arrive(&sched_full[slot]);  // own CTA: plain store + release arrive
-        const uint32_t peer_bar = ptx::mapa(ptx::smem_u32(&sched_full[slot]), crank ^ 1u);
-        ptx::mbar_arrive_expect_tx_cluster(peer_bar, 4);  // peer CTA: the word travels with its own completion
-        ptx::st_async_u32(ptx::mapa(ptx::smem_u32(&sched_id[slot]), crank ^ 1u), static_cast<uint32_t>(w), peer_bar);
-      };
-      auto publish = [&](int i, int w) {
-        if (w >= 0) {
-          if (w == dyn_work + num_pairs - 1) atomicExch(p.sched, 0);  // the last ticket of this launch
-          if (w >= dyn_work) {
-            w = -1;
-            drew_end = true;
-          } else {
-            w += num_pairs;
-          }
-        }
-        post(i, w);
-      };
-      if (dyn && leader && issue) {
-        pending = draw();    // ticket of iteration 1
-        post(0, pair_id);    // nobody waits for slot 0 now (iteration 0 is static), but its phase must advance for iteration 16
-      }
-      for (int it = 0;; ++it) {
-        const int w = next_work(it);
-        if (w < 0) break;
+      for (int w = pair_id; w < total_work; w += num_pairs) {
         const int split = w % p.splits;
         const bool is_half = w >= p.half_from;   // (half tiles only with splits == 1: w is the tile index below half_from)
         const int tile = is_half ? p.half_from + ((w - p.half_from) >> 1) : w / p.splits;
@@ -777,10 +704,6 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
             phase ^= 1;
           }
         }
-        if (dyn && leader && issue) {  // this tile's loads are out: hand the next work item to both CTAs, draw one more
-          publish(it + 1, pending);
-          pending = draw();
-        }
       }
       if (issue && p.stats) atomicAdd(&p.stats[0], static_cast<unsigned long long>(w0));
     }
@@ -794,9 +717,7 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
       constexpr uint32_t idesc_half = ptx::umma_idesc_bf16(256, BN / 2, A_MN ? 1 : 0, B_MN ? 1 : 0);
       int stage = 0;
       uint32_t phase = 0;
-      for (int it = 0;; ++it) {
-        const int w = next_work(it);
-        if (w < 0) break;
+      for (int it = 0, w = pair_id; w < total_work; ++it, w += num_pairs) {
         const uint32_t idesc = w >= p.half_from ? idesc_half : idesc_full;
         const int split = w % p.splits;
         const int kb0 = split * p.kb_per_split;
@@ -844,9 +765,7 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
     const int quarter = warp & 3;
     const int half = (warp - kEpiWarp0) >> 2;      // which quarter of the BN columns
     constexpr int COLS_PER_WARP = BN / (kNumEpiWarps / 4);
-    for (int it = 0;; ++it) {
-      const int w = next_work(it);
-      if (w < 0) break;
+    for (int it = 0, w = pair_id; w < total_work; ++it, w += num_pairs) {
       const bool is_half = w >= p.half_from;
       const int tile = is_half ? p.half_from + ((w - p.half_from) >> 1) : w / p.splits;
       const int m_unit = tile / p.num_n_blk;
@@ -1070,34 +989,6 @@ int dispatch_epi2(int epi, const CUtensorMap& tmA, const CUtensorMap& tmB, const
   return fail(-1, "unknown GEMM epilogue %d", epi);
 }
 
-// one ticket counter per (device, stream) that has launched a pair GEMM (kernels on one stream run one after another; two
-// streams must not share a counter).  Opt-in (ABCGPT_DYNAMIC_TILES=1): measured neutral under 4-GPU data parallelism
-// (26.0 ms either way) and -0.7 % on one GPU, see the comment above gemm2_kernel.
-int* sched_counter(cudaStream_t stream) {
-  struct Entry { int dev; cudaStream_t st; int* ptr; };
-  static std::mutex mu;
-  static std::vector<Entry> pool;
-  static int enabled = -1;
-  if (enabled < 0) {
-    const char* e = getenv("ABCGPT_DYNAMIC_TILES");
-    enabled = (e == nullptr || e[0] == '\0') ? 2 : (e[0] == '1' ? 1 : 0);   // 2: not forced, the caller decides (set_dynamic_tiles)
-  }
-  if (enabled == 0 || (enabled == 2 && !g_dynamic_tiles)) return nullptr;
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess) return nullptr;
-  std::lock_guard<std::mutex> lock(mu);
-  for (const Entry& e : pool)
-    if (e.dev == dev && e.st == stream) return e.ptr;
-  if (pool.size() >= 256) return nullptr;
-  cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-  if (cudaStreamIsCapturing(stream, &cap) != cudaSuccess || cap != cudaStreamCaptureStatusNone) return nullptr;
-  int* ptr = nullptr;
-  if (cudaMalloc(&ptr, 128) != cudaSuccess) return nullptr;
-  if (cudaMemset(ptr, 0, 128) != cudaSuccess || cudaDeviceSynchronize() != cudaSuccess) return nullptr;
-  pool.push_back({dev, stream, ptr});
-  return ptr;
-}
-
 int dispatch_major2(int a_mn, int b_mn, int epi, const CUtensorMap& tmA, const CUtensorMap& tmB, const GemmParams& p,
                     long long grid, cudaStream_t stream) {
   if (!a_mn && !b_mn) return dispatch_epi2<false, false>(epi, tmA, tmB, p, grid, stream);
@@ -1203,7 +1094,7 @@ int gemm_bf16(const void* a, int a_mn, long long lda, const void* b, int b_mn, l
   p.M = M; p.N = N; p.K = K;
   p.num_m_blk = num_m_blk; p.num_n_blk = num_n_blk; p.num_k_blk = num_k_blk;
   p.splits = splits; p.kb_per_split = kb_per_split;
-  p.c = c; p.ldc = ldc; p.c2 = c2; p.ldc2 = ldc2; p.aux = aux; p.ldaux = ldaux; p.bias = bias; p.act_tanh = act_tanh; p.head_stride = (epi == ABCGPT_EPI_BF16 && c2 == nullptr) ? ldc2 : 0; p.sched = pair ? sched_counter(stream) : nullptr; p.stats = g_gemm_stats; p.drop = make_drop(drop_p, drop_key);
+  p.c = c; p.ldc = ldc; p.c2 = c2; p.ldc2 = ldc2; p.aux = aux; p.ldaux = ldaux; p.bias = bias; p.act_tanh = act_tanh; p.head_stride = (epi == ABCGPT_EPI_BF16 && c2 == nullptr) ? ldc2 : 0; p.stats = g_gemm_stats; p.drop = make_drop(drop_p, drop_key);
   {
     const bool f32_out = (epi == ABCGPT_EPI_RESID || epi == ABCGPT_EPI_F32 || epi == ABCGPT_EPI_F32_RED);
     const long long cb = f32_out ? 4 : 2, ab = (epi == ABCGPT_EPI_RESID) ? 4 : 2;
@@ -1216,7 +1107,7 @@ int gemm_bf16(const void* a, int a_mn, long long lda, const void* b, int b_mn, l
   long long total = static_cast<long long>(num_m_units) * num_n_blk * splits;
   p.half_from = 0x7fffffff;
   p.half_extra = 0;
-  if (pair && splits == 1 && epi != ABCGPT_EPI_F32_RED && p.sched == nullptr) {
+  if (pair && splits == 1 && epi != ABCGPT_EPI_F32_RED) {
     // half tiles for a short last round of the static schedule (see gemm2_kernel)
     const long long r = total % units;
     if (total > units && r > 0 && 2 * r <= units && total + r < 0x7fffffff) {

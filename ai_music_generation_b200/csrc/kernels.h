@@ -73,7 +73,6 @@ int sample_batch(const void* data, int token_bytes, long long n_tokens, const in
                  cudaStream_t stream);
 int nvls_allreduce_sumsq(void* grad_mc, long long n, int rank, int world, float scale, void* partials_mc, int blocks_per_rank,
                          int threads, cudaStream_t stream);
-void set_dynamic_tiles(bool on);
 int sumsq_partials(const float* partials, int nparts, float* out, cudaStream_t stream);
 int colsum_bf16(const void* dy, long long ld, int M, int N, float* out, cudaStream_t stream);
 int argmax_rows(const void* logits, long long ldl, int V, int64_t* out, long long out_stride, int B,

@@ -366,26 +366,6 @@ __device__ __forceinline__ void bar_sync(int id, int nthreads) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }
 
-// Message to the peer CTA of a cluster (dynamic tile scheduler of the pair GEMM): st.async writes one word into the peer's
-// shared memory and credits its bytes to the peer's mbarrier (complete_tx), so the word is visible to anyone who observed
-// that barrier phase with an ordinary CTA-scope wait.  (A cluster-scope acquire wait costs a CCTL.IVALL per waiter.)
-__device__ __forceinline__ void mbar_arrive_expect_tx_cluster(uint32_t cluster_bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cluster.b64 _, [%0], %1;" ::"r"(cluster_bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void st_async_u32(uint32_t cluster_addr, uint32_t v, uint32_t cluster_bar) {
-  asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.b32 [%0], %1, [%2];" ::"r"(cluster_addr), "r"(v),
-               "r"(cluster_bar)
-               : "memory");
-}
-__device__ __forceinline__ uint32_t ld_shared_u32_volatile(const uint32_t* p) {
-  uint32_t v;
-  asm volatile("ld.volatile.shared::cta.u32 %0, [%1];" : "=r"(v) : "r"(smem_u32(p)) : "memory");
-  return v;
-}
-__device__ __forceinline__ void st_shared_u32_volatile(uint32_t* p, uint32_t v) {
-  asm volatile("st.volatile.shared::cta.u32 [%0], %1;" ::"r"(smem_u32(p)), "r"(v) : "memory");
-}
-
 // programmatic dependent launch (see launch_k in common.h)
 #ifndef ABCGPT_NO_PDL
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }

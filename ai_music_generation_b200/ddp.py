@@ -237,13 +237,7 @@ def nvls_setup(m, process_group=None):
     # overlap (default): bucket by bucket beside the backward, `blocks` CTAs of `threads` threads per launch (one 128-thread CTA per SM
     # fits next to a persistent GEMM CTA); the ranges released when the backward has ended go out in one full-size launch.
     # ABCGPT_NVLS_OVERLAP=0: one exchange of the whole arena after the backward.
-    # Measured alternative (opt-in, ABCGPT_NVLS_DYNAMIC_TILES=1 with ABCGPT_NVLS_BLOCKS=16 ABCGPT_NVLS_THREADS=256): a co-resident CTA slows
-    # the GEMM CTA it shares an SM with by ~25 %, and a static tile schedule waits for the slowest SM (+13..48 % per GEMM in
-    # tools/coresidency_probe.py, +3..7 % with the ticket-based scheduler and 16 exchange CTAs) — in the 2-GPU step both forms measured
-    # the same (25.08 / 25.16 vs 25.14 ms), so the form validated on 8 GPUs stays the default.
     overlap = os.environ.get("ABCGPT_NVLS_OVERLAP", "1") != "0"
-    if overlap and os.environ.get("ABCGPT_NVLS_DYNAMIC_TILES", "0") == "1":
-        ops.set_dynamic_tiles(True)
     return {"hdl": hdl, "thdl": thdl, "table": table, "overlap": overlap,
             "blocks": int(os.environ.get("ABCGPT_NVLS_BLOCKS", "148")), "threads": int(os.environ.get("ABCGPT_NVLS_THREADS", "128"))}
 

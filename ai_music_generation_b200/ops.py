@@ -521,11 +521,6 @@ def nvls_allreduce_sumsq(grad_mc_ptr, n, rank, world, partials_mc_ptr, blocks_pe
           1.0 / world, int(partials_mc_ptr), int(blocks_per_rank), int(threads), _stream())
 
 
-def set_dynamic_tiles(on):
-    """include/abcgpt.h abcgpt_set_dynamic_tiles: ticket-based tile scheduler for the pair GEMM launches that follow."""
-    _C.lib().abcgpt_set_dynamic_tiles(1 if on else 0)
-
-
 def sumsq_partials(partials, nparts, out):
     _call("sumsq_partials", 1, (nparts,), _C.lib().abcgpt_sumsq_partials, partials.data_ptr(), int(nparts), out.data_ptr(), _stream())
 

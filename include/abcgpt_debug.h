@@ -1,6 +1,6 @@
 /*
  * libabcgpt_debug — instrumentation and hardware micro-benchmarks used by the scripts under tools/ (tools/gemm_stats.py,
- * tools/attn_trace.py, tools/attn_cta_timeline.py, tools/mma_bench.py, tools/tmem_bench.py).  These entry points are NOT in
+ * tools/gemm_timeline.py, tools/mma_bench.py, tools/tmem_bench.py).  These entry points are NOT in
  * the product library libabcgpt.so: `python -m ai_music_generation_b200.build --debug` links them (csrc/debug_api.cu,
  * csrc/microbench.cu) together with the product objects into libabcgpt_debug.so.
  */
@@ -18,10 +18,6 @@ extern "C" {
  * only, %globaltimer nanoseconds over all CTAs (the caller presets the min slots to ~0): [8] min kernel entry, [9] max / [15] min
  * prologue done, [10] min / [11] max first operand stage landed, [12] max last MMA committed, [13] max epilogue done, [14] max exit. */
 int abcgpt_debug_gemm_stats(void* device_counters);
-/* Debug aid: device pointer to int64[num_kv_tiles * 8]; one CTA of the next attention forward launches stamps clock64
- * at its phase boundaries (NULL disables). */
-int abcgpt_debug_attn_trace(void* device_stamps);
-int abcgpt_debug_attn_cta_trace(void* device_records);
 int abcgpt_debug_mma_bench(void* out, int iters, int n, int mode, void* stream);
 int abcgpt_debug_tmem_ld_bench(void* out, int iters, int nwarps, int inflight, void* stream);
 /* Operand-format probe of the CTA-pair MMA: d[256,64] fp32 = a[256,64] bf16 x B; mode bit 0: b is B^T [n][k] (K-major halves) instead
